@@ -2,7 +2,7 @@
 """Benchmark of the swarm hot path (BASELINE.json metric: swarm env-steps/s & locust-updates/s).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c4|c2|n80|paac3|paac5] [--scaling strong|weak]
-                    [--impl ours|reference]
+                    [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one batch-step: every env of the rank's shard advances once through the fused kernel
@@ -14,12 +14,14 @@ scaling -- the named batch is split over the ranks like the reference splits its
 data-path collective.  `--scaling weak` gives every GPU the whole named batch; at N > 1 the default line carries that
 figure too (secondary.weak).  Rank 0 prints ONE JSON line.
 
-The timed region is never shorter than 256 steps (two whole 128-step episodes, i.e. two lock-step auto-reset
-boundaries) nor than 0.25 s, whatever --steps says (`steps` = what was timed, `steps_requested` = the flag).
+The timed region is exactly --steps batch-steps and starts 8 steps into a fresh episode, so it holds (K + 8) // 128
+lock-step auto-reset boundaries (every env runs the reset's 10 burn-in steps inside one batch-step).
+
+--dump-outputs DIR writes what the last timed step returned to its caller (see dump_outputs).  Inputs are seeded, so two
+builds run with the same arguments can be compared array for array.
 """
 import argparse
 import json
-import math
 import os
 import statistics
 import subprocess
@@ -46,7 +48,8 @@ PAAC = {
 A, G = 10, 84
 FLOPS_PER_PAIR = 18            # SURVEY.md 8(d)
 MUFU_PER_CLK_SM = 15.93        # measured, scripts/microbench.cu (profiles/r01_microbench.jsonl)
-MIN_STEPS, MIN_SECONDS = 256, 0.25
+MIN_STEPS = 256                # end-to-end (host-buffer) figure
+DUMP_ENVS = 512                # --dump-outputs: at most this many envs (a seeded sample), about 31 MB at 84x84 and N = 256
 
 
 def ncu_traffic(workload):
@@ -126,7 +129,7 @@ class ClockSampler(object):
             return None
         inside = [r for r in rows if t_begin - 0.02 <= r[0] <= t_end + 0.02]
         where = "timed region"
-        if not inside:                      # cannot happen any more (the region is >= 0.25 s); kept as a guard
+        if not inside:                      # a short timed region can fall between two 20 ms samples
             inside = sorted(rows, key=lambda r: r[1])[len(rows) // 2:]
             where = "whole run (no sample inside the timed region)"
         reasons = sorted({n for r in inside for n in r[2]})
@@ -282,10 +285,27 @@ def run_paac(args, wl, key):
         dist.destroy_process_group()
 
 
-def measure_env(M, torch, dist, dev, world, rank, E, N, first_id, K_req, W, math_mode, use_graph, sampler=None,
-                want_extras=True):
-    """Times the device-resident batch-step of E envs x N locusts on this rank.  Returns a dict of measurements;
-    every time is the MAX over ranks."""
+def dump_outputs(out_dir, env):
+    """Writes what the last step returned to its caller -- the state (x, xa), reward, done and the observation (grid,
+    positions) -- as out_dir/<name>.npy, the state in float64 and the rest in float32.  Batches of more than DUMP_ENVS
+    envs keep a fixed seeded sample of DUMP_ENVS of them; env_index.npy lists which (local env ids)."""
+    import numpy as np
+    import torch
+    E = env.E
+    idx = np.arange(E) if E <= DUMP_ENVS else np.sort(np.random.RandomState(0).choice(E, DUMP_ENVS, replace=False))
+    sel = torch.as_tensor(idx, device=env.device)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "env_index.npy"), idx.astype(np.float64))
+    for name, t in (("x", env.x), ("xa", env.xa), ("reward", env.reward), ("done", env.done_u8), ("grid", env.grid),
+                    ("positions", env.positions)):
+        a = t.index_select(0, sel).cpu().numpy()
+        np.save(os.path.join(out_dir, name + ".npy"), a if a.dtype == np.float64 else a.astype(np.float32))
+
+
+def measure_env(M, torch, dist, dev, world, rank, E, N, first_id, K, W, math_mode, use_graph, sampler=None,
+                want_extras=True, dump_dir=None):
+    """Times K device-resident batch-steps of E envs x N locusts on this rank.  Returns a dict of measurements;
+    every time is the MAX over ranks.  dump_dir: where to write the last timed step's outputs (dump_outputs)."""
     env = M.BatchedSwarmEnv(E, n_locusts=N, n_agents=A, grid_size=G, max_episode_steps=128, seed=1234,
                             env_id_offset=first_id, device=dev, math_mode=math_mode, auto_reset=True, rasterize=True)
     env.reset()
@@ -344,16 +364,17 @@ def measure_env(M, torch, dist, dev, world, rank, E, N, first_id, K_req, W, math
             for i in range(8):
                 step(i)
     run8 = (lambda i: graph.replay()) if graph is not None else (lambda i: [step(j) for j in range(8)])
-    # calibration (untimed for the result): 64 steps -> how many steps make >= MIN_SECONDS
-    cal_ms = timed(run8, 8) / 64.0
-    K = max(int(K_req), MIN_STEPS, int(math.ceil(MIN_SECONDS * 1e3 / max(cal_ms, 1e-6))))
-    K = ((K + 127) // 128) * 128            # whole 128-step episodes: every timed region holds K/128 auto-reset boundaries
-    K = int(rank_max(K))
-    env.reset()                             # start the timed region on an episode boundary (elapsed = 0 everywhere)
+    # untimed: the first replays upload the graph.  Ending them in a synchronise (timed() does) before the reset below
+    # measured 0.1 % faster timed steps than letting the reset queue behind them.
+    timed(run8, 8)
+    env.reset()                             # start the timed region in a fresh episode (elapsed = 8 everywhere)
     for i in range(8):
         step(i)
-    t_ms = timed(run8, K // 8)
+    # K steps in order ring[0], ring[1], ...: whole 8-step replays, then the remainder launched one by one
+    t_ms = timed(lambda i: run8(i) if i < K // 8 else step(i - K // 8), K // 8 + K % 8)
     clocks = sampler.stop(wall[0], wall[1]) if sampler else None
+    if dump_dir is not None:
+        dump_outputs(dump_dir, env)
     out = dict(E=E, N=N, K=K, ms=t_ms, ms_per_step=t_ms / K, plan=plan, clocks=clocks, region_s=wall[1] - wall[0])
     # per-8-step latencies over one episode: the lock-step boundary (10 burn-in steps inside one step) shows as the max
     env.reset()
@@ -426,7 +447,13 @@ def main():
     ap.add_argument("--no-paac", action="store_true", help="skip the secondary PAAC frames/s figure (config 3)")
     ap.add_argument("--no-graph", action="store_true", help="launch every step from Python instead of replaying a CUDA graph")
     ap.add_argument("--cpu-seconds", type=float, default=12.0, help="target wall time of the CPU-baseline sample")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step as DIR/<name>.npy (rank 0's envs; --impl ours, c4/c2/n80)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload not in WORKLOADS):
+        ap.error("--dump-outputs needs --impl ours and one of the workloads %s" % "/".join(sorted(WORKLOADS)))
     if args.workload in PAAC:
         if args.impl == "reference":
             print(json.dumps({"impl": "reference", "unavailable": "the reference learner needs TensorFlow 1.4 (not in this image)"}))
@@ -459,7 +486,7 @@ def main():
     E_total = E * world
     sampler = ClockSampler(local) if rank == 0 else None      # started early: nvidia-smi takes a moment to come up
     m = measure_env(M, torch, dist, dev, world, rank, E, N, first, args.steps, args.warmup, args.math, not args.no_graph,
-                    sampler=sampler, want_extras=True)
+                    sampler=sampler, want_extras=True, dump_dir=args.dump_outputs if rank == 0 else None)
     K, ms_step = m["K"], m["ms_per_step"]
     env_steps = E_total / (ms_step * 1e-3)
     pairs_per_launch = E * N * (N + A)                        # per rank: what ONE launch of the dominant kernel does
@@ -557,15 +584,15 @@ def main():
         e2e_val = E_total * N / (m["e2e_ms_per_step"] * 1e-3)
         out = {
             "metric": "locust_updates_per_sec", "value": env_steps * N, "unit": "locust-updates/s",
-            "n_gpus": world, "steps": K, "steps_requested": args.steps, "warmup": args.warmup, "ms_per_step": ms_step,
+            "n_gpus": world, "steps": K, "warmup": args.warmup, "ms_per_step": ms_step,
             "higher_is_better": True, "scaling": args.scaling, "vs_baseline": None,
             "dtype": "f32 pair forces / f64 integrator state", "data": "synthetic",
             "config": {"workload": wl["name"] + "; fused step + TimeLimit(128) + auto-reset + 84x84 compact rasterise",
                        "envs_total": E_total, "envs_per_gpu": E, "n_locusts": N, "n_agents": A, "grid": G, "math": args.math,
                        "actions": "N(0,1) clipped to unit norm, 8 pre-generated device tensors",
                        "launch": "python per step" if args.no_graph else "CUDA graph of 8 steps replayed",
-                       "timed_region": "%d steps = %d whole 128-step episodes (lock-step auto-reset boundaries included), %.2f s"
-                                       % (K, K // 128, m["region_s"]),
+                       "timed_region": "%d steps from step 8 of an episode, %d lock-step auto-reset boundaries included, %.2f s"
+                                       % (K, (K + 8) // 128, m["region_s"]),
                        "l2": ("no explicit flush: each step streams %.0f MB of observations per GPU, more than the 126 MB L2"
                               if E * G * G * 8 > 126e6 else
                               "no explicit flush: each step streams %.0f MB of observations per GPU (smaller than the 126 MB "

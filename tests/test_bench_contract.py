@@ -1,10 +1,11 @@
-"""bench.py contract checks that run without a GPU: the reference arm (CPU port on the host cores) prints ONE JSON
-line with the keys the driver reads, and non-zero ranks stay silent."""
+"""bench.py contract checks: the reference arm (CPU port on the host cores) prints ONE JSON line with the keys a caller
+reads, non-zero ranks stay silent; on the GPU, --steps sets the timed steps and --dump-outputs is reproducible."""
 import json
 import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -42,6 +43,41 @@ def test_reference_arm_other_ranks_are_silent():
     res = run(["--impl", "reference", "--workload", "c2", "--steps", "3", "--warmup", "3", "--gpus", "2"],
               env={"RANK": "1", "WORLD_SIZE": "2", "LOCAL_RANK": "1"})
     assert res.returncode == 0 and res.stdout.strip() == ""
+
+
+def test_dump_outputs_only_for_the_gpu_env_path(tmp_path):
+    for args in (["--impl", "reference"], ["--workload", "paac3"], ["--steps", "0"]):
+        res = run(args + ["--dump-outputs", str(tmp_path / "out")])
+        assert res.returncode == 2 and "usage" in res.stderr, args
+    assert not (tmp_path / "out").exists()
+
+
+@pytest.mark.gpu
+def test_dump_outputs_are_the_last_timed_step_and_reproducible(tmp_path):
+    """Exactly --steps steps are timed (not a multiple of the 8-step graph); the dump is float32/float64, at most 64 MB,
+    a seeded sample of the 1024 envs, self-consistent (grid and positions rasterise the dumped state bit for bit) and
+    identical on a second run with the same arguments."""
+    from oracle import swarm_oracle as so
+    args = ["--workload", "c2", "--steps", "13", "--warmup", "3", "--no-cpu-baseline", "--no-secondary", "--no-paac"]
+    dumps = []
+    for k in range(2):
+        out = tmp_path / str(k)
+        res = run(args + ["--dump-outputs", str(out)])
+        assert res.returncode == 0, res.stderr
+        assert json.loads(res.stdout.strip().splitlines()[-1])["steps"] == 13
+        files = sorted(out.glob("*.npy"))
+        assert sum(p.stat().st_size for p in files) <= 64 << 20
+        d = {p.stem: np.load(p) for p in files}
+        assert set(d) == {"env_index", "x", "xa", "reward", "done", "grid", "positions"}
+        assert all(a.dtype in (np.float32, np.float64) for a in d.values())
+        assert d["x"].shape == (512, 64, 2) and d["x"].dtype == np.float64 and d["grid"].shape == (512, 84, 84, 2)
+        assert len(set(d["env_index"].tolist())) == 512 and d["env_index"].max() < 1024
+        for e in (0, 255, 511):
+            g, p = so.rasterize(d["x"][e], d["xa"][e], 84)
+            assert np.array_equal(d["grid"][e], g.astype(np.float32)) and np.array_equal(d["positions"][e], p)
+        dumps.append(d)
+    for name, a in dumps[0].items():
+        assert np.array_equal(a, dumps[1][name]), name
 
 
 def test_strong_scaling_is_the_default_and_shards_like_np_split(pkg):
