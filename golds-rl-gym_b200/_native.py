@@ -32,6 +32,7 @@ SWARM_STEP_CLIP_ACTIONS = 2
 SWARM_STEP_ACTIONS_F64 = 4
 SWARM_STEP_NO_ACTION_WIND = 8
 SWARM_STEP_INKERNEL_RASTER = 16
+SWARM_STEP_FRESH_NOISE = 32
 # SwarmParams.tuning: bits 4-5 = rasteriser placement (0 automatic); every other bit must be 0
 TUNE_RASTER_FOLLOW, TUNE_RASTER_WARPS, TUNE_RASTER_SELF = 1 << 4, 2 << 4, 3 << 4
 
@@ -84,6 +85,8 @@ SYMBOLS = {
     "swarm_clip_actions": (c_int, [c_void_p, c_int64, c_float, c_void_p]),
     "swarm_philox_draws": (c_int, [_P(SwarmParams), _P(SwarmState), c_void_p, c_void_p, c_void_p, c_void_p,
                                    c_void_p, c_void_p]),
+    "swarm_philox_noise_rows": (c_int, [_P(SwarmParams), _P(SwarmState), c_int32, c_int32, c_void_p, c_void_p,
+                                        c_void_p]),
     "swarm_philox_raw": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_void_p]),
 }
 

@@ -24,8 +24,9 @@ from .emulator_runner import SwarmRunner
 
 class SwarmPolicyMonitor(object):
     def __init__(self, env=None, global_policy_net=None, state_processor=None, summary_writer=None, saver=None,
-                 network_conf=None, out_dir="."):
-        self.env = env if env is not None else ma.make("Swarm-eval-v0")
+                 network_conf=None, out_dir=".", fresh_noise=False):
+        # fresh_noise: the default eval env follows the training envs' noise mode (SURVEY Q1 fixed or not)
+        self.env = env if env is not None else ma.make("Swarm-eval-v0", fresh_noise=fresh_noise)
         self.global_policy_net = global_policy_net
         self.state_processor = state_processor
         self.summary_writer = summary_writer

@@ -28,15 +28,19 @@ __device__ __forceinline__ void prefetch_env(const Stage& sg, const KP& kp, cons
     for (int i = g.tid; i < N; i += g.n) cp_async<16>(sg.xs + i, gx + i);
     const double2* ga = reinterpret_cast<const double2*>(st.xa) + (size_t)e * A;
     const double2* gna = reinterpret_cast<const double2*>(io.noise_a ? io.noise_a : st.noise_a) + (size_t)e * A;
+    const bool fetch_an = !kp.fresh || io.noise_a;     // fresh noise: the step draws the agent row itself
     for (int k = g.tid; k < A; k += g.n) {
         cp_async<16>(sg.as + k, ga + k);
-        cp_async<16>(sg.an + k, gna + k);
+        if (fetch_an) cp_async<16>(sg.an + k, gna + k);
         if (io.flags & SWARM_STEP_ACTIONS_F64)
             cp_async<16>(sg.araw + 16 * k, reinterpret_cast<const double2*>(io.actions_f64) + (size_t)e * A + k);
         else
             cp_async<8>(sg.araw + 16 * k, reinterpret_cast<const float2*>(io.actions_f32) + (size_t)e * A + k);
     }
-    if (g.tid == g.n - 1) cp_async<4>(sg.misc, st.elapsed + e);
+    if (g.tid == g.n - 1) {
+        cp_async<4>(sg.misc, st.elapsed + e);
+        if (kp.fresh) cp_async<4>(sg.misc + 1, st.episode + e);
+    }
 }
 
 // SwarmEnv._step + TimeLimit + SwarmRunner auto-reset + process_state for the whole batch.
@@ -100,15 +104,30 @@ __global__ void __maxnreg__(64) k_step(const KP kp, const SwarmState st, const S
                 if (!filler) raster_zero_fill(io.grid + (size_t)e * cells * 2, cells, g.tid, g.n);
             }
             if (dyn && it > 0) e1 = sm.mail[1];
-            {   // this env's locust noise row: each thread fetches the rows of its own targets, so that its
+            // Fresh noise: the step uses row n_burn + elapsed of noise streams 3 / 4 of the env's current episode (the last
+            // reset was keyed with the counter's value before its increment), drawn below instead of read from HBM
+            DrawCtx nd;
+            nd.key = kp.key;
+            nd.env = kp.env_off + (uint32_t)e;
+            nd.episode = (uint32_t)sm.st.misc[1] - 1u;
+            const uint32_t nrow = (uint32_t)kp.n_burn + (uint32_t)sm.st.misc[0];
+            {   // this env's locust noise row: each thread fetches (or draws) the rows of its own targets, so that its
                 // own wait (before the integration) is all the synchronisation it needs
-                const double2* gnx = reinterpret_cast<const double2*>(io.noise_x ? io.noise_x : st.noise_x) + (size_t)e * N;
+                if (kp.fresh && !io.noise_x) {
 #pragma unroll
-                for (int t = 0; t < T; ++t) {
-                    const int j = target_index<MODE>(g, t, kp);
-                    if (j < N) cp_async<16>(sm.nx + j, gnx + j);
+                    for (int t = 0; t < T; ++t) {
+                        const int j = target_index<MODE>(g, t, kp);
+                        if (j < N) sm.nx[j] = draw_normal2(nd, STREAM_NOISE_X, nrow, (uint32_t)j);
+                    }
+                } else {
+                    const double2* gnx = reinterpret_cast<const double2*>(io.noise_x ? io.noise_x : st.noise_x) + (size_t)e * N;
+#pragma unroll
+                    for (int t = 0; t < T; ++t) {
+                        const int j = target_index<MODE>(g, t, kp);
+                        if (j < N) cp_async<16>(sm.nx + j, gnx + j);
+                    }
                 }
-                cp_async_commit();
+                cp_async_commit();      // (an empty group with fresh noise: env_step's wait counts groups)
             }
             if (e1 < kp.E) prefetch_env(stage_at(smem_raw, N, A, (it + 1) & 1), kp, st, io, e1, g);
             cp_async_commit();     // (possibly empty) group of the next env: env_step waits for all but this one
@@ -141,6 +160,8 @@ __global__ void __maxnreg__(64) k_step(const KP kp, const SwarmState st, const S
                     }
                 }
                 sm.act[k] = a;
+                // fresh noise: the agent's row, by the thread that moves the agent in env_step
+                if (kp.fresh && !io.noise_a) sm.st.an[k] = draw_normal2(nd, STREAM_NOISE_A, nrow, (uint32_t)k);
             }
 
             // One env_step call site serves the step proper and, if the episode ends here, the burn-in
@@ -499,6 +520,25 @@ __global__ void k_philox_draws(const KP kp, const SwarmState st, double2* __rest
         }
         for (int i = threadIdx.x; i < N; i += blockDim.x)
             pn[((size_t)e * rows + r) * N + i] = draw_normal2(ctx, STREAM_NOISE_X, r, i);
+    }
+}
+
+// rows row0.. of noise streams 3 / 4 of every env's current episode (what a SWARM_STEP_FRESH_NOISE step draws);
+// blockIdx.y strides over the rows
+__global__ void k_philox_noise_rows(const KP kp, const SwarmState st, const int row0, const int n_rows,
+                                    double2* __restrict__ an, double2* __restrict__ pn) {
+    const int e = blockIdx.x;
+    const int N = kp.N, A = kp.A;
+    DrawCtx ctx;
+    ctx.key = kp.key;
+    ctx.env = kp.env_off + (uint32_t)e;
+    ctx.episode = st.episode[e] - 1u;
+    for (int r = blockIdx.y; r < n_rows; r += gridDim.y) {
+        const uint32_t row = (uint32_t)row0 + (uint32_t)r;
+        for (int k = threadIdx.x; k < A; k += blockDim.x)
+            an[((size_t)e * n_rows + r) * A + k] = draw_normal2(ctx, STREAM_NOISE_A, row, k);
+        for (int i = threadIdx.x; i < N; i += blockDim.x)
+            pn[((size_t)e * n_rows + r) * N + i] = draw_normal2(ctx, STREAM_NOISE_X, row, i);
     }
 }
 
@@ -875,7 +915,7 @@ int plan_step(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io,
     if ((io->flags & SWARM_STEP_ACTIONS_F64) ? !io->actions_f64 : !io->actions_f32) return SWARM_ERR_NULL;
     if ((io->grid != nullptr) != (io->positions != nullptr)) return SWARM_ERR_FLAGS;
     if (io->flags & ~(SWARM_STEP_AUTO_RESET | SWARM_STEP_CLIP_ACTIONS | SWARM_STEP_ACTIONS_F64 | SWARM_STEP_NO_ACTION_WIND |
-                      SWARM_STEP_INKERNEL_RASTER))
+                      SWARM_STEP_INKERNEL_RASTER | SWARM_STEP_FRESH_NOISE))
         return SWARM_ERR_FLAGS;
     if (reset_draws && !draws_complete(reset_draws)) return SWARM_ERR_NULL;
     if (st->work_words && !st->work) return SWARM_ERR_NULL;
@@ -1003,6 +1043,7 @@ int swarm_step(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io
     kp.n_stage = pl.n_stage;
     kp.dynamic = pl.dynamic;
     kp.wind_step = (io->flags & SWARM_STEP_NO_ACTION_WIND) ? 0 : 1;
+    kp.fresh = (io->flags & SWARM_STEP_FRESH_NOISE) ? 1 : 0;
     const SwarmInjectedDraws dr = reset_draws ? *reset_draws : kNoDraws;
     const int has = reset_draws ? 1 : 0;
     cudaStream_t s = (cudaStream_t)stream;
@@ -1313,6 +1354,19 @@ int swarm_philox_draws(const SwarmParams* p, const SwarmState* st, double* x0, d
         reinterpret_cast<double2*>(xa0), reinterpret_cast<double2*>(burn_actions),
         reinterpret_cast<double2*>(agent_noise), reinterpret_cast<double2*>(particle_noise));
     return check_launch("swarm_philox_draws");
+}
+
+int swarm_philox_noise_rows(const SwarmParams* p, const SwarmState* st, int32_t row0, int32_t n_rows, double* agent_noise,
+                            double* particle_noise, swarm_stream_t stream) {
+    int rc = validate(p);
+    if (rc) return rc;
+    if (!st || !st->episode || !agent_noise || !particle_noise) return SWARM_ERR_NULL;
+    if (row0 < 0 || n_rows <= 0) return SWARM_ERR_SIZE;
+    const KP kp = make_kp(p);
+    const dim3 grid((unsigned)kp.E, (unsigned)(n_rows < 65535 ? n_rows : 65535));
+    k_philox_noise_rows<<<grid, 128, 0, (cudaStream_t)stream>>>(kp, *st, row0, n_rows, reinterpret_cast<double2*>(agent_noise),
+                                                               reinterpret_cast<double2*>(particle_noise));
+    return check_launch("swarm_philox_noise_rows");
 }
 
 int swarm_philox_raw(const uint32_t* ctr, const uint32_t* key, uint32_t* out, int64_t n, swarm_stream_t stream) {

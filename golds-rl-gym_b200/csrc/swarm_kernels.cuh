@@ -54,6 +54,8 @@ struct KP {
                       // group rasterises its own env after the step (points = the stage buffer)
     int filler;       // raster == 2: one extra warp per CTA issues the TMA zero fill of the env's grid and waits for it
     int wind_step;    // 0: the step proper does not add the wind to the actions (SwarmEnv._step(add_wind=False))
+    int fresh;        // k_step (SWARM_STEP_FRESH_NOISE): the step proper draws Philox row n_burn + elapsed instead of
+                      // reading the frozen row
     unsigned long long* trace;   // debug (swarm_debug_trace): per-CTA phase timestamps, nullptr in production
     long long trace_slots;       // capacity of trace in records of 2 * TR_PHASES words
     // rasteriser constants the host can round exactly like numpy does
@@ -64,13 +66,13 @@ struct KP {
 
 // One STAGE buffer = what is prefetched for the step of one env (the locust noise row follows
 // later, straight into Smem::nx):
-//   x (N) | xa (A) | noise_a (A) | raw actions (A x 16 B) | misc (16 B: elapsed)
+//   x (N) | xa (A) | noise_a (A) | raw actions (A x 16 B) | misc (16 B: elapsed, episode)
 struct Stage {
     double2* xs;            // N   locust positions (FP64 integrator state, updated in place)
     double2* as;            // A   agent positions
     double2* an;            // A   agent noise row
     unsigned char* araw;    // A x 16 B: the env's actions as they sit in HBM (f32 pair or f64 pair)
-    int* misc;              // [0] = TimeLimit elapsed steps
+    int* misc;              // [0] = TimeLimit elapsed steps, [1] = resets so far (fresh noise only)
 };
 
 struct Smem {

@@ -4,11 +4,13 @@
 // stateless generator keyed by (seed, GLOBAL env id, episode), so an env's draws do not
 // depend on how the batch is sharded over GPUs, and any draw can be regenerated in place.
 //
-// Draw layout (restated for the tests in oracle/philox.py):
+// Draw layout (restated for the tests in oracle/philox.py; rows past n_burn in tests/_fresh_noise.py):
 //   key     = (seed & 0xffffffff, seed >> 32)
 //   counter = (element index, row, global env id, (episode << 3) | stream)
 //   stream 0: x0   1: xa0   2: burn-in actions (rows 0..n_burn-1)
-//          3: agent noise (rows 0..n_burn)   4: particle noise (rows 0..n_burn)
+//          3: agent noise (rows 0..n_burn + elapsed)   4: particle noise (rows 0..n_burn + elapsed)
+//   (rows 0..n_burn-1 feed the burn-in, row n_burn the first step after the reset -- and every later step
+//   in the frozen mode of the reference; with SWARM_STEP_FRESH_NOISE step `elapsed` uses row n_burn + elapsed)
 #pragma once
 #include <stdint.h>
 

@@ -75,6 +75,8 @@ class BatchedSwarmEnv(object):
     With ``rasterize=True`` (default) the step kernel also writes ``self.grid`` (E,G,G,2) f32 and
     ``self.positions`` (E,A,2) u8 -- SwarmStateProcessor.process_state of the returned state.
     With ``auto_reset=True`` finished envs are reset inside the step (SwarmRunner._run semantics).
+    With ``noise="fresh"`` every step draws the next row of the episode's noise tables (the reference with
+    SURVEY Q1 fixed) instead of re-using row N_BURN_IN; the default ``"frozen"`` is the reference as it is.
     """
 
     # fed_gym/envs/multiagent.py:8-21
@@ -90,13 +92,19 @@ class BatchedSwarmEnv(object):
 
     def __init__(self, num_envs, n_locusts=None, n_agents=None, grid_size=84, max_episode_steps=128,
                  seed=0, env_id_offset=0, device=None, math_mode="fast", auto_reset=True, rasterize=True,
-                 binding="torch", tuning=0):
+                 binding="torch", tuning=0, noise="frozen"):
         """binding: "torch" = the hot calls go through torch.ops.swarm_b200.* (the C ABI as a PyTorch
         extension, csrc/torch_binding.cpp), "ctypes" = straight into the C ABI.  Same kernels either way.
-        tuning: SwarmParams.tuning (0 = automatic launch shape; anything else only changes speed, never bits)."""
+        tuning: SwarmParams.tuning (0 = automatic launch shape; anything else only changes speed, never bits).
+        noise: "frozen" (the reference: every step after a reset re-uses noise row N_BURN_IN) or "fresh" (step k of
+        an episode uses row N_BURN_IN + k, drawn by Philox inside the step kernel; SWARM_STEP_FRESH_NOISE)."""
         self.lib = nat.load()
         if binding not in ("torch", "ctypes"):
             raise ValueError("binding must be 'torch' or 'ctypes'")
+        if noise not in ("frozen", "fresh"):
+            raise ValueError("noise must be 'frozen' or 'fresh'")
+        self.noise = noise
+        self._noise_flag = nat.SWARM_STEP_FRESH_NOISE if noise == "fresh" else 0
         self.ops = nat.load_torch_ops() if binding == "torch" else None
         if not torch.cuda.is_available():
             raise nat.SwarmNativeError("BatchedSwarmEnv needs a CUDA device (sm_100a); there is no CPU path")
@@ -191,7 +199,7 @@ class BatchedSwarmEnv(object):
         rasterize = self.rasterize if rasterize is None else rasterize
         auto_reset = self.auto_reset if auto_reset is None else auto_reset
         flags = (nat.SWARM_STEP_AUTO_RESET if auto_reset else 0) | (nat.SWARM_STEP_CLIP_ACTIONS if clip else 0) | \
-                (0 if add_wind else nat.SWARM_STEP_NO_ACTION_WIND)
+                (0 if add_wind else nat.SWARM_STEP_NO_ACTION_WIND) | self._noise_flag
         if self.ops is not None:
             if actions.dtype not in (torch.float32, torch.float64):
                 raise ValueError("actions must be float32 or float64")
@@ -269,7 +277,7 @@ class BatchedSwarmEnv(object):
             io.reward, io.done = self.reward.data_ptr(), self.done_u8.data_ptr()
             self._io_host_ref = ctypes.byref(io)
         io.grid, io.positions = (self._grid_ptr, self._pos_ptr) if self.rasterize else (None, None)
-        io.flags = nat.SWARM_STEP_AUTO_RESET if self.auto_reset else 0
+        io.flags = (nat.SWARM_STEP_AUTO_RESET if self.auto_reset else 0) | self._noise_flag
         with self._ctx:
             rc = self.lib.swarm_step_host(self._params_ref, self._state_ref, self._io_host_ref, host_actions.data_ptr(),
                                           host_reward.data_ptr(), host_done.data_ptr(),
@@ -331,6 +339,19 @@ class BatchedSwarmEnv(object):
                                                   *[_ptr(b) for b in bufs], _stream(self.device)), "swarm_philox_draws")
         return InjectedDraws(*bufs, device=d)
 
+    def philox_noise_rows(self, row0, n_rows):
+        """Rows row0 .. row0+n_rows-1 of every env's CURRENT episode's noise tables, as drawn by Philox ->
+        (agent_noise (E,n_rows,A,2), particle_noise (E,n_rows,N,2)) f64, unscaled.  Row N_BURN_IN + k is what step k
+        of the episode uses with noise="fresh"; rows 0..N_BURN_IN are the ones its reset used."""
+        E, N, A, d = self.E, self.N, self.A, self.device
+        an = torch.empty(E, int(n_rows), A, 2, dtype=torch.float64, device=d)
+        pn = torch.empty(E, int(n_rows), N, 2, dtype=torch.float64, device=d)
+        with self._ctx:
+            nat.check(self.lib.swarm_philox_noise_rows(ctypes.byref(self.params), ctypes.byref(self.state_c), int(row0),
+                                                       int(n_rows), _ptr(an), _ptr(pn), _stream(self.device)),
+                      "swarm_philox_noise_rows")
+        return an, pn
+
     # ------------------------------------------------------------------ checkpointing
     def state_dict(self):
         keys = ("x", "xa", "noise_x", "noise_a", "elapsed", "episode")
@@ -349,6 +370,9 @@ class SwarmEnv(object):
     (multiagent.py:48-56), so ``SwarmEnv(seed=s)`` sees the very same random numbers as the
     reference env -- they are injected into the device reset.  The raw class has no TimeLimit;
     ``make('Swarm-v0')`` adds the 128-step limit the gym registry attaches.
+    With ``fresh_noise=True`` it is the reference with SURVEY Q1 fixed: ``self.t`` advances after every step, so
+    step k of an episode uses row N_BURN_IN + k of the 138-row noise tables (and step 129 without a TimeLimit
+    raises IndexError, as the fixed reference would).
     """
     N_LOCUSTS = 80
     N_AGENTS = 10
@@ -361,20 +385,23 @@ class SwarmEnv(object):
     dt = 0.05
     N_BURN_IN = 10
 
-    def __init__(self, seed=None, max_episode_steps=0, math_mode="fast", device=None):
+    def __init__(self, seed=None, max_episode_steps=0, math_mode="fast", device=None, fresh_noise=False):
         self.n_seed = seed
         self.states = None
         self.t = 0
         self._max_episode_steps = max_episode_steps
         self._math_mode = math_mode
         self._device = device
+        self._fresh = bool(fresh_noise)
+        self._tables = None              # fresh noise: the episode's (138,1,A,2) / (138,1,N,2) noise tables on the device
         self._env = None
 
     def _backend(self):
         if self._env is None or self._env.N != self.N_LOCUSTS or self._env.A != self.N_AGENTS:
             self._env = BatchedSwarmEnv(1, n_locusts=self.N_LOCUSTS, n_agents=self.N_AGENTS, grid_size=84,
                                         max_episode_steps=self._max_episode_steps, device=self._device,
-                                        math_mode=self._math_mode, auto_reset=False, rasterize=False)
+                                        math_mode=self._math_mode, auto_reset=False, rasterize=False,
+                                        noise="fresh" if self._fresh else "frozen")
             for k in ("NOISE", "GRAVITY", "WIND_SPEED", "F", "L", "dt"):
                 setattr(self._env.params, {"NOISE": "noise", "GRAVITY": "gravity", "WIND_SPEED": "wind",
                                            "F": "F", "L": "L", "dt": "dt"}[k], float(getattr(self, k)))
@@ -412,6 +439,8 @@ class SwarmEnv(object):
         pn = np.random.normal(size=(128 + nb, N, 2))
         draws = InjectedDraws(x0[None], xa0[None], burn[None], an[None, :nb + 1], pn[None, :nb + 1], env.device)
         env.reset(draws=draws)
+        if self._fresh:                   # every row is read, one per step: the step gets it as its override
+            self._tables = (torch.as_tensor(an[:, None]).to(env.device), torch.as_tensor(pn[:, None]).to(env.device))
         self.t = nb                       # multiagent.py:59-61 leaves t == N_BURN_IN forever (Q1)
         self.states = None
         return self._sync_out()
@@ -421,7 +450,14 @@ class SwarmEnv(object):
             raise TypeError("cannot unpack non-iterable NoneType object")   # multiagent.py:31 before reset
         env = self._env
         a = torch.as_tensor(np.ascontiguousarray(v_action, dtype=np.float64)[None]).to(env.device)
-        _, reward, done, _ = env.step(a, add_wind=bool(add_wind))      # multiagent.py:35-36
+        if self._fresh:
+            an, pn = self._tables
+            if self.t >= an.shape[0]:     # multiagent.py:38 indexes agent_noise[self.t] first
+                raise IndexError("index %d is out of bounds for axis 0 with size %d" % (self.t, an.shape[0]))
+            _, reward, done, _ = env.step(a, noise_a=an[self.t], noise_x=pn[self.t], add_wind=bool(add_wind))
+            self.t += 1
+        else:
+            _, reward, done, _ = env.step(a, add_wind=bool(add_wind))      # multiagent.py:35-36
         self._sync_out()
         return self.states, np.float64(reward[0].item()), np.bool_(done[0].item()), {}
 

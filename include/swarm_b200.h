@@ -70,7 +70,8 @@ typedef struct SwarmParams {
 
 /* The env batch's persistent state (SwarmEnv.states / .agent_noise[t] / .particle_noise[t] /
  * TimeLimit._elapsed_steps).  noise_* hold the FROZEN row N_BURN_IN that every post-reset step
- * re-uses because SwarmEnv._step never advances self.t (multiagent.py:38,40; SURVEY Q1). */
+ * re-uses because SwarmEnv._step never advances self.t (multiagent.py:38,40; SURVEY Q1).  They are
+ * written at every reset; a step with SWARM_STEP_FRESH_NOISE does not read them. */
 typedef struct SwarmState {
     double* x;                  /* (E,N,2) */
     double* xa;                 /* (E,A,2) */
@@ -104,11 +105,17 @@ typedef struct SwarmInjectedDraws {
                                        * actions are used as they are (burn-in steps of an auto-reset still
                                        * add the wind, like the reference's _reset -> step)                */
 #define SWARM_STEP_INKERNEL_RASTER 16u /* never use the follower kernel (see swarm_step); same results     */
+#define SWARM_STEP_FRESH_NOISE  32u /* the reference with SURVEY Q1 fixed (self.t advances): env e's step uses
+                                     * Philox row n_burn_in + elapsed[e] of noise streams 3 and 4 of its current
+                                     * episode (episode word st->episode[e] - 1), drawn inside the step kernel,
+                                     * instead of the frozen row st->noise_*.  The first step after a Philox
+                                     * reset is the same in both modes.  io->noise_a / io->noise_x still
+                                     * override their own row when given.  Without the flag nothing changes. */
 
 typedef struct SwarmStepIO {
     float* actions_f32;         /* (E,A,2) PAAC shared_actions dtype (paac.py:269); in/out if CLIP  */
     double* actions_f64;        /* (E,A,2) gym-facade dtype; used when SWARM_STEP_ACTIONS_F64        */
-    const double* noise_a;      /* nullable (E,A,2): per-step override of the frozen row            */
+    const double* noise_a;      /* nullable (E,A,2): per-step override of the frozen (or fresh) row */
     const double* noise_x;      /* nullable (E,N,2)                                                 */
     float* reward;              /* (E)  = -mean_j |v_j|^2                                           */
     uint8_t* done;              /* (E)  reward >= 0 || ++elapsed >= max_episode_steps               */
@@ -217,6 +224,14 @@ int swarm_clip_actions(float* actions, int64_t n_rows, float max_norm, swarm_str
 int swarm_philox_draws(const SwarmParams* p, const SwarmState* st, double* x0, double* xa0,
                        double* burn_actions, double* agent_noise, double* particle_noise,
                        swarm_stream_t stream);
+
+/* Materialise rows row0 .. row0+n_rows-1 of the noise streams 3 and 4 of every env's CURRENT
+ * episode (episode word st->episode[e] - 1, i.e. the episode the last reset started): the rows a
+ * SWARM_STEP_FRESH_NOISE step draws (row n_burn_in + elapsed) and the reset's own rows 0..n_burn_in,
+ * bit for bit.  agent_noise (E,n_rows,A,2), particle_noise (E,n_rows,N,2), unscaled N(0,1).
+ * SWARM_ERR_NULL / SWARM_ERR_SIZE (row0 < 0, n_rows <= 0) are returned before any CUDA call. */
+int swarm_philox_noise_rows(const SwarmParams* p, const SwarmState* st, int32_t row0, int32_t n_rows,
+                            double* agent_noise, double* particle_noise, swarm_stream_t stream);
 
 /* Raw Philox4x32-10 blocks for known-answer tests: out[i] = philox(ctr[i], key[i]). */
 int swarm_philox_raw(const uint32_t* ctr /*(n,4)*/, const uint32_t* key /*(n,2)*/,

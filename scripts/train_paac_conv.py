@@ -5,7 +5,7 @@
     torchrun --nproc-per-node 8 scripts/train_paac_conv.py -ec 8192 --clip_norm=1    # config 5: env batch sharded
 
 Flag names and defaults are the reference's; additions: --n_locusts, --max_updates, --no_cuda_graph,
---reward_indexing, --mask_terminals.  '-d/--device' accepts the reference's '/gpu:0' spelling.
+--reward_indexing, --mask_terminals, --fresh_noise.  '-d/--device' accepts the reference's '/gpu:0' spelling.
 """
 import argparse
 import copy
@@ -34,7 +34,8 @@ def get_network_and_environment_creator(args, random_seed=3):
     import golds_rl_gym_b200 as pkg
     ec = pkg.submodule("agents.paac.environment_creator")
     pv = pkg.submodule("agents.paac.policy_v_network")
-    env_creator = ec.SwarmEnvironmentCreator(n_locusts=args.n_locusts, grid_size=args.height)
+    env_creator = ec.SwarmEnvironmentCreator(n_locusts=args.n_locusts, grid_size=args.height,
+                                             noise="fresh" if getattr(args, "fresh_noise", False) else "frozen")
     args.num_actions = env_creator.num_actions
     args.random_seed = random_seed
     network_conf = {
@@ -94,6 +95,8 @@ def get_arg_parser():
     parser.add_argument('--no_cuda_graph', action='store_true')
     parser.add_argument('--reward_indexing', default='reference', choices=['reference', 'per_agent'])
     parser.add_argument('--mask_terminals', action='store_true')
+    parser.add_argument('--fresh_noise', action='store_true',
+                        help="advance the env noise row every step (SURVEY Q1 fixed); default: the reference's frozen row")
     parser.add_argument('--eval_every', default=30.0, type=float,
                         help="seconds between evaluation episodes on Swarm-eval-v0 (policy_monitor.py); 0 = off")
     parser.add_argument('--net_precision', default='fp32', choices=['fp32', 'tf32', 'bf16'],
@@ -133,7 +136,7 @@ def main(args):
         sp = pkg.submodule("agents.state_processors")
         monitor = pm.SwarmPolicyMonitor(global_policy_net=learner.network,
                                         state_processor=sp.SwarmStateProcessor(grid_size=args.height),
-                                        out_dir=args.debugging_folder)
+                                        out_dir=args.debugging_folder, fresh_noise=args.fresh_noise)
     fps = learner.train(max_updates=args.max_updates, monitor=monitor, eval_every=args.eval_every,
                         summary_dir=args.debugging_folder)     # scalars: global_norm, rl/reward (summaries.jsonl)
     if int(os.environ.get("RANK", "0")) == 0:
