@@ -597,6 +597,10 @@ size_t step_smem(const SwarmParams* p, int raster, int n_stage, int mode) {
     return smem_bytes(p->n_locusts, p->n_agents, p->grid_size, n_stage, true, raster, force_sym(mode));
 }
 
+// The kernels read and write a grid cell's two channels as one float2: the grid must be 8-byte aligned.  (Any further
+// alignment is optional: 16 bytes enables the TMA zero fill, the filler warp and 16-byte stores.)
+bool grid_aligned(const void* grid) { return (reinterpret_cast<uintptr_t>(grid) & 7) == 0; }
+
 int validate(const SwarmParams* p, int min_agents = 1) {
     if (!p) return SWARM_ERR_NULL;
     if (p->n_envs < 1 || p->n_locusts < 1 || p->n_locusts > kMaxLocusts) return SWARM_ERR_SIZE;
@@ -914,6 +918,7 @@ int plan_step(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io,
     if (!io->reward || !io->done) return SWARM_ERR_NULL;
     if ((io->flags & SWARM_STEP_ACTIONS_F64) ? !io->actions_f64 : !io->actions_f32) return SWARM_ERR_NULL;
     if ((io->grid != nullptr) != (io->positions != nullptr)) return SWARM_ERR_FLAGS;
+    if (!grid_aligned(io->grid)) return SWARM_ERR_FLAGS;
     if (io->flags & ~(SWARM_STEP_AUTO_RESET | SWARM_STEP_CLIP_ACTIONS | SWARM_STEP_ACTIONS_F64 | SWARM_STEP_NO_ACTION_WIND |
                       SWARM_STEP_INKERNEL_RASTER | SWARM_STEP_FRESH_NOISE))
         return SWARM_ERR_FLAGS;
@@ -1253,6 +1258,7 @@ int swarm_rasterize(const SwarmParams* p, const double* x, const double* xa, flo
     if (rc) return rc;
     if (!x || !grid) return SWARM_ERR_NULL;
     if (p->n_agents > 0 && (!xa || !positions)) return SWARM_ERR_NULL;
+    if (!grid_aligned(grid)) return SWARM_ERR_FLAGS;
     const KP kp = make_kp(p);
     const size_t smem = smem_bytes(kp.N, kp.A, kp.G, 0, false, 1, 0);
     const int nt = (kp.N + kp.A) <= 128 ? 64 : 128;
@@ -1271,6 +1277,7 @@ int swarm_expand_obs(const SwarmParams* p, const float* grid, const uint8_t* pos
     int rc = validate(p);
     if (rc) return rc;
     if (!grid || !positions || !expanded) return SWARM_ERR_NULL;
+    if (!grid_aligned(grid)) return SWARM_ERR_FLAGS;
     const int cells = p->grid_size * p->grid_size;
     dim3 g((cells + 255) / 256, (unsigned)(p->n_envs * p->n_agents));
     if (g.y > 65535u) {

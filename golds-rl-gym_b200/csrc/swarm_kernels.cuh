@@ -1009,16 +1009,19 @@ __device__ __forceinline__ double edge_at(int i, double lo, double hi, double st
     return i >= G ? hi : __dadd_rn(__dmul_rn((double)i, step), lo);
 }
 
-// The bin is guessed with a reciprocal multiply.  The guess q = (p - lo) / step is within ~1e-13 of the real
-// position of p between numpy's edges (each edge is within 2 ulp of lo + i*step, the subtraction and the
-// multiply add a few ulp more), so a guess whose fractional part is further than 1e-9 from 0 and 1 is certain;
-// anything else -- points on or next to an edge, outside [lo, hi) -- is settled against the exact edges.
+// The bin is guessed with a reciprocal multiply.  Each of numpy's edges is within an ulp of max(|lo|, |hi|) of
+// lo + i*step (the rounding of fl(i*step) + lo), and the subtraction and the multiply of the guess
+// q = (p - lo) / step add a few ulp of the bin width, so q is within slack = 1e-9 + 16 max(|lo|, |hi|) 2^-52 / step
+// bins of the real position of p between numpy's edges: a guess whose fractional part is further than that from
+// 0 and 1 is certain.  Anything else -- points on or next to an edge, outside [lo, hi) -- is settled against the
+// exact edges.  (The magnitude term matters far from the origin: at |lo| ~ 1e6 one ulp is already ~3e-9 bins.)
 __device__ __forceinline__ int count_le(double p, double lo, double hi, double step, double inv_step, int G) {
     if (p == lo) return 1;                       // e[0] = lo exactly (the grounded locusts' y = 0 lands here)
     const double q = (p - lo) * inv_step;
     const double fl = floor(q);
     const double fr = q - fl;
-    if (q > 0.0 && q < (double)G && fr > 1e-9 && fr < 1.0 - 1e-9) return (int)fl + 1;
+    const double slack = 1e-9 + 16.0 * fmax(fabs(lo), fabs(hi)) * 2.220446049250313e-16 * inv_step;
+    if (q > 0.0 && q < (double)G && fr > slack && fr < 1.0 - slack) return (int)fl + 1;
     if (!(p == p)) return G + 1;                 // NaN sorts last
     int g = q < -1.0 ? -1 : (q > (double)G ? G : (int)fl);
     while (g < G && edge_at(g + 1, lo, hi, step, G) <= p) ++g;
@@ -1026,9 +1029,10 @@ __device__ __forceinline__ int count_le(double p, double lo, double hi, double s
     return g + 1;                                // #{i in [0,G] : e[i] <= p}
 }
 
-// Streaming zero fill of one env's (G,G,2) f32 grid by n threads (evict-first stores).
+// Streaming zero fill of one env's (G,G,2) f32 grid by n threads (evict-first stores): 16-byte stores where the grid
+// is 16-byte aligned, 8-byte ones otherwise (a grid only needs 8-byte alignment, e.g. a slot of a caller's buffer).
 __device__ __forceinline__ void raster_zero_fill(float* __restrict__ grid_e, int cells, int tid, int n) {
-    if ((cells & 1) == 0) {
+    if ((cells & 1) == 0 && (reinterpret_cast<uintptr_t>(grid_e) & 15) == 0) {
         float4* g4 = reinterpret_cast<float4*>(grid_e);
         const float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
         for (int i = tid; i < cells / 2; i += n) __stcs(g4 + i, z);

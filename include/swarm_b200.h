@@ -15,6 +15,7 @@
  *   - return value: 0 = ok, negative = SwarmStatus error (swarm_strerror);
  *   - layouts are C order.  x:(E,N,2) f64, xa:(E,A,2) f64, actions:(E,A,2),
  *     grid:(E,G,G,2) f32 indexed [env][x_bin][y_bin][channel], positions:(E,A,2) u8.
+ *     A grid must be 8-byte aligned (SWARM_ERR_FLAGS otherwise); 16-byte alignment is faster.
  *
  * Arithmetic: the O(N) integrator state is FP64 like the reference's numpy arrays
  * (fed_gym/envs/multiagent.py:30-86); the O(N^2) pair forces (multiagent.py:88-115) are FP32.

@@ -6,28 +6,30 @@ edges, searchsorted).  This test restates the acceptance rule in NumPy, arithmet
 checks the two properties the kernel relies on, on random and adversarial states:
   (1) soundness: whenever the rule accepts an env, the speculative x counts equal numpy's own (oracle) for EVERY point;
   (2) usefulness: random states are practically always accepted, states with a point on / next to an edge never are.
-The CUDA path itself is compared with the oracle in tests/test_gpu_parity.py
-(test_rasterizer_verified_parallel_mean_next_to_edges and every fused-rasteriser test).
+The CUDA path itself is compared with the oracle on such states in tests/test_gpu_parity.py
+(test_rasterizer_verified_parallel_mean_next_to_edges: the standalone rasteriser behind observe()) and in
+tests/test_gpu_raster_edges.py (the rasteriser inside the step, in every launch shape; it uses spec_counts to prove that
+its states take the branch each of them targets).
 """
 import numpy as np
 
 from oracle import swarm_oracle as so
 
 G, W = 84, so.BOX_WIDTH
-INV_X = G / W                      # KP.inv_x (make_kp)
 EPS = 2.220446049250313e-16
 
 
-def spec_counts(x, xa, order):
-    """(#edges <= p for every point, accepted?) the way env_raster's speculative phase computes them.  `order` permutes the
-    points before a pairwise sum: any summation order stands in for the kernel's warp-shuffle tree."""
+def spec_counts(x, xa, order, G=G):
+    """(#edges <= p for every point, accepted?) the way env_raster's speculative phase computes them for a G x G grid.
+    `order` permutes the points before a pairwise sum: any summation order stands in for the kernel's warp-shuffle tree."""
+    inv_x = G / W                                        # KP.inv_x (make_kp)
     px = np.concatenate([x[:, 0], xa[:, 0]])
     P = px.size
     tot = float(np.sum(px[order]))                       # pairwise, not sequential
     xmax = float(np.max(np.abs(px)))
     lo_s = tot * (1.0 / P) - W / 2.0
-    tol = 1e-9 + 2.0 * ((P + 16) * xmax + 32.0 * (W / 2.0)) * EPS * INV_X
-    qs = (px - lo_s) * INV_X
+    tol = 1e-9 + 2.0 * ((P + 16) * xmax + 32.0 * (W / 2.0)) * EPS * inv_x
+    qs = (px - lo_s) * inv_x
     fl = np.floor(qs)
     fr = qs - fl
     ok = bool(tol < 0.25) and bool(np.all((fr > tol) & (fr < 1.0 - tol)))
