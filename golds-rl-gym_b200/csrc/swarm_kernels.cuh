@@ -277,9 +277,12 @@ __device__ __forceinline__ double div_by_const(const double a, const double b, c
 // in log2(e)-scaled coordinates:  w = (F 2^(-r/L) - 2^(-r)) / (r + c eps).
 // Positions arrive as FP32 hi/lo pairs of the FP64 state, so the difference
 //   d = (hi_i - hi_j) + (lo_i - lo_j)
-// carries ~2^-24 RELATIVE error however close the two particles are (plain FP32 positions lose
-// the direction of close pairs, where s/(r+eps) is steepest).  Coincident points (and the self
-// pair of the ordered loop) have d = 0 exactly and contribute exactly 0.
+// carries ~2^-24 RELATIVE error of the difference of the two REPRESENTED points however close they
+// are (plain FP32 positions lose the direction of close pairs, where s/(r+eps) is steepest).  hi + lo
+// itself represents a coordinate only to ~2^-48 |x|, so d is also off by up to ~2^-47 (|x_i| + |x_j|)
+// absolutely: nothing near the origin, where TimeLimit episodes stay, but up to ~6e-6 in a close
+// pair's force at |x| ~ 1e4 (envelope: DESIGN 3.1).  Coincident points (and the
+// self pair of the ordered loop) have d = 0 exactly and contribute exactly 0.
 // 1 / (r + eps) from rinv ~ 1/r without a third trip to the XU pipe (the busiest pipe of the pair loop):
 //   1/(r + eps) = rinv / (1 + eps rinv) = rinv - (eps rinv) rinv + O((eps/r)^2),
 // one FMUL + one FFMA.  The dropped term is below 2^-24 -- the rounding of the result -- when eps rinv <= 2^-12, i.e. for
