@@ -16,7 +16,7 @@ _REPO = os.path.dirname(_PKG_DIR)
 LIB_PATH = os.path.join(_PKG_DIR, "libswarm_b200.so")
 # experiments only (scripts/build_variants.py): load another build of the same ABI through the ctypes binding
 _LIB_OVERRIDE = os.environ.get("SWARM_B200_LIB")
-SOURCES = [os.path.join(_CSRC, f) for f in ("swarm_b200.cu", "swarm_kernels.cuh", "swarm_philox.cuh")]
+SOURCES = [os.path.join(_CSRC, f) for f in ("swarm_b200.cu", "swarm_kernels.cuh", "swarm_cluster.cuh", "swarm_philox.cuh")]
 HEADER = os.path.join(_REPO, "include", "swarm_b200.h")
 
 NVCC_FLAGS = ["-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo",
@@ -33,8 +33,20 @@ SWARM_STEP_ACTIONS_F64 = 4
 SWARM_STEP_NO_ACTION_WIND = 8
 SWARM_STEP_INKERNEL_RASTER = 16
 SWARM_STEP_FRESH_NOISE = 32
-# SwarmParams.tuning: bits 4-5 = rasteriser placement (0 automatic); every other bit must be 0
+# SwarmParams.tuning: bits 4-5 = rasteriser placement (0 automatic); bits 8-12 = the cluster layout (0 one CTA per env,
+# 1..16 a thread-block cluster of K CTAs per env, 31 the library picks K; 512 < N <= 8192); every other bit must be 0
 TUNE_RASTER_FOLLOW, TUNE_RASTER_WARPS, TUNE_RASTER_SELF = 1 << 4, 2 << 4, 3 << 4
+TUNE_CLUSTER_SHIFT = 8
+TUNE_CLUSTER_MASK = 31 << TUNE_CLUSTER_SHIFT
+TUNE_CLUSTER_AUTO = 31 << TUNE_CLUSTER_SHIFT
+CLUSTER_MAX_K = 16
+CLUSTER_MIN_LOCUSTS, CLUSTER_MAX_LOCUSTS = 513, 8192
+MAX_LOCUSTS_ONE_CTA = 2048
+
+
+def tune_cluster(k):
+    """The tuning bits of the cluster layout: k CTAs per env, or None for the library's choice."""
+    return TUNE_CLUSTER_AUTO if k is None else (int(k) & 31) << TUNE_CLUSTER_SHIFT
 
 
 class SwarmParams(ctypes.Structure):

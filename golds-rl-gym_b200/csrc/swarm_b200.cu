@@ -13,6 +13,7 @@
 #include <utility>
 
 #include "swarm_kernels.cuh"
+#include "swarm_cluster.cuh"
 
 using namespace swarm;
 
@@ -548,6 +549,279 @@ __global__ void k_philox_raw(const uint4* __restrict__ ctr, const uint2* __restr
     if (i < n) out[i] = philox4x32_10(ctr[i], key[i]);
 }
 
+// ---- CLUSTER layout (swarm_cluster.cuh, DESIGN 3.4): env blockIdx.x / K on the K CTAs of one thread-block cluster.
+// nf = the one-CTA kernel's force threads (the virtual mapping); launched with cudaLaunchKernelEx and a cluster
+// dimension.
+
+// Noise row r of the env's locust j: r < 0 the step proper's row (override, frozen or fresh), else reset row r.
+struct ClNoise {
+    const KP& kp;
+    const SwarmState& st;
+    const SwarmStepIO* io;
+    const SwarmInjectedDraws& dr;
+    DrawCtx fresh_d, reset_d;
+    uint32_t fresh_row;
+    int e;
+    bool inj;
+    __device__ __forceinline__ double2 operator()(const int r, const int j) const {
+        if (r < 0) {
+            if (kp.fresh && !io->noise_x) return draw_normal2(fresh_d, STREAM_NOISE_X, fresh_row, (uint32_t)j);
+            return reinterpret_cast<const double2*>(io->noise_x ? io->noise_x : st.noise_x)[(size_t)e * kp.N + j];
+        }
+        return inj ? reinterpret_cast<const double2*>(dr.particle_noise)[((size_t)e * (kp.n_burn + 1) + r) * kp.N + j]
+                   : draw_normal2(reset_d, STREAM_NOISE_X, (uint32_t)r, (uint32_t)j);
+    }
+};
+
+// reset_begin of the cluster: every CTA draws its own targets' initial positions (into global memory) and all agents'
+__device__ __forceinline__ void cl_reset_begin(const CSmem& sm, const KP& kp, const CMap& m, const int e, double2* xe,
+                                               const ClNoise& nz) {
+    const int N = kp.N, A = kp.A, tid = (int)threadIdx.x;
+    if (m.active) {
+        for (int j = m.vtid; j < N; j += m.nf)
+            xe[j] = nz.inj ? reinterpret_cast<const double2*>(nz.dr.x0)[(size_t)e * N + j] : draw_uniform2(nz.reset_d, STREAM_X0, j);
+    }
+    if (tid < A)
+        sm.as[tid] = nz.inj ? reinterpret_cast<const double2*>(nz.dr.xa0)[(size_t)e * A + tid] : draw_uniform2(nz.reset_d, STREAM_XA0, tid);
+}
+
+// reset_row of the cluster: agent noise row r and burn-in action r (every CTA); for r == n_burn the frozen rows are
+// stored (own targets; rank 0 the agents') and true is returned
+__device__ __forceinline__ bool cl_reset_row(const CSmem& sm, const KP& kp, const CMap& m, const int e, const int r,
+                                             const SwarmState& st, const ClNoise& nz) {
+    const int N = kp.N, A = kp.A, tid = (int)threadIdx.x, rows = kp.n_burn + 1;
+    const bool last = r >= kp.n_burn;
+    if (tid < A) {
+        const double2 z = nz.inj ? reinterpret_cast<const double2*>(nz.dr.agent_noise)[((size_t)e * rows + r) * A + tid]
+                                 : draw_normal2(nz.reset_d, STREAM_NOISE_A, r, tid);
+        sm.an[tid] = z;
+        if (last) {
+            if (m.rank == 0) reinterpret_cast<double2*>(st.noise_a)[(size_t)e * A + tid] = z;
+        } else {
+            sm.act[tid] = nz.inj ? reinterpret_cast<const double2*>(nz.dr.burn_actions)[((size_t)e * kp.n_burn + r) * A + tid]
+                                 : draw_normal2(nz.reset_d, STREAM_BURN, r, tid);
+        }
+    }
+    if (last && m.active)
+        for (int j = m.vtid; j < N; j += m.nf) reinterpret_cast<double2*>(st.noise_x)[(size_t)e * N + j] = nz(r, j);
+    return last;
+}
+
+// One SwarmEnv._step of the cluster's env up to the new positions in pn (nothing written yet); v_out: this env's.
+template <int MODE, bool PRECISE>
+__device__ __forceinline__ void cl_step_forces(const CSmem& sm, const KP& kp, const CMap& m, const double2* xe,
+                                               const double2* xae, const double wind_a, const int r, const ClNoise& nz,
+                                               float* v_out, double2 (&pn)[ModeT<MODE>::T]) {
+    constexpr int T = ModeT<MODE>::T;
+    cl_stage<true>(sm, kp, xe, xae, wind_a);
+    if (m.active) {
+        float vx[T], vy[T];
+        cl_forces<MODE, PRECISE>(sm, kp, m, vx, vy);
+#pragma unroll
+        for (int t = 0; t < T; ++t) {
+            const int j = m.vtid + t * m.nf;
+            double2 p = make_double2(0.0, 0.0);
+            if (j < kp.N) {
+                if (v_out) reinterpret_cast<float2*>(v_out)[j] = make_float2(vx[t], vy[t]);
+                p = __ldcg(xe + j);
+                move_particle(p, make_double2((double)vx[t], (double)vy[t]), nz(r, j), kp.dt, kp.sigma);
+            }
+            pn[t] = p;
+        }
+    }
+}
+
+template <int T>
+__device__ __forceinline__ void cl_store(const KP& kp, const CMap& m, double2* xe, const double2 (&pn)[T]) {
+    if (m.active) {
+#pragma unroll
+        for (int t = 0; t < T; ++t) {
+            const int j = m.vtid + t * m.nf;
+            if (j < kp.N) xe[j] = pn[t];
+        }
+    }
+}
+
+// SwarmEnv._step + TimeLimit + auto-reset + process_state (k_step's contract) for the cluster layout.
+template <int MODE, bool PRECISE>
+__global__ void __maxnreg__(64) k_step_cluster(const KP kp, const SwarmState st, const SwarmStepIO io,
+                                               const SwarmInjectedDraws dr, const int has_draws, const int nf) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    constexpr int T = ModeT<MODE>::T;
+    const int N = kp.N, A = kp.A, tid = (int)threadIdx.x;
+    const CMap m = cl_map(nf);
+    const CSmem sm = cl_carve(smem_raw, N, A, kp.G, m.K, true);
+    const int e = (int)blockIdx.x / m.K;
+    const bool lead = m.rank == 0;
+    double2* xe = reinterpret_cast<double2*>(st.x) + (size_t)e * N;
+    double2* xae = reinterpret_cast<double2*>(st.xa) + (size_t)e * A;
+    const int elapsed0 = st.elapsed[e];
+    const uint32_t episode0 = st.episode[e];
+    ClNoise nz{kp, st, &io, dr, {}, {}, 0u, e, has_draws != 0};
+    nz.fresh_d.key = kp.key;
+    nz.fresh_d.env = kp.env_off + (uint32_t)e;
+    nz.fresh_d.episode = episode0 - 1u;      // the episode the last reset started
+    nz.fresh_row = (uint32_t)kp.n_burn + (uint32_t)elapsed0;
+    nz.reset_d = nz.fresh_d;
+    nz.reset_d.episode = episode0;
+    // the agents, in every CTA: state, noise row, actions (HBM dtype -> FP64, optional clip; rank 0 writes the clipped
+    // actions back once every CTA has read them)
+    bool clipped = false;
+    double2 aclip = make_double2(0.0, 0.0);
+    if (tid < A) {
+        const int k = tid;
+        sm.as[k] = xae[k];
+        if (kp.fresh && !io.noise_a) sm.an[k] = draw_normal2(nz.fresh_d, STREAM_NOISE_A, nz.fresh_row, (uint32_t)k);
+        else sm.an[k] = reinterpret_cast<const double2*>(io.noise_a ? io.noise_a : st.noise_a)[(size_t)e * A + k];
+        double2 a;
+        if (io.flags & SWARM_STEP_ACTIONS_F64) {
+            a = reinterpret_cast<const double2*>(io.actions_f64)[(size_t)e * A + k];
+        } else {
+            const float2 f = reinterpret_cast<const float2*>(io.actions_f32)[(size_t)e * A + k];
+            a = make_double2((double)f.x, (double)f.y);
+        }
+        if (io.flags & SWARM_STEP_CLIP_ACTIONS) {
+            if (io.flags & SWARM_STEP_ACTIONS_F64) {
+                const double d = sqrt(__dadd_rn(__dmul_rn(a.x, a.x), __dmul_rn(a.y, a.y)));
+                if (d >= 1.0) {
+                    a.x = a.x / d; a.y = a.y / d;
+                    clipped = true;
+                }
+            } else {
+                const float fx = (float)a.x, fy = (float)a.y;
+                const float d = __fsqrt_rn(__fadd_rn(__fmul_rn(fx, fx), __fmul_rn(fy, fy)));
+                if (d >= 1.0f) {
+                    a = make_double2((double)__fdiv_rn(fx, d), (double)__fdiv_rn(fy, d));
+                    clipped = true;
+                }
+            }
+        }
+        sm.act[k] = a;
+        aclip = a;
+    }
+    float* v_out = io.v_out ? io.v_out + (size_t)e * N * 2 : nullptr;
+    int elapsed = 0;
+    for (int r = -1;;) {
+        double2 pn[T];
+        cl_step_forces<MODE, PRECISE>(sm, kp, m, xe, xae, (r < 0 && !kp.wind_step) ? 0.0 : kp.wind, r, nz, v_out, pn);
+        cluster_sync();     // every CTA has read the old state (and its actions): the new one may be written
+        cl_store(kp, m, xe, pn);
+        const double reward = cl_reward(sm, kp, m);
+        if (r < 0) {
+            elapsed = elapsed0 + 1;
+            const bool done = (reward >= 0.0) || (kp.max_steps > 0 && elapsed >= kp.max_steps);
+            if (lead && tid == 0) {
+                io.reward[e] = (float)reward;
+                io.done[e] = done ? 1 : 0;
+            }
+            if (!(done && (io.flags & SWARM_STEP_AUTO_RESET))) break;      // cluster-uniform
+            cl_reset_begin(sm, kp, m, e, xe, nz);
+            v_out = nullptr;
+            elapsed = 0;
+        }
+        if (cl_reset_row(sm, kp, m, e, ++r, st, nz)) {
+            if (lead && tid == 0) st.episode[e] = episode0 + 1;
+            break;
+        }
+        cluster_sync();     // the new state is in memory before any CTA reads it again
+    }
+    if (lead) {
+        if (tid == 0) st.elapsed[e] = elapsed;
+        if (tid < A) {
+            xae[tid] = sm.as[tid];
+            if (clipped) {
+                const double2 a = aclip;
+                if (io.flags & SWARM_STEP_ACTIONS_F64) reinterpret_cast<double2*>(io.actions_f64)[(size_t)e * A + tid] = a;
+                else reinterpret_cast<float2*>(io.actions_f32)[(size_t)e * A + tid] = make_float2((float)a.x, (float)a.y);
+            }
+        }
+    }
+    if (io.grid)
+        cl_raster<T, false>(sm, kp, m, xe, xae, io.grid + (size_t)e * kp.G * kp.G * 2, io.positions + (size_t)e * A * 2, nullptr);
+    cluster_sync();         // no CTA leaves while a peer may still read its shared memory
+}
+
+// SwarmEnv._reset for the masked envs, cluster layout.
+template <int MODE, bool PRECISE>
+__global__ void __maxnreg__(64) k_reset_cluster(const KP kp, const SwarmState st, const uint8_t* __restrict__ mask,
+                                                const SwarmInjectedDraws dr, const int has_draws, const int nf) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    constexpr int T = ModeT<MODE>::T;
+    const int N = kp.N, A = kp.A, tid = (int)threadIdx.x;
+    const CMap m = cl_map(nf);
+    const int e = (int)blockIdx.x / m.K;
+    if (mask && !mask[e]) return;            // the whole cluster
+    const CSmem sm = cl_carve(smem_raw, N, A, kp.G, m.K, true);
+    double2* xe = reinterpret_cast<double2*>(st.x) + (size_t)e * N;
+    double2* xae = reinterpret_cast<double2*>(st.xa) + (size_t)e * A;
+    const uint32_t ep = st.episode[e];
+    ClNoise nz{kp, st, nullptr, dr, {}, {}, 0u, e, has_draws != 0};
+    nz.reset_d.key = kp.key;
+    nz.reset_d.env = kp.env_off + (uint32_t)e;
+    nz.reset_d.episode = ep;
+    cl_reset_begin(sm, kp, m, e, xe, nz);
+    for (int r = 0; !cl_reset_row(sm, kp, m, e, r, st, nz); ++r) {
+        cluster_sync();     // the state is in memory before any CTA reads it
+        double2 pn[T];
+        cl_step_forces<MODE, PRECISE>(sm, kp, m, xe, xae, kp.wind, r, nz, nullptr, pn);
+        cluster_sync();     // every CTA has read the old state
+        cl_store(kp, m, xe, pn);
+    }
+    cluster_sync();         // every CTA has read the episode counter
+    if (m.rank == 0) {
+        if (tid == 0) {
+            st.elapsed[e] = 0;
+            st.episode[e] = ep + 1;
+        }
+        if (tid < A) xae[tid] = sm.as[tid];
+    }
+}
+
+// SwarmEnv.v_calculate for the batch, cluster layout.
+template <int MODE, bool PRECISE>
+__global__ void __maxnreg__(64) k_forces_cluster(const KP kp, const double* __restrict__ x, const double* __restrict__ xa,
+                                                 float* __restrict__ v, float* __restrict__ reward, const int nf) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    constexpr int T = ModeT<MODE>::T;
+    const CMap m = cl_map(nf);
+    const CSmem sm = cl_carve(smem_raw, kp.N, kp.A, kp.G, m.K, true);
+    const int e = (int)blockIdx.x / m.K;
+    const double2* xe = reinterpret_cast<const double2*>(x) + (size_t)e * kp.N;
+    const double2* xae = reinterpret_cast<const double2*>(xa) + (size_t)e * kp.A;
+    cl_stage<false>(sm, kp, xe, xae, 0.0);
+    if (m.active) {
+        float vx[T], vy[T];
+        cl_forces<MODE, PRECISE>(sm, kp, m, vx, vy);
+        if (v) {
+#pragma unroll
+            for (int t = 0; t < T; ++t) {
+                const int j = m.vtid + t * m.nf;
+                if (j < kp.N) reinterpret_cast<float2*>(v)[(size_t)e * kp.N + j] = make_float2(vx[t], vy[t]);
+            }
+        }
+    }
+    cluster_sync();         // every energy slot is in place
+    const double r = cl_reward(sm, kp, m);
+    if (reward && m.rank == 0 && threadIdx.x == 0) reward[e] = (float)r;
+    cluster_sync();
+}
+
+// SwarmStateProcessor.process_state for the batch, cluster layout (k_rasterize's contract).
+template <int T, bool EXACT>
+__global__ void __launch_bounds__(1024) k_rasterize_cluster(const KP kp, const double* __restrict__ x,
+                                                            const double* __restrict__ xa, float* __restrict__ grid,
+                                                            uint8_t* __restrict__ positions, double* __restrict__ box,
+                                                            const int nf) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    const CMap m = cl_map(nf);
+    const CSmem sm = cl_carve(smem_raw, kp.N, kp.A, kp.G, m.K, false);
+    const int e = (int)blockIdx.x / m.K;
+    cl_raster<T, EXACT>(sm, kp, m, reinterpret_cast<const double2*>(x) + (size_t)e * kp.N,
+                        reinterpret_cast<const double2*>(xa) + (size_t)e * kp.A, grid + (size_t)e * kp.G * kp.G * 2,
+                        positions + (size_t)e * kp.A * 2, box ? box + 4 * (size_t)e : nullptr);
+    cluster_sync();
+}
+
 // ------------------------------------------------------------------------------------------ host side
 
 thread_local char g_cuda_err[256] = "";
@@ -601,15 +875,44 @@ size_t step_smem(const SwarmParams* p, int raster, int n_stage, int mode) {
 // alignment is optional: 16 bytes enables the TMA zero fill, the filler warp and 16-byte stores.)
 bool grid_aligned(const void* grid) { return (reinterpret_cast<uintptr_t>(grid) & 7) == 0; }
 
+// ---- CLUSTER layout: SwarmParams::tuning bits 8-12 = K (1..16 CTAs per env), kClusterAuto = the library picks K
+constexpr int kClusterShift = 8, kClusterAuto = 31;
+int tuning_cluster(const SwarmParams* p) { return p->tuning > 0 ? (p->tuning >> kClusterShift) & 31 : 0; }
+// virtual warps of the env (the one-CTA kernel's force warps) and the cluster sizes they allow: at most one CTA per
+// warp and kClusterMaxK; at least as many CTAs as it takes to keep a CTA within kMaxThreads
+int cl_warps(int N) { return block_threads(N, force_mode(N)) >> 5; }
+int cl_kmin(int N) { return (cl_warps(N) * 32 + kMaxThreads - 1) / kMaxThreads; }
+int cl_kmax(int N) { return cl_warps(N) < kClusterMaxK ? cl_warps(N) : kClusterMaxK; }
+bool cl_fits(const SwarmParams* p, int K, bool force) {
+    return K >= cl_kmin(p->n_locusts) && cl_smem_bytes(p->n_locusts, p->n_agents, p->grid_size, K, force) <= kMaxSmem;
+}
+int validate_cluster(const SwarmParams* p, int cl) {
+    if ((p->tuning & 0x30) || (cl > kClusterMaxK && cl != kClusterAuto)) return SWARM_ERR_FLAGS;
+    // N <= 512: the one-CTA kernels take unordered pairs, which a cluster cannot reproduce bit for bit
+    if (p->n_locusts < kClusterMinLocusts) return SWARM_ERR_FLAGS;
+    if (cl != kClusterAuto) {
+        if (cl > cl_kmax(p->n_locusts)) return SWARM_ERR_FLAGS;        // a CTA without a warp
+        return cl_fits(p, cl, true) ? SWARM_OK : SWARM_ERR_SIZE;
+    }
+    for (int K = cl_kmin(p->n_locusts); K <= cl_kmax(p->n_locusts); ++K)
+        if (cl_fits(p, K, true)) return SWARM_OK;
+    return SWARM_ERR_SIZE;
+}
+
 int validate(const SwarmParams* p, int min_agents = 1) {
     if (!p) return SWARM_ERR_NULL;
-    if (p->n_envs < 1 || p->n_locusts < 1 || p->n_locusts > kMaxLocusts) return SWARM_ERR_SIZE;
+    const int cl = tuning_cluster(p);
+    if (p->n_envs < 1 || p->n_locusts < 1 || p->n_locusts > (cl ? kClusterMaxLocusts : kMaxLocusts)) return SWARM_ERR_SIZE;
     if (p->n_agents < min_agents || p->n_agents > 32) return SWARM_ERR_SIZE;
     if (p->grid_size < 2 || p->grid_size > 255) return SWARM_ERR_SIZE;      // positions are uint8
     if (p->n_burn_in < 0 || p->max_episode_steps < 0) return SWARM_ERR_SIZE;
     if (p->math_mode != 0 && p->math_mode != 1) return SWARM_ERR_FLAGS;
-    if (p->tuning < 0 || (p->tuning & ~0x30)) return SWARM_ERR_FLAGS;
-    if (step_smem(p, 1, 2, force_mode(p->n_locusts)) > kMaxSmem) return SWARM_ERR_SIZE;
+    if (p->tuning < 0 || (p->tuning & ~(0x30 | (31 << kClusterShift)))) return SWARM_ERR_FLAGS;
+    if (cl) {
+        if (int rc = validate_cluster(p, cl)) return rc;
+    } else if (step_smem(p, 1, 2, force_mode(p->n_locusts)) > kMaxSmem) {
+        return SWARM_ERR_SIZE;
+    }
     if (p->env_id_offset < 0 || p->env_id_offset + p->n_envs > (int64_t)0xffffffffLL) return SWARM_ERR_SIZE;
     return SWARM_OK;
 }
@@ -757,6 +1060,106 @@ int check_launch(const char* what) {
     return err == cudaSuccess ? SWARM_OK : cuda_fail(err, what);
 }
 
+// ---- CLUSTER layout: shape and launch ------------------------------------------------------------------------------
+struct ClusterShape {
+    int K, nf, nt;
+    size_t smem;
+};
+
+// clusters of K CTAs of this kernel that the device can hold at once (0: unschedulable), cached per device
+template <typename Kern>
+int cluster_occupancy(Kern kernel, int K, int nt, size_t smem, int* out) {
+    int dev = 0;
+    if (int rc = current_device(&dev)) return rc;
+    KernelCache& c = cache();
+    std::lock_guard<std::mutex> lk(c.mu);
+    const auto key = std::make_tuple(dev, (const void*)kernel, nt * 32 + K, smem);
+    auto o = c.occupancy.find(key);
+    if (o == c.occupancy.end()) {
+        cudaLaunchConfig_t cfg;
+        memset(&cfg, 0, sizeof(cfg));
+        cfg.gridDim = dim3((unsigned)K);
+        cfg.blockDim = dim3((unsigned)nt);
+        cfg.dynamicSmemBytes = smem;
+        cudaLaunchAttribute attr[1];
+        attr[0].id = cudaLaunchAttributeClusterDimension;
+        attr[0].val.clusterDim.x = (unsigned)K;
+        attr[0].val.clusterDim.y = 1;
+        attr[0].val.clusterDim.z = 1;
+        cfg.attrs = attr;
+        cfg.numAttrs = 1;
+        int n = 0;
+        const cudaError_t err = cudaOccupancyMaxActiveClusters(&n, kernel, &cfg);
+        if (err != cudaSuccess) {
+            cudaGetLastError();
+            n = 0;                     // e.g. a cluster size the device does not support: refused, not a failure
+        }
+        o = c.occupancy.emplace(key, n).first;
+    }
+    *out = o->second;
+    return SWARM_OK;
+}
+
+// The cluster size of a call and its launch shape.  Refuses (SWARM_ERR_SIZE) a size whose shared memory or cluster does
+// not fit the device -- before anything is launched.  The library's choice (kClusterAuto) is the largest K whose clusters
+// the device can hold for the whole batch at once (cudaOccupancyMaxActiveClusters >= E: one wave), else the smallest K.
+// Measured (profiles/r04_cluster.md): K beyond one wave costs a second wave (8192 x 16: K = 6 2.18 ms, K = 7 4.32 ms),
+// and in multi-wave batches more CTAs per env only add the per-CTA work (N = 2048, E = 148: K = 1 0.67 ms, K = 4 0.95).
+template <typename Kern>
+int cluster_shape(const SwarmParams* p, Kern kernel, bool force, ClusterShape* out) {
+    const int N = p->n_locusts, cl = tuning_cluster(p);
+    const int nf = block_threads(N, force_mode(N)), nw = nf >> 5;
+    const bool pick = cl == kClusterAuto;
+    const int k_hi = pick ? cl_kmax(N) : cl, k_lo = pick ? cl_kmin(N) : cl;
+    ClusterShape fallback = {0, 0, 0, 0};
+    for (int K = k_hi; K >= k_lo; --K) {
+        if (!cl_fits(p, K, force)) continue;
+        const int nt = cl_threads(nw, K);
+        const size_t smem = cl_smem_bytes(N, p->n_agents, p->grid_size, K, force);
+        int rc = prep(kernel, smem);
+        if (rc) return rc;
+        if (K > 8) {
+            const cudaError_t err = cudaFuncSetAttribute(kernel, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
+            if (err != cudaSuccess) {
+                cudaGetLastError();
+                continue;
+            }
+        }
+        int n = 0;
+        if ((rc = cluster_occupancy(kernel, K, nt, smem, &n))) return rc;
+        if (n < 1) continue;
+        const ClusterShape sh = {K, nf, nt, smem};
+        if (!pick || n >= p->n_envs) {
+            *out = sh;
+            return SWARM_OK;
+        }
+        fallback = sh;                 // the smallest schedulable K so far
+    }
+    if (fallback.K == 0) return SWARM_ERR_SIZE;
+    *out = fallback;
+    return SWARM_OK;
+}
+
+template <typename Kern, typename... Args>
+int launch_cluster(Kern kernel, const ClusterShape& sh, int n_envs, cudaStream_t s, const char* what, Args... args) {
+    cudaLaunchConfig_t cfg;
+    memset(&cfg, 0, sizeof(cfg));
+    cfg.gridDim = dim3((unsigned)((long long)n_envs * sh.K));
+    cfg.blockDim = dim3((unsigned)sh.nt);
+    cfg.dynamicSmemBytes = sh.smem;
+    cfg.stream = s;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeClusterDimension;
+    attr[0].val.clusterDim.x = (unsigned)sh.K;
+    attr[0].val.clusterDim.y = 1;
+    attr[0].val.clusterDim.z = 1;
+    cfg.attrs = attr;
+    cfg.numAttrs = 1;
+    const cudaError_t err = cudaLaunchKernelEx(&cfg, kernel, args...);
+    if (err != cudaSuccess) return cuda_fail(err, what);
+    return check_launch(what);
+}
+
 #define DISPATCH_T(T_, ...)              \
     switch (T_) {                        \
         case 1: { constexpr int TT = 1; __VA_ARGS__; } break; \
@@ -823,6 +1226,11 @@ StepKernel step_kernel(int mode, bool precise, int place) {
     return place == 2 ? step_kernel_p<2>(mode, precise) : (place == 3 ? step_kernel_p<3>(mode, precise) : step_kernel_p<0>(mode, precise));
 }
 
+StepKernel step_kernel_cluster(int mode, bool precise) {
+    return mode == 2 ? (precise ? k_step_cluster<2, true> : k_step_cluster<2, false>)
+                     : (precise ? k_step_cluster<4, true> : k_step_cluster<4, false>);
+}
+
 const SwarmInjectedDraws kNoDraws = {nullptr, nullptr, nullptr, nullptr, nullptr};
 
 bool draws_complete(const SwarmInjectedDraws* d) {
@@ -834,7 +1242,8 @@ bool draws_complete(const SwarmInjectedDraws* d) {
 //   FOLLOW  k_raster_follow on the side stream trails a rasteriser-less, one-env-per-CTA k_step (needs 2 + E flags)
 //   WARPS   a raster warp group inside persistent k_step CTAs, one env behind the force group
 //   SELF    the step's own threads rasterise their env right after stepping it (one env per CTA)
-enum RasterPlace { RASTER_NONE = 0, RASTER_FOLLOW = 1, RASTER_WARPS = 2, RASTER_SELF = 3 };
+//   CLUSTER the env's K CTAs of a thread-block cluster rasterise it after the step (the cluster layout, tuning bits 8-12)
+enum RasterPlace { RASTER_NONE = 0, RASTER_FOLLOW = 1, RASTER_WARPS = 2, RASTER_SELF = 3, RASTER_CLUSTER = 4 };
 
 struct StepShape {
     int mode;        // force mode (1..6)
@@ -860,9 +1269,13 @@ const char* swarm_strerror(int status) {
     switch (status) {
         case SWARM_OK: return "ok";
         case SWARM_ERR_NULL: return "required pointer is NULL";
-        case SWARM_ERR_SIZE: return "unsupported size (E>=1, 1<=N<=2048, 1<=A<=32, 2<=G<=255, shared memory <= 227 KB)";
+        case SWARM_ERR_SIZE:
+            return "unsupported size (E>=1, 1<=N<=2048 in one CTA per env or 513<=N<=8192 in the cluster layout, 1<=A<=32, "
+                   "2<=G<=255, shared memory <= 227 KB, a cluster the device can schedule)";
         case SWARM_ERR_LAUNCH: return "CUDA launch/runtime error (see swarm_last_cuda_error)";
-        case SWARM_ERR_FLAGS: return "inconsistent flags or missing optional buffer";
+        case SWARM_ERR_FLAGS:
+            return "inconsistent flags or missing optional buffer (the cluster layout: N > 512, K <= 16 and at most one CTA "
+                   "per force warp, no raster placement)";
         default: return "unknown status";
     }
 }
@@ -879,10 +1292,21 @@ int swarm_reset(const SwarmParams* p, const SwarmState* st, const uint8_t* mask,
     if (draws && !draws_complete(draws)) return SWARM_ERR_NULL;
     const int mode = force_mode(p->n_locusts);
     const KP kp = make_kp(p, mode);
+    cudaStream_t s = (cudaStream_t)stream;
+    if (tuning_cluster(p)) {
+        const SwarmInjectedDraws dr = draws ? *draws : kNoDraws;
+        const int has = draws ? 1 : 0;
+        ClusterShape sh;
+        auto go = [&](auto kernel) {
+            int r = cluster_shape(p, kernel, true, &sh);
+            return r ? r : launch_cluster(kernel, sh, kp.E, s, "swarm_reset", kp, *st, mask, dr, has, sh.nf);
+        };
+        if (mode == 2) return p->math_mode ? go(k_reset_cluster<2, true>) : go(k_reset_cluster<2, false>);
+        return p->math_mode ? go(k_reset_cluster<4, true>) : go(k_reset_cluster<4, false>);
+    }
     const size_t smem = step_smem(p, 0, 1, mode);
     const int nt = block_threads(kp.N, mode);
     if (nt > kMaxThreads) return SWARM_ERR_SIZE;
-    cudaStream_t s = (cudaStream_t)stream;
     DISPATCH_T(mode,
         if (p->math_mode) {
             if ((rc = prep(k_reset<TT, true>, smem))) return rc;
@@ -905,6 +1329,7 @@ struct StepPlan {
     int follow_threads, rgrid;    // follower launch (place == RASTER_FOLLOW)
     size_t smem, follow_smem;
     StepKernel kernel;
+    int cluster;                  // CTAs per env (place == RASTER_CLUSTER)
 };
 
 // Validates the arguments of swarm_step and decides its launch shape (automatic, or forced through
@@ -946,6 +1371,19 @@ int plan_step(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io,
     const int filler_threads = 32;                           // the SELF shape's TMA zero-fill warp
     const int mode = force_mode(N);
     const int nf = block_threads(N, mode);
+    out->cluster = 0;
+    if (tuning_cluster(p)) {
+        // one env per thread-block cluster; the observation (if any) comes from the cluster itself, st->work is not used
+        ClusterShape sh;
+        out->kernel = step_kernel_cluster(mode, p->math_mode != 0);
+        if ((rc = cluster_shape(p, out->kernel, true, &sh))) return rc;
+        out->mode = mode; out->place = RASTER_CLUSTER;
+        out->raster = 0; out->n_stage = 0; out->filler = 0; out->dynamic = 0;
+        out->nf = sh.nf; out->nt = sh.nt; out->smem = sh.smem; out->cluster = sh.K;
+        out->grid = (int)((long long)E * sh.K);
+        out->follow_threads = 0; out->follow_smem = 0; out->rgrid = 0;
+        return SWARM_OK;
+    }
     if (nf > kMaxThreads) return SWARM_ERR_SIZE;
     // With the per-env flags the observation can be produced by a second kernel that follows the step on a higher-priority
     // stream (k_raster_follow).  The follower spins until the step publishes an env, so the step must always be able to get
@@ -1032,7 +1470,7 @@ int swarm_step_plan(const SwarmParams* p, const SwarmState* st, const SwarmStepI
     const int rc = plan_step(p, st, io, nullptr, &pl);
     if (rc) return rc;
     out[0] = pl.mode; out[1] = pl.filler; out[2] = pl.place; out[3] = pl.nt; out[4] = pl.grid;
-    out[5] = (int32_t)pl.smem; out[6] = pl.place == RASTER_FOLLOW ? pl.rgrid : 0;
+    out[5] = (int32_t)pl.smem; out[6] = pl.place == RASTER_FOLLOW ? pl.rgrid : (pl.place == RASTER_CLUSTER ? pl.cluster : 0);
     out[7] = pl.place == RASTER_FOLLOW ? 2 : 1;
     return SWARM_OK;
 }
@@ -1055,6 +1493,10 @@ int swarm_step(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io
     const StepKernel kernel = pl.kernel;
     const int grid = pl.grid, nt = pl.nt, nf = pl.nf, rgrid = pl.rgrid, follow_threads = pl.follow_threads;
     const size_t smem = pl.smem, follow_smem = pl.follow_smem;
+    if (pl.place == RASTER_CLUSTER) {      // no PDL: a cluster launch is an ordinary dependent of its predecessor
+        const ClusterShape sh = {pl.cluster, nf, nt, smem};
+        return launch_cluster(kernel, sh, p->n_envs, s, "swarm_step", kp, *st, *io, dr, has, nf);
+    }
     if (pl.place != RASTER_FOLLOW) {
         // Single-kernel shapes are launched as programmatic dependents of whatever precedes them in the stream: when that is
         // the previous step (back-to-back env steps, a captured rollout graph) its tail overlaps with this kernel's launch
@@ -1260,6 +1702,16 @@ int swarm_rasterize(const SwarmParams* p, const double* x, const double* xa, flo
     if (p->n_agents > 0 && (!xa || !positions)) return SWARM_ERR_NULL;
     if (!grid_aligned(grid)) return SWARM_ERR_FLAGS;
     const KP kp = make_kp(p);
+    if (tuning_cluster(p)) {
+        const cudaStream_t s = (cudaStream_t)stream;
+        ClusterShape sh;
+        auto go = [&](auto kernel) {
+            int r = cluster_shape(p, kernel, false, &sh);
+            return r ? r : launch_cluster(kernel, sh, kp.E, s, "swarm_rasterize", kp, x, xa, grid, positions, box, sh.nf);
+        };
+        if (force_mode(kp.N) == 2) return box ? go(k_rasterize_cluster<2, true>) : go(k_rasterize_cluster<2, false>);
+        return box ? go(k_rasterize_cluster<4, true>) : go(k_rasterize_cluster<4, false>);
+    }
     const size_t smem = smem_bytes(kp.N, kp.A, kp.G, 0, false, 1, 0);
     const int nt = (kp.N + kp.A) <= 128 ? 64 : 128;
     if (box) {
@@ -1304,10 +1756,19 @@ int swarm_forces(const SwarmParams* p, const double* x, const double* xa, float*
     if (!x || !xa || (!v && !reward)) return SWARM_ERR_NULL;
     const int mode = force_mode(p->n_locusts);
     const KP kp = make_kp(p, mode);
+    cudaStream_t s = (cudaStream_t)stream;
+    if (tuning_cluster(p)) {
+        ClusterShape sh;
+        auto go = [&](auto kernel) {
+            int r = cluster_shape(p, kernel, true, &sh);
+            return r ? r : launch_cluster(kernel, sh, kp.E, s, "swarm_forces", kp, x, xa, v, reward, sh.nf);
+        };
+        if (mode == 2) return p->math_mode ? go(k_forces_cluster<2, true>) : go(k_forces_cluster<2, false>);
+        return p->math_mode ? go(k_forces_cluster<4, true>) : go(k_forces_cluster<4, false>);
+    }
     const size_t smem = step_smem(p, 0, 1, mode);
     const int nt = block_threads(kp.N, mode);
     if (nt > kMaxThreads) return SWARM_ERR_SIZE;
-    cudaStream_t s = (cudaStream_t)stream;
     DISPATCH_T(mode,
         if (p->math_mode) {
             if ((rc = prep(k_forces<TT, true>, smem))) return rc;

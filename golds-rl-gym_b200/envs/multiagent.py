@@ -92,12 +92,14 @@ class BatchedSwarmEnv(object):
 
     def __init__(self, num_envs, n_locusts=None, n_agents=None, grid_size=84, max_episode_steps=128,
                  seed=0, env_id_offset=0, device=None, math_mode="fast", auto_reset=True, rasterize=True,
-                 binding="torch", tuning=0, noise="frozen"):
+                 binding="torch", tuning=0, noise="frozen", cluster=None):
         """binding: "torch" = the hot calls go through torch.ops.swarm_b200.* (the C ABI as a PyTorch
         extension, csrc/torch_binding.cpp), "ctypes" = straight into the C ABI.  Same kernels either way.
         tuning: SwarmParams.tuning (0 = automatic launch shape; anything else only changes speed, never bits).
         noise: "frozen" (the reference: every step after a reset re-uses noise row N_BURN_IN) or "fresh" (step k of
-        an episode uses row N_BURN_IN + k, drawn by Philox inside the step kernel; SWARM_STEP_FRESH_NOISE)."""
+        an episode uses row N_BURN_IN + k, drawn by Philox inside the step kernel; SWARM_STEP_FRESH_NOISE).
+        cluster: None = one CTA per env up to 2048 locusts and a thread-block cluster of the library's size above; an
+        integer K = a cluster of K CTAs per env (1..16, for 512 < n_locusts <= 8192; bitwise the same results)."""
         self.lib = nat.load()
         if binding not in ("torch", "ctypes"):
             raise ValueError("binding must be 'torch' or 'ctypes'")
@@ -113,11 +115,16 @@ class BatchedSwarmEnv(object):
         self.N = int(n_locusts if n_locusts is not None else self.N_LOCUSTS)
         self.A = int(n_agents if n_agents is not None else self.N_AGENTS)
         self.G = int(grid_size)
+        tuning = int(tuning)
+        if cluster is not None:
+            tuning |= nat.tune_cluster(int(cluster))
+        elif self.N > nat.MAX_LOCUSTS_ONE_CTA and not tuning & nat.TUNE_CLUSTER_MASK:
+            tuning |= nat.TUNE_CLUSTER_AUTO
         self.auto_reset = bool(auto_reset)
         self.rasterize = bool(rasterize)
         self.params = nat.SwarmParams(
             n_envs=self.E, n_locusts=self.N, n_agents=self.A, grid_size=self.G, n_burn_in=self.N_BURN_IN,
-            max_episode_steps=int(max_episode_steps), math_mode={"fast": 0, "precise": 1}[math_mode], tuning=int(tuning),
+            max_episode_steps=int(max_episode_steps), math_mode={"fast": 0, "precise": 1}[math_mode], tuning=tuning,
             noise=self.NOISE, gravity=self.GRAVITY, wind=self.WIND_SPEED, F=self.F, L=self.L, dt=self.dt,
             box_width=3.0, box_height=3.0, seed=int(seed) & (2 ** 64 - 1), env_id_offset=int(env_id_offset))
         nat.check(self.lib.swarm_validate(ctypes.byref(self.params)), "swarm_validate")
@@ -261,7 +268,13 @@ class BatchedSwarmEnv(object):
             nat.check(self.lib.swarm_step_plan(self._params_ref, self._state_ref, ctypes.byref(io), out), "swarm_step_plan")
         keys = ("force_mode", "filler_warp", "raster_place", "threads", "ctas", "smem_bytes", "follower_ctas", "launches")
         d = dict(zip(keys, list(out)))
-        d["raster_place"] = ("none", "follower kernel", "raster warps in k_step", "k_step's own threads")[d["raster_place"]]
+        cluster = d["raster_place"] == 4
+        d["raster_place"] = ("none", "follower kernel", "raster warps in k_step", "k_step's own threads",
+                             "the env's cluster")[d["raster_place"]]
+        d["layout"] = "cluster" if cluster else "one CTA per env"
+        d["cluster_size"] = d["follower_ctas"] if cluster else 1      # out[6] holds K in the cluster layout
+        if cluster:
+            d["follower_ctas"] = 0
         return d
 
     # ------------------------------------------------------------------ host-buffer (end-to-end) form
@@ -498,8 +511,9 @@ class SwarmEnv(object):
         lib = nat.load()
         x_t = torch.as_tensor(np.ascontiguousarray(x, dtype=np.float64)[None]).cuda()
         xa_t = torch.as_tensor(np.ascontiguousarray(xa, dtype=np.float64)[None]).cuda()
+        tuning = nat.TUNE_CLUSTER_AUTO if x_t.shape[1] > nat.MAX_LOCUSTS_ONE_CTA else 0
         p = nat.SwarmParams(n_envs=1, n_locusts=x_t.shape[1], n_agents=xa_t.shape[1], grid_size=84, n_burn_in=10,
-                            max_episode_steps=0, math_mode=0, tuning=0, noise=1e-4, gravity=float(G),
+                            max_episode_steps=0, math_mode=0, tuning=tuning, noise=1e-4, gravity=float(G),
                             wind=float(U), F=float(F), L=float(L), dt=0.05, box_width=3.0, box_height=3.0,
                             seed=0, env_id_offset=0)
         v = torch.empty(1, x_t.shape[1], 2, dtype=torch.float32, device=x_t.device)

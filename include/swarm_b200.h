@@ -53,9 +53,14 @@ typedef struct SwarmParams {
     int32_t n_burn_in;          /* SwarmEnv.N_BURN_IN (10)                                  */
     int32_t max_episode_steps;  /* gym TimeLimit (128); 0 = raw SwarmEnv, no limit          */
     int32_t math_mode;          /* 0 = fast (MUFU rsqrt/ex2/rcp), 1 = precise (IEEE)        */
-    int32_t tuning;             /* 0 = automatic launch shape.  Otherwise (tests / experiments; results are bitwise
-                                 * the same for every value): bits 4-5 = rasteriser placement (1 follower kernel,
-                                 * 2 raster warps in the step kernel, 3 the step's own threads after the step);
+    int32_t tuning;             /* 0 = automatic launch shape.  Otherwise (results are bitwise the same for every
+                                 * value): bits 4-5 = rasteriser placement (1 follower kernel, 2 raster warps in the
+                                 * step kernel, 3 the step's own threads after the step);
+                                 * bits 8-12 = the CLUSTER layout: 0 one CTA per env (N <= 2048), 1..16 one env per
+                                 * thread-block cluster of K CTAs, 31 the library picks K.  It takes 512 < N <= 8192
+                                 * (SWARM_ERR_FLAGS for N <= 512, K > 16, K above the env's force warps, or with
+                                 * placement bits; SWARM_ERR_SIZE when the layout does not fit the device) and
+                                 * applies to swarm_step / _reset / _forces / _rasterize;
                                  * all other bits must be 0                                                   */
     double noise;               /* NOISE 1e-4   */
     double gravity;             /* GRAVITY -1   */
@@ -131,7 +136,8 @@ int swarm_abi_version(void);
 const char* swarm_strerror(int status);
 const char* swarm_last_cuda_error(void);
 
-/* Size / resource check for a parameter set; SWARM_OK or SWARM_ERR_SIZE.  No GPU work. */
+/* Size / resource check for a parameter set; SWARM_OK, SWARM_ERR_SIZE or SWARM_ERR_FLAGS.  No GPU work (whether a
+ * cluster can be scheduled is checked by the calls themselves, before they launch anything). */
 int swarm_validate(const SwarmParams* p);
 
 /* SwarmEnv._reset (multiagent.py:46-63): draws + n_burn_in burn-in steps; elapsed=0; episode+=1.
@@ -160,7 +166,8 @@ int swarm_step(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io
 
 /* The launch shape swarm_step would use for these arguments (no launch; needs the device for occupancy queries):
  * out = { force mode, filler warp (0/1), rasteriser placement (0 none, 1 follower kernel, 2 raster warps, 3 the step's
- * own threads), threads per CTA, CTAs, dynamic shared memory bytes, follower CTAs, kernel launches }. */
+ * own threads, 4 the env's thread-block cluster), threads per CTA, CTAs (E K in the cluster layout), dynamic shared
+ * memory bytes, follower CTAs (the cluster layout: K), kernel launches }. */
 int swarm_step_plan(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io, int32_t out[8]);
 
 /* Same call with HOST buffers for the per-step inputs/results; synchronises the stream before
