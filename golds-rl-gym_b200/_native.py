@@ -74,6 +74,11 @@ class SwarmStepIO(ctypes.Structure):
                 ("positions", c_void_p), ("v_out", c_void_p), ("flags", c_uint32), ("reserved", c_uint32)]
 
 
+class SwarmStepFinal(ctypes.Structure):
+    _fields_ = [("x", c_void_p), ("xa", c_void_p), ("terminated", c_void_p), ("truncated", c_void_p),
+                ("grid", c_void_p), ("positions", c_void_p)]
+
+
 # name -> (restype, argtypes); every symbol include/swarm_b200.h declares
 _P = ctypes.POINTER
 SYMBOLS = {
@@ -83,6 +88,8 @@ SYMBOLS = {
     "swarm_validate": (c_int, [_P(SwarmParams)]),
     "swarm_reset": (c_int, [_P(SwarmParams), _P(SwarmState), c_void_p, _P(SwarmInjectedDraws), c_void_p]),
     "swarm_step": (c_int, [_P(SwarmParams), _P(SwarmState), _P(SwarmStepIO), _P(SwarmInjectedDraws), c_void_p]),
+    "swarm_step_final": (c_int, [_P(SwarmParams), _P(SwarmState), _P(SwarmStepIO), _P(SwarmStepFinal),
+                                 _P(SwarmInjectedDraws), c_void_p]),
     "swarm_step_plan": (c_int, [_P(SwarmParams), _P(SwarmState), _P(SwarmStepIO), c_void_p]),
     "swarm_step_host": (c_int, [_P(SwarmParams), _P(SwarmState), _P(SwarmStepIO), c_void_p, c_void_p, c_void_p,
                                 c_void_p, c_void_p, c_void_p]),

@@ -3,6 +3,7 @@
 ``create_environment()`` keeps the reference meaning (one 'Swarm-v0' env, 128-step TimeLimit);
 ``create_batched_environment(E, ...)`` is what the device-resident learner uses instead of E of them.
 ``noise``: "frozen" (the reference) or "fresh" (SURVEY Q1 fixed), see BatchedSwarmEnv.
+``final_obs=True``: the batched env also keeps each ended episode's terminal state and observation (BatchedSwarmEnv).
 """
 from ...envs import multiagent as ma
 
@@ -18,8 +19,8 @@ class SwarmEnvironmentCreator(object):
     def create_environment(self):
         return ma.make("Swarm-v0", fresh_noise=self.noise == "fresh")
 
-    def create_batched_environment(self, num_envs, seed=0, env_id_offset=0, device=None):
+    def create_batched_environment(self, num_envs, seed=0, env_id_offset=0, device=None, final_obs=False):
         return ma.BatchedSwarmEnv(num_envs, n_locusts=self.n_locusts, grid_size=self.grid_size,
                                   max_episode_steps=ma.REGISTRY["Swarm-v0"]["max_episode_steps"], seed=seed,
                                   env_id_offset=env_id_offset, device=device, math_mode=self.math_mode,
-                                  auto_reset=True, rasterize=True, noise=self.noise)
+                                  auto_reset=True, rasterize=True, noise=self.noise, final_obs=final_obs)

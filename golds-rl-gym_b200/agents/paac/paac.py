@@ -16,6 +16,9 @@ NCCL once per update -- the only collective; clipping and Adam then run identica
 Reference quirks at this boundary (SURVEY.md section 8a), selectable:
   reward_indexing="reference"  rewards[t, e_idx] for e_idx < E only (paac.py:331-338, Q6); "per_agent" = fixed
   mask_terminals=False         returns bootstrap through episode ends (paac.py:363 commented mask, Q7)
+  bootstrap_truncated=True     (with mask_terminals=True) a TimeLimit truncation is bootstrapped from V of the episode's
+                               terminal observation instead of being cut to 0 like a termination:
+                               ret_t = r_t + gamma [(1 - done_t) ret_t+1 + truncated_t (1 - terminated_t) V(final_t)]
 """
 import logging
 import time
@@ -33,7 +36,7 @@ class GridPAACLearner(object):
 
     def __init__(self, network_creator, environment_creator, args, emulator_class=SwarmRunner, state_processor=None,
                  device=None, reward_indexing="reference", mask_terminals=False, use_cuda_graph=True,
-                 compact_obs="auto", net_precision="fp32"):
+                 compact_obs="auto", net_precision="fp32", bootstrap_truncated=False):
         self.args = args
         self.emulator_class = emulator_class
         self.max_local_steps = args.max_local_steps
@@ -46,6 +49,10 @@ class GridPAACLearner(object):
         self.clip_norm_type = args.clip_norm_type
         self.reward_indexing = reward_indexing
         self.mask_terminals = mask_terminals
+        if bootstrap_truncated and not mask_terminals:
+            raise ValueError("bootstrap_truncated=True needs mask_terminals=True (without the mask every return already "
+                             "runs on through the episode end)")
+        self.bootstrap_truncated = bool(bootstrap_truncated)
         self.use_cuda_graph = use_cuda_graph
         # compact_obs: the net consumes (grid (E,G,G,2), positions (E,A,2)) through forward_compact -- exactly the
         # same function of the observation, without ever materialising the reference's (E,A,G,G,3) layout
@@ -65,8 +72,9 @@ class GridPAACLearner(object):
 
         self.total_emulators = args.emulator_counts
         first, self.emulator_counts = sharding.shard_envs(self.total_emulators, self.world, self.rank)
+        extra = dict(final_obs=True) if self.bootstrap_truncated else {}
         self.env = environment_creator.create_batched_environment(
-            self.emulator_counts, seed=getattr(args, "random_seed", 3), env_id_offset=first, device=self.device)
+            self.emulator_counts, seed=getattr(args, "random_seed", 3), env_id_offset=first, device=self.device, **extra)
         self.N_AGENTS = self.env.A
         self.real_batch_size = self.emulator_counts * self.N_AGENTS
         # "auto": the factorised path pays off once the policy batch is large enough to be bandwidth/FLOP bound
@@ -114,6 +122,13 @@ class GridPAACLearner(object):
         self.not_over = torch.ones(T, B, dtype=torch.float32, device=d)
         self.y_batch = torch.zeros(T, B, dtype=torch.float32, device=d)
         self.adv_batch = torch.zeros(T, B, dtype=torch.float32, device=d)
+        if self.bootstrap_truncated:
+            # slot t: the terminal observation of the envs whose episode ended at step t (compact in both obs modes),
+            # and the step's done split
+            self.final_grids = torch.zeros(T, E, G, G, 2, dtype=torch.float32, device=d)
+            self.final_positions = torch.zeros(T, E, A, 2, dtype=torch.uint8, device=d)
+            self.terminated = torch.zeros(T, B, dtype=torch.float32, device=d)
+            self.truncated = torch.zeros(T, B, dtype=torch.float32, device=d)
         # episode statistics, accumulated on the device (read back only when logging)
         self.episode_return = torch.zeros(E, dtype=torch.float32, device=d)
         self.finished_return_sum = torch.zeros((), dtype=torch.float64, device=d)
@@ -147,10 +162,15 @@ class GridPAACLearner(object):
         self.actions[t].copy_(next_actions)
         self.values[t].copy_(v)
         # one fused step launch + one expand launch, straight into the next ring slot
+        fin = dict(final_grid_out=self.final_grids[t], final_positions_out=self.final_positions[t]) \
+            if self.bootstrap_truncated else {}
         if self.compact_obs:
-            self.runners.update_environments(grid_out=self.grids[t + 1], positions_out=self.positions[t + 1])
+            self.runners.update_environments(grid_out=self.grids[t + 1], positions_out=self.positions[t + 1], **fin)
         else:
-            self.runners.update_environments(states_out=self.states[t + 1])
+            self.runners.update_environments(states_out=self.states[t + 1], **fin)
+        if self.bootstrap_truncated:
+            self.terminated[t].copy_(self.env.terminated.to(torch.float32).repeat_interleave(A))
+            self.truncated[t].copy_(self.env.truncated.to(torch.float32).repeat_interleave(A))
         reward, over = self.env.reward, self.env.done_u8
         if self.reward_indexing == "reference":
             self.rewards[t, :E].copy_(reward)                      # paac.py:338  rewards[t, e_idx], e_idx < E
@@ -170,8 +190,19 @@ class GridPAACLearner(object):
     def _returns(self):
         T = self.max_local_steps
         ret = self._predict(T)["vs"].clone()                                # paac.py:351-358
+        if self.bootstrap_truncated:
+            # V of every terminal observation of the rollout in one forward (T E envs); weight 0 where no episode was
+            # truncated (the slots of the other envs hold stale, finite observations)
+            E, A = self.emulator_counts, self.N_AGENTS
+            with self._autocast():
+                v_fin = self.network.predict_compact(self.final_grids.view(T * E, *self.final_grids.shape[2:]),
+                                                     self.final_positions.view(T * E, A, 2))["vs"].float()
+            boot = v_fin.view(T, -1) * self.truncated * (1.0 - self.terminated)
         for t in reversed(range(T)):                                        # paac.py:362-365
-            ret = self.rewards[t] + self.gamma * ret * (self.not_over[t] if self.mask_terminals else 1.0)
+            if self.bootstrap_truncated:
+                ret = self.rewards[t] + self.gamma * (ret * self.not_over[t] + boot[t])
+            else:
+                ret = self.rewards[t] + self.gamma * ret * (self.not_over[t] if self.mask_terminals else 1.0)
             self.y_batch[t].copy_(ret)
             self.adv_batch[t].copy_(ret - self.values[t])
 

@@ -37,6 +37,7 @@ class GridRunners(object):
         self.actions = env.actions                      # (E,A,2) f32, written in place by the learner
         self.variables = [self.states, self.histories, env.positions, self.rewards, self.episode_over, self.actions]
         self._started = False
+        self.final_info = {}
 
     def start(self, states_out=None):
         """runners.py:34-36.  Initial reset + first observation (paac.py:247-251 does this in the parent).
@@ -55,15 +56,23 @@ class GridRunners(object):
     def get_shared_variables(self):
         return self.variables
 
-    def update_environments(self, states_out=None, grid_out=None, positions_out=None):
+    def update_environments(self, states_out=None, grid_out=None, positions_out=None, final_grid_out=None,
+                            final_positions_out=None):
         """states_out: optional (E,A,G,G,3) tensor that receives the new expanded observation directly (the
-        device-resident learner points it at its rollout ring, saving one 847 KB/env copy per step)."""
+        device-resident learner points it at its rollout ring, saving one 847 KB/env copy per step).
+        final_grid_out / final_positions_out: the same for the terminal observation of the envs whose episode ended
+        (an env built with final_obs=True; its info dict -- terminated, truncated, final_* -- is self.final_info)."""
         if self.coord is not None and self.coord.should_stop():
             self.stop()
             return
         env = self.env
-        _, reward, done, _ = env.step(self.actions, rasterize=True, auto_reset=True, grid_out=grid_out,
-                                      positions_out=positions_out)
+        if getattr(env, "final_obs", False):
+            _, reward, done, self.final_info = env.step(self.actions, rasterize=True, auto_reset=True, grid_out=grid_out,
+                                                        positions_out=positions_out, final_grid_out=final_grid_out,
+                                                        final_positions_out=final_positions_out)
+        else:
+            _, reward, done, _ = env.step(self.actions, rasterize=True, auto_reset=True, grid_out=grid_out,
+                                          positions_out=positions_out)
         if grid_out is not None:
             pass                                    # compact consumer: no expanded observation at all
         elif states_out is not None:

@@ -57,9 +57,14 @@ __device__ __forceinline__ void prefetch_env(const Stage& sg, const KP& kp, cons
 // PLACE (compile time, so that every instantiation only carries the code it runs -- the kernel is instruction-cache
 // sensitive): 0 no rasteriser in this kernel (none wanted, or k_raster_follow trails it), 2 a raster GROUP rides along,
 // 3 the force group rasterises its own env after the step (SELF; optionally with a filler warp for the TMA zero fill).
-template <int MODE, bool PRECISE, int PLACE>
+// FIN (swarm_step_final; fin's pointers nullable): the done split of every env and the terminal state of the done ones,
+// copied out of the stage buffer in the (rare) done branch before the auto-reset overwrites it.  Compile time, so that
+// swarm_step's kernels (FIN = false) stay exactly what they were: the same code behind a runtime branch re-schedules
+// the whole kernel and was measured to cost 2.8 % of the C4 step with the feature off (0.1703 -> 0.1751 ms).
+template <int MODE, bool PRECISE, int PLACE, bool FIN>
 __global__ void __maxnreg__(64) k_step(const KP kp, const SwarmState st, const SwarmStepIO io,
-                                       const SwarmInjectedDraws dr, const int has_draws, const int n_force) {
+                                       const SwarmInjectedDraws dr, const int has_draws, const int n_force,
+                                       const SwarmStepFinal fin) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int N = kp.N, A = kp.A;
     const int n_all = blockDim.x, n_raster = n_all - n_force;
@@ -185,6 +190,22 @@ __global__ void __maxnreg__(64) k_step(const KP kp, const SwarmState st, const S
                     if (g.tid == 0) {
                         io.reward[e] = (float)reward;
                         io.done[e] = done ? 1 : 0;
+                        if constexpr (FIN) {
+                            if (fin.terminated) fin.terminated[e] = reward >= 0.0 ? 1 : 0;
+                            if (fin.truncated) fin.truncated[e] = (kp.max_steps > 0 && elapsed >= kp.max_steps) ? 1 : 0;
+                        }
+                    }
+                    if constexpr (FIN) {
+                        // the terminal state, final since env_step's closing barrier; reset_begin's leading barrier
+                        // orders these reads before its writes
+                        if (done && fin.x) {
+                            double2* fx = reinterpret_cast<double2*>(fin.x) + (size_t)e * N;
+                            for (int i = g.tid; i < N; i += g.n) fx[i] = sm.st.xs[i];
+                        }
+                        if (done && fin.xa) {
+                            double2* fa = reinterpret_cast<double2*>(fin.xa) + (size_t)e * A;
+                            for (int k = g.tid; k < A; k += g.n) fa[k] = sm.st.as[k];
+                        }
                     }
                     if (!(done && (io.flags & SWARM_STEP_AUTO_RESET))) break;      // group-uniform
                     ep = st.episode[e];
@@ -396,12 +417,15 @@ __global__ void __launch_bounds__(128) k_raster_follow(const KP kp, const double
 
 // SwarmStateProcessor.process_state for the batch (standalone: one CTA per env).  EXACT: the caller wants the bounding
 // box (_get_bounding_box), so numpy's sequential mean is always walked; otherwise the same verified parallel mean as the step.
+// mask: nullable (E) u8, only envs with mask != 0 are rasterised (the terminal observations of swarm_step_final).
 template <bool EXACT>
 __global__ void __launch_bounds__(256) k_rasterize(const KP kp, const double* __restrict__ x,
                                                    const double* __restrict__ xa, float* __restrict__ grid,
-                                                   uint8_t* __restrict__ positions, double* __restrict__ box) {
+                                                   uint8_t* __restrict__ positions, double* __restrict__ box,
+                                                   const uint8_t* __restrict__ mask) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int e = blockIdx.x;
+    if (mask && !mask[e]) return;
     const int cells = kp.G * kp.G;
     const Smem sm = carve(smem_raw, kp.N, kp.A, kp.G, 0, false, 0, 1);
     const RGrp g = {(int)threadIdx.x, (int)blockDim.x};
@@ -643,9 +667,11 @@ __device__ __forceinline__ void cl_store(const KP& kp, const CMap& m, double2* x
 }
 
 // SwarmEnv._step + TimeLimit + auto-reset + process_state (k_step's contract) for the cluster layout.
-template <int MODE, bool PRECISE>
+// FIN: k_step's; each CTA copies its own targets' terminal positions from pn[], rank 0 the agents' from sm.as.
+template <int MODE, bool PRECISE, bool FIN>
 __global__ void __maxnreg__(64) k_step_cluster(const KP kp, const SwarmState st, const SwarmStepIO io,
-                                               const SwarmInjectedDraws dr, const int has_draws, const int nf) {
+                                               const SwarmInjectedDraws dr, const int has_draws, const int nf,
+                                               const SwarmStepFinal fin) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     constexpr int T = ModeT<MODE>::T;
     const int N = kp.N, A = kp.A, tid = (int)threadIdx.x;
@@ -713,6 +739,14 @@ __global__ void __maxnreg__(64) k_step_cluster(const KP kp, const SwarmState st,
             if (lead && tid == 0) {
                 io.reward[e] = (float)reward;
                 io.done[e] = done ? 1 : 0;
+                if constexpr (FIN) {
+                    if (fin.terminated) fin.terminated[e] = reward >= 0.0 ? 1 : 0;
+                    if (fin.truncated) fin.truncated[e] = (kp.max_steps > 0 && elapsed >= kp.max_steps) ? 1 : 0;
+                }
+            }
+            if constexpr (FIN) {
+                if (done && fin.x) cl_store(kp, m, reinterpret_cast<double2*>(fin.x) + (size_t)e * N, pn);
+                if (done && fin.xa && lead && tid < A) reinterpret_cast<double2*>(fin.xa)[(size_t)e * A + tid] = sm.as[tid];
             }
             if (!(done && (io.flags & SWARM_STEP_AUTO_RESET))) break;      // cluster-uniform
             cl_reset_begin(sm, kp, m, e, xe, nz);
@@ -811,11 +845,12 @@ template <int T, bool EXACT>
 __global__ void __launch_bounds__(1024) k_rasterize_cluster(const KP kp, const double* __restrict__ x,
                                                             const double* __restrict__ xa, float* __restrict__ grid,
                                                             uint8_t* __restrict__ positions, double* __restrict__ box,
-                                                            const int nf) {
+                                                            const int nf, const uint8_t* __restrict__ mask) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const CMap m = cl_map(nf);
-    const CSmem sm = cl_carve(smem_raw, kp.N, kp.A, kp.G, m.K, false);
     const int e = (int)blockIdx.x / m.K;
+    if (mask && !mask[e]) return;            // the whole cluster
+    const CSmem sm = cl_carve(smem_raw, kp.N, kp.A, kp.G, m.K, false);
     cl_raster<T, EXACT>(sm, kp, m, reinterpret_cast<const double2*>(x) + (size_t)e * kp.N,
                         reinterpret_cast<const double2*>(xa) + (size_t)e * kp.A, grid + (size_t)e * kp.G * kp.G * 2,
                         positions + (size_t)e * kp.A * 2, box ? box + 4 * (size_t)e : nullptr);
@@ -1210,28 +1245,38 @@ T* mapped_host(T* host) {
     return a.type == cudaMemoryTypeHost ? static_cast<T*>(a.devicePointer) : nullptr;
 }
 
-typedef void (*StepKernel)(const KP, const SwarmState, const SwarmStepIO, const SwarmInjectedDraws, const int, const int);
+typedef void (*StepKernel)(const KP, const SwarmState, const SwarmStepIO, const SwarmInjectedDraws, const int, const int,
+                           const SwarmStepFinal);
 
-template <int PLACE>
+template <int PLACE, bool FIN>
 StepKernel step_kernel_p(int mode, bool precise) {
     switch (mode) {
-        case 1: return precise ? k_step<1, true, PLACE> : k_step<1, false, PLACE>;
-        case 2: return precise ? k_step<2, true, PLACE> : k_step<2, false, PLACE>;
-        case 3: return precise ? k_step<3, true, PLACE> : k_step<3, false, PLACE>;
-        default: return precise ? k_step<4, true, PLACE> : k_step<4, false, PLACE>;
+        case 1: return precise ? k_step<1, true, PLACE, FIN> : k_step<1, false, PLACE, FIN>;
+        case 2: return precise ? k_step<2, true, PLACE, FIN> : k_step<2, false, PLACE, FIN>;
+        case 3: return precise ? k_step<3, true, PLACE, FIN> : k_step<3, false, PLACE, FIN>;
+        default: return precise ? k_step<4, true, PLACE, FIN> : k_step<4, false, PLACE, FIN>;
     }
 }
-// place: RasterPlace (NONE / FOLLOW share the rasteriser-less kernel)
-StepKernel step_kernel(int mode, bool precise, int place) {
-    return place == 2 ? step_kernel_p<2>(mode, precise) : (place == 3 ? step_kernel_p<3>(mode, precise) : step_kernel_p<0>(mode, precise));
+template <bool FIN>
+StepKernel step_kernel_f(int mode, bool precise, int place) {
+    return place == 2 ? step_kernel_p<2, FIN>(mode, precise)
+                      : (place == 3 ? step_kernel_p<3, FIN>(mode, precise) : step_kernel_p<0, FIN>(mode, precise));
+}
+// place: RasterPlace (NONE / FOLLOW share the rasteriser-less kernel); fin: the swarm_step_final variant
+StepKernel step_kernel(int mode, bool precise, int place, bool fin) {
+    return fin ? step_kernel_f<true>(mode, precise, place) : step_kernel_f<false>(mode, precise, place);
 }
 
-StepKernel step_kernel_cluster(int mode, bool precise) {
-    return mode == 2 ? (precise ? k_step_cluster<2, true> : k_step_cluster<2, false>)
-                     : (precise ? k_step_cluster<4, true> : k_step_cluster<4, false>);
+StepKernel step_kernel_cluster(int mode, bool precise, bool fin) {
+    if (fin)
+        return mode == 2 ? (precise ? k_step_cluster<2, true, true> : k_step_cluster<2, false, true>)
+                         : (precise ? k_step_cluster<4, true, true> : k_step_cluster<4, false, true>);
+    return mode == 2 ? (precise ? k_step_cluster<2, true, false> : k_step_cluster<2, false, false>)
+                     : (precise ? k_step_cluster<4, true, false> : k_step_cluster<4, false, false>);
 }
 
 const SwarmInjectedDraws kNoDraws = {nullptr, nullptr, nullptr, nullptr, nullptr};
+const SwarmStepFinal kNoFinal = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
 
 bool draws_complete(const SwarmInjectedDraws* d) {
     return d->x0 && d->xa0 && d->burn_actions && d->agent_noise && d->particle_noise;
@@ -1335,7 +1380,7 @@ struct StepPlan {
 // Validates the arguments of swarm_step and decides its launch shape (automatic, or forced through
 // SwarmParams::tuning).  Touches the GPU only for attribute / occupancy queries (cached per device).
 int plan_step(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io, const SwarmInjectedDraws* reset_draws,
-              StepPlan* out) {
+              StepPlan* out, const bool fin = false) {
     int rc = validate(p);
     if (rc) return rc;
     if (!st || !io) return SWARM_ERR_NULL;
@@ -1375,7 +1420,7 @@ int plan_step(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io,
     if (tuning_cluster(p)) {
         // one env per thread-block cluster; the observation (if any) comes from the cluster itself, st->work is not used
         ClusterShape sh;
-        out->kernel = step_kernel_cluster(mode, p->math_mode != 0);
+        out->kernel = step_kernel_cluster(mode, p->math_mode != 0, fin);
         if ((rc = cluster_shape(p, out->kernel, true, &sh))) return rc;
         out->mode = mode; out->place = RASTER_CLUSTER;
         out->raster = 0; out->n_stage = 0; out->filler = 0; out->dynamic = 0;
@@ -1395,7 +1440,7 @@ int plan_step(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io,
     while (follow_per_sm > 0 &&
            follow_per_sm * (follow_smem + 1024) + step_smem(p, 0, 1, mode) + 1024 > kMaxSmem) --follow_per_sm;
     const bool no_follower = (io->flags & SWARM_STEP_INKERNEL_RASTER) || env_flag("SWARM_B200_NO_FOLLOWER");
-    const StepKernel kernel = step_kernel(mode, p->math_mode != 0, RASTER_FOLLOW);     // the rasteriser-less kernel
+    const StepKernel kernel = step_kernel(mode, p->math_mode != 0, RASTER_FOLLOW, fin);     // the rasteriser-less kernel
     bool follow_fits = have_flags && !no_follower && follow_per_sm > 0 && follow_per_sm * follow_threads + nf <= 2048;
     int rgrid = 0;
     if (want_grid && follow_fits) {
@@ -1444,7 +1489,7 @@ int plan_step(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io,
     out->filler = (self && ((p->grid_size * p->grid_size) & 7) == 0 && (reinterpret_cast<uintptr_t>(io->grid) & 15) == 0 &&
                    nf + 32 <= kMaxThreads && E <= (long long)sms * (65536 / (64 * (nf + 32)))) ? 1 : 0;
     out->nt = nf + (warps ? raster_threads(N, A, nf, E, sms) : 0) + (out->filler ? 32 : 0);
-    out->kernel = step_kernel(mode, p->math_mode != 0, place);
+    out->kernel = step_kernel(mode, p->math_mode != 0, place, fin);
     if ((rc = prep(out->kernel, out->smem))) return rc;
     int grid = 0;
     if ((rc = persistent_grid(out->kernel, out->nt, out->smem, E, &grid))) return rc;
@@ -1475,10 +1520,39 @@ int swarm_step_plan(const SwarmParams* p, const SwarmState* st, const SwarmStepI
     return SWARM_OK;
 }
 
-int swarm_step(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io, const SwarmInjectedDraws* reset_draws,
-               swarm_stream_t stream) {
+// SwarmStateProcessor.process_state of the batch (or of the envs with mask[e] != 0): swarm_rasterize's launches.
+static int rasterize_launch(const SwarmParams* p, const double* x, const double* xa, float* grid, uint8_t* positions,
+                            double* box, const uint8_t* mask, swarm_stream_t stream) {
+    int rc = 0;
+    const KP kp = make_kp(p);
+    if (tuning_cluster(p)) {
+        const cudaStream_t s = (cudaStream_t)stream;
+        ClusterShape sh;
+        auto go = [&](auto kernel) {
+            int r = cluster_shape(p, kernel, false, &sh);
+            return r ? r : launch_cluster(kernel, sh, kp.E, s, "swarm_rasterize", kp, x, xa, grid, positions, box, sh.nf, mask);
+        };
+        if (force_mode(kp.N) == 2) return box ? go(k_rasterize_cluster<2, true>) : go(k_rasterize_cluster<2, false>);
+        return box ? go(k_rasterize_cluster<4, true>) : go(k_rasterize_cluster<4, false>);
+    }
+    const size_t smem = smem_bytes(kp.N, kp.A, kp.G, 0, false, 1, 0);
+    const int nt = (kp.N + kp.A) <= 128 ? 64 : 128;
+    if (box) {
+        if ((rc = prep(k_rasterize<true>, smem))) return rc;
+        k_rasterize<true><<<kp.E, nt, smem, (cudaStream_t)stream>>>(kp, x, xa, grid, positions, box, mask);
+    } else {
+        if ((rc = prep(k_rasterize<false>, smem))) return rc;
+        k_rasterize<false><<<kp.E, nt, smem, (cudaStream_t)stream>>>(kp, x, xa, grid, positions, box, mask);
+    }
+    return check_launch("swarm_rasterize");
+}
+
+// swarm_step's launches; with terminal outputs (fin_out != NULL) the FIN variants of the step kernels
+static int step_launch(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io, const SwarmStepFinal* fin_out,
+                       const SwarmInjectedDraws* reset_draws, swarm_stream_t stream) {
     StepPlan pl;
-    int rc = plan_step(p, st, io, reset_draws, &pl);
+    int rc = plan_step(p, st, io, reset_draws, &pl, fin_out != nullptr);
+    const SwarmStepFinal fin = fin_out ? *fin_out : kNoFinal;
     if (rc) return rc;
     KP kp = make_kp(p, pl.mode);
     kp.raster = pl.raster;
@@ -1495,7 +1569,7 @@ int swarm_step(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io
     const size_t smem = pl.smem, follow_smem = pl.follow_smem;
     if (pl.place == RASTER_CLUSTER) {      // no PDL: a cluster launch is an ordinary dependent of its predecessor
         const ClusterShape sh = {pl.cluster, nf, nt, smem};
-        return launch_cluster(kernel, sh, p->n_envs, s, "swarm_step", kp, *st, *io, dr, has, nf);
+        return launch_cluster(kernel, sh, p->n_envs, s, "swarm_step", kp, *st, *io, dr, has, nf, fin);
     }
     if (pl.place != RASTER_FOLLOW) {
         // Single-kernel shapes are launched as programmatic dependents of whatever precedes them in the stream: when that is
@@ -1516,7 +1590,7 @@ int swarm_step(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io
         const bool pdl = !no_pdl && (pl.place == RASTER_WARPS ? p->n_envs <= sms
                                                                : (p->n_locusts < 160 || p->n_envs <= 2 * sms));
         if (!pdl) {
-            kernel<<<grid, nt, smem, s>>>(kp, *st, *io, dr, has, nf);
+            kernel<<<grid, nt, smem, s>>>(kp, *st, *io, dr, has, nf, fin);
             return check_launch("swarm_step");
         }
         cudaLaunchConfig_t cfg;
@@ -1530,7 +1604,7 @@ int swarm_step(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io
         attr[0].val.programmaticStreamSerializationAllowed = 1;
         cfg.attrs = attr;
         cfg.numAttrs = 1;
-        const cudaError_t le = cudaLaunchKernelEx(&cfg, kernel, kp, *st, *io, dr, has, nf);
+        const cudaError_t le = cudaLaunchKernelEx(&cfg, kernel, kp, *st, *io, dr, has, nf, fin);
         if (le != cudaSuccess) return cuda_fail(le, "swarm_step (cudaLaunchKernelEx)");
         return check_launch("swarm_step");
     }
@@ -1564,7 +1638,7 @@ int swarm_step(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io
     err = cudaEventRecord(ss.fork, s);
     if (err == cudaSuccess) err = cudaStreamWaitEvent(ss.stream, ss.fork, 0);
     if (err != cudaSuccess) return cuda_fail(err, "fork");
-    kernel<<<grid, nt, smem, s>>>(kp, *st, *io, dr, has, nf);
+    kernel<<<grid, nt, smem, s>>>(kp, *st, *io, dr, has, nf, fin);
     if ((rc = check_launch("swarm_step"))) return rc;
     k_raster_follow<<<rgrid, follow_threads, follow_smem, ss.stream>>>(kp, st->x, st->xa, io->grid, io->positions,
                                                                         st->work + 2);
@@ -1573,6 +1647,25 @@ int swarm_step(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io
     if (err == cudaSuccess) err = cudaStreamWaitEvent(s, ss.join, 0);
     if (err != cudaSuccess) return cuda_fail(err, "join");
     return check_launch("swarm_step");
+}
+
+int swarm_step(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io, const SwarmInjectedDraws* reset_draws,
+               swarm_stream_t stream) {
+    return step_launch(p, st, io, nullptr, reset_draws, stream);
+}
+
+int swarm_step_final(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io, const SwarmStepFinal* fin,
+                     const SwarmInjectedDraws* reset_draws, swarm_stream_t stream) {
+    if (!fin) return step_launch(p, st, io, nullptr, reset_draws, stream);
+    if ((fin->grid != nullptr) != (fin->positions != nullptr)) return SWARM_ERR_FLAGS;
+    if (fin->grid && (!fin->x || !fin->xa || !grid_aligned(fin->grid))) return SWARM_ERR_FLAGS;
+    int rc = step_launch(p, st, io, fin, reset_draws, stream);
+    if (rc || !fin->grid) return rc;
+    // The terminal observations: the standalone rasteriser over the done envs, as an ORDINARY launch behind the step (and
+    // the follower's join), so it reads fin->x / io->done only once the step grid has completed -- k_step triggers its
+    // programmatic dependents early, this kernel is not one.  The next step's PDL launch then depends on this kernel
+    // and waits (griddepcontrol.wait) for its completion before touching the state, done or grid.
+    return rasterize_launch(p, fin->x, fin->xa, fin->grid, fin->positions, nullptr, io->done, stream);
 }
 
 void swarm_step_host_clear(void) { host_cache().clear(); }
@@ -1701,27 +1794,7 @@ int swarm_rasterize(const SwarmParams* p, const double* x, const double* xa, flo
     if (!x || !grid) return SWARM_ERR_NULL;
     if (p->n_agents > 0 && (!xa || !positions)) return SWARM_ERR_NULL;
     if (!grid_aligned(grid)) return SWARM_ERR_FLAGS;
-    const KP kp = make_kp(p);
-    if (tuning_cluster(p)) {
-        const cudaStream_t s = (cudaStream_t)stream;
-        ClusterShape sh;
-        auto go = [&](auto kernel) {
-            int r = cluster_shape(p, kernel, false, &sh);
-            return r ? r : launch_cluster(kernel, sh, kp.E, s, "swarm_rasterize", kp, x, xa, grid, positions, box, sh.nf);
-        };
-        if (force_mode(kp.N) == 2) return box ? go(k_rasterize_cluster<2, true>) : go(k_rasterize_cluster<2, false>);
-        return box ? go(k_rasterize_cluster<4, true>) : go(k_rasterize_cluster<4, false>);
-    }
-    const size_t smem = smem_bytes(kp.N, kp.A, kp.G, 0, false, 1, 0);
-    const int nt = (kp.N + kp.A) <= 128 ? 64 : 128;
-    if (box) {
-        if ((rc = prep(k_rasterize<true>, smem))) return rc;
-        k_rasterize<true><<<kp.E, nt, smem, (cudaStream_t)stream>>>(kp, x, xa, grid, positions, box);
-    } else {
-        if ((rc = prep(k_rasterize<false>, smem))) return rc;
-        k_rasterize<false><<<kp.E, nt, smem, (cudaStream_t)stream>>>(kp, x, xa, grid, positions, box);
-    }
-    return check_launch("swarm_rasterize");
+    return rasterize_launch(p, x, xa, grid, positions, box, nullptr, stream);
 }
 
 int swarm_expand_obs(const SwarmParams* p, const float* grid, const uint8_t* positions, float* expanded,

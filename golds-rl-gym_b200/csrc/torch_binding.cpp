@@ -1,5 +1,5 @@
 // libswarm_b200_torch.so -- the C ABI of include/swarm_b200.h exposed as a PyTorch extension:
-//   torch.ops.swarm_b200.{step, step_host, reset, rasterize, expand_obs, clip_actions, forces}
+//   torch.ops.swarm_b200.{step, step_final, step_host, reset, rasterize, expand_obs, clip_actions, forces}
 // Each op checks device / dtype / contiguity / shape of its tensors, takes the CURRENT CUDA stream of
 // the tensors' device and forwards plain pointers to the extern "C" entry point of libswarm_b200.so.
 // No arithmetic happens here.  `params` is a CPU uint8 tensor holding the SwarmParams POD
@@ -128,6 +128,40 @@ void op_step(const at::Tensor& params, at::Tensor x, at::Tensor xa, at::Tensor n
     check(swarm_step(&p, &st, &io, reset_draws.size() ? &dr : nullptr, stream_of(x)), "swarm_step");
 }
 
+// op_step + what the auto-reset overwrites (swarm_step_final): the done split, the terminal state and, with final_grid,
+// the terminal observation of the envs that are done
+void op_step_final(const at::Tensor& params, at::Tensor x, at::Tensor xa, at::Tensor noise_x, at::Tensor noise_a,
+                   at::Tensor elapsed, at::Tensor episode, c10::optional<at::Tensor> work, at::Tensor actions,
+                   c10::optional<at::Tensor> noise_a_step, c10::optional<at::Tensor> noise_x_step, at::Tensor reward,
+                   at::Tensor done, c10::optional<at::Tensor> grid, c10::optional<at::Tensor> positions,
+                   c10::optional<at::Tensor> v_out, int64_t flags, at::TensorList reset_draws,
+                   c10::optional<at::Tensor> final_x, c10::optional<at::Tensor> final_xa,
+                   c10::optional<at::Tensor> terminated, c10::optional<at::Tensor> truncated,
+                   c10::optional<at::Tensor> final_grid, c10::optional<at::Tensor> final_positions) {
+    const SwarmParams p = unpack(params);
+    c10::cuda::CUDAGuard guard(x.device());
+    const SwarmState st = make_state(p, x, xa, noise_x, noise_a, elapsed, episode, work);
+    const SwarmStepIO io = make_io(p, actions, noise_a_step, noise_x_step, reward, done, grid, positions, v_out, flags);
+    const int64_t E = p.n_envs, N = p.n_locusts, A = p.n_agents, G = p.grid_size;
+    if (final_x.has_value()) need(*final_x, at::kDouble, {E, N, 2}, "final_x");
+    if (final_xa.has_value()) need(*final_xa, at::kDouble, {E, A, 2}, "final_xa");
+    if (terminated.has_value()) need(*terminated, at::kByte, {E}, "terminated");
+    if (truncated.has_value()) need(*truncated, at::kByte, {E}, "truncated");
+    if (final_grid.has_value()) need(*final_grid, at::kFloat, {E, G, G, 2}, "final_grid");
+    if (final_positions.has_value()) need(*final_positions, at::kByte, {E, A, 2}, "final_positions");
+    bool same = actions.get_device() == x.get_device() && reward.get_device() == x.get_device() &&
+                done.get_device() == x.get_device();
+    for (const c10::optional<at::Tensor>* t : {&grid, &positions, &final_x, &final_xa, &terminated, &truncated, &final_grid,
+                                               &final_positions})
+        same = same && (!t->has_value() || (*t)->get_device() == x.get_device());
+    TORCH_CHECK(same, "step_final: all tensors must be on x's device");
+    SwarmInjectedDraws dr;
+    if (reset_draws.size()) dr = make_draws(p, reset_draws);
+    const SwarmStepFinal fin{ptr<double>(final_x), ptr<double>(final_xa), ptr<uint8_t>(terminated), ptr<uint8_t>(truncated),
+                             ptr<float>(final_grid), ptr<uint8_t>(final_positions)};
+    check(swarm_step_final(&p, &st, &io, &fin, reset_draws.size() ? &dr : nullptr, stream_of(x)), "swarm_step_final");
+}
+
 void op_reset(const at::Tensor& params, at::Tensor x, at::Tensor xa, at::Tensor noise_x, at::Tensor noise_a, at::Tensor elapsed,
               at::Tensor episode, c10::optional<at::Tensor> mask, at::TensorList draws) {
     const SwarmParams p = unpack(params);
@@ -199,6 +233,12 @@ TORCH_LIBRARY(swarm_b200, m) {
           "Tensor(f!) episode, Tensor(m!)? work, Tensor(g!) actions, Tensor? noise_a_step, Tensor? noise_x_step, Tensor(h!) reward, "
           "Tensor(i!) done, Tensor(j!)? grid, Tensor(k!)? positions, Tensor(l!)? v_out, int flags, Tensor[] reset_draws) -> ()",
           &op_step);
+    m.def("step_final(Tensor params, Tensor(a!) x, Tensor(b!) xa, Tensor(c!) noise_x, Tensor(d!) noise_a, Tensor(e!) elapsed, "
+          "Tensor(f!) episode, Tensor(m!)? work, Tensor(g!) actions, Tensor? noise_a_step, Tensor? noise_x_step, "
+          "Tensor(h!) reward, Tensor(i!) done, Tensor(j!)? grid, Tensor(k!)? positions, Tensor(l!)? v_out, int flags, "
+          "Tensor[] reset_draws, Tensor(n!)? final_x, Tensor(o!)? final_xa, Tensor(p!)? terminated, Tensor(q!)? truncated, "
+          "Tensor(r!)? final_grid, Tensor(s!)? final_positions) -> ()",
+          &op_step_final);
     m.def("reset(Tensor params, Tensor(a!) x, Tensor(b!) xa, Tensor(c!) noise_x, Tensor(d!) noise_a, Tensor(e!) elapsed, "
           "Tensor(f!) episode, Tensor? mask, Tensor[] draws) -> ()", &op_reset);
     m.def("rasterize(Tensor params, Tensor x, Tensor? xa, Tensor(a!) grid, Tensor(b!)? positions, Tensor(c!)? box) -> ()",

@@ -77,6 +77,10 @@ class BatchedSwarmEnv(object):
     With ``auto_reset=True`` finished envs are reset inside the step (SwarmRunner._run semantics).
     With ``noise="fresh"`` every step draws the next row of the episode's noise tables (the reference with
     SURVEY Q1 fixed) instead of re-using row N_BURN_IN; the default ``"frozen"`` is the reference as it is.
+    With ``final_obs=True`` step() also keeps what the auto-reset overwrites (swarm_step_final) and returns it as the info
+    dict: ``terminated`` (reward >= 0) and ``truncated`` (TimeLimit) as (E,) bool, and for the envs that are done the
+    terminal state ``final_x`` / ``final_xa`` and, when rasterising, its observation ``final_grid`` / ``final_positions``
+    (the rows of the other envs keep their old bytes).  They alias buffers of the env, like reward and done.
     """
 
     # fed_gym/envs/multiagent.py:8-21
@@ -92,7 +96,7 @@ class BatchedSwarmEnv(object):
 
     def __init__(self, num_envs, n_locusts=None, n_agents=None, grid_size=84, max_episode_steps=128,
                  seed=0, env_id_offset=0, device=None, math_mode="fast", auto_reset=True, rasterize=True,
-                 binding="torch", tuning=0, noise="frozen", cluster=None):
+                 binding="torch", tuning=0, noise="frozen", cluster=None, final_obs=False):
         """binding: "torch" = the hot calls go through torch.ops.swarm_b200.* (the C ABI as a PyTorch
         extension, csrc/torch_binding.cpp), "ctypes" = straight into the C ABI.  Same kernels either way.
         tuning: SwarmParams.tuning (0 = automatic launch shape; anything else only changes speed, never bits).
@@ -154,6 +158,20 @@ class BatchedSwarmEnv(object):
         self._was_reset = False
         self._blob_bytes, self._blob_t = None, None
         self._ctx = _on(self.device)
+        self.final_obs = bool(final_obs)
+        self.final_x = self.final_xa = self.terminated = self.truncated = None
+        self.final_grid = self.final_positions = None
+        if self.final_obs:
+            self.final_x = torch.zeros(E, N, 2, dtype=f64, device=d)
+            self.final_xa = torch.zeros(E, A, 2, dtype=f64, device=d)
+            self.terminated = torch.zeros(E, dtype=torch.uint8, device=d)
+            self.truncated = torch.zeros(E, dtype=torch.uint8, device=d)
+            if self.rasterize:
+                self.final_grid = torch.zeros(E, G, G, 2, dtype=torch.float32, device=d)
+                self.final_positions = torch.zeros(E, A, 2, dtype=torch.uint8, device=d)
+            self._fin = nat.SwarmStepFinal(_ptr(self.final_x), _ptr(self.final_xa), _ptr(self.terminated),
+                                           _ptr(self.truncated), None, None)
+            self._fin_ref = ctypes.byref(self._fin)
         self.refresh_params()
 
     def refresh_params(self):
@@ -190,13 +208,16 @@ class BatchedSwarmEnv(object):
         return self.x, self.xa
 
     def step(self, actions, noise_a=None, noise_x=None, clip=False, reset_draws=None, v_out=None,
-             rasterize=None, auto_reset=None, grid_out=None, positions_out=None, add_wind=True):
+             rasterize=None, auto_reset=None, grid_out=None, positions_out=None, add_wind=True,
+             final_grid_out=None, final_positions_out=None):
         """One env step for the whole batch; a single kernel launch.
 
         actions: (E,A,2) float32 or float64 CUDA tensor (float32 is the PAAC shared_actions dtype).
         With clip=True actions with |a|>=1 are normalised IN PLACE first (transform_actions_for_env).
         grid_out / positions_out: optional (E,G,G,2) f32 / (E,A,2) u8 tensors that receive the observation
         instead of self.grid / self.positions (e.g. a slot of a rollout ring).
+        final_grid_out / final_positions_out: the same for the terminal observation (final_obs=True).
+        With final_obs=True the 4th element is the info dict of the terminal outputs (see the class), else {}.
         """
         if not self._was_reset:
             # the reference raises TypeError unpacking self.states=None (multiagent.py:31)
@@ -212,6 +233,13 @@ class BatchedSwarmEnv(object):
                 raise ValueError("actions must be float32 or float64")
             g_t = (grid_out if grid_out is not None else self.grid) if rasterize else None
             p_t = (positions_out if positions_out is not None else self.positions) if rasterize else None
+            if self.final_obs:
+                fg, fp = self._final_obs_bufs(rasterize, final_grid_out, final_positions_out)
+                self.ops.step_final(self._blob, *self._state_t, actions, noise_a, noise_x, self.reward, self.done_u8,
+                                    g_t, p_t, v_out, flags,
+                                    reset_draws.tensors() if reset_draws is not None else [],
+                                    self.final_x, self.final_xa, self.terminated, self.truncated, fg, fp)
+                return (self.x, self.xa), self.reward, self._done_view, self._info(fg, fp)
             self.ops.step(self._blob, *self._state_t, actions, noise_a, noise_x, self.reward, self.done_u8,
                           g_t, p_t, v_out, flags,
                           reset_draws.tensors() if reset_draws is not None else [])
@@ -233,6 +261,16 @@ class BatchedSwarmEnv(object):
             io.grid, io.positions = None, None
         io.v_out = v_out.data_ptr() if v_out is not None else None
         io.flags = flags
+        if self.final_obs:
+            fg, fp = self._final_obs_bufs(rasterize, final_grid_out, final_positions_out)
+            self._fin.grid, self._fin.positions = _ptr(fg), _ptr(fp)
+            with self._ctx:
+                rc = self.lib.swarm_step_final(self._params_ref, self._state_ref, self._io_ref, self._fin_ref,
+                                               ctypes.byref(reset_draws.c) if reset_draws is not None else None,
+                                               torch.cuda.current_stream(self.device).cuda_stream)
+            if rc:
+                nat.check(rc, "swarm_step_final")
+            return (self.x, self.xa), self.reward, self._done_view, self._info(fg, fp)
         with self._ctx:
             rc = self.lib.swarm_step(self._params_ref, self._state_ref, self._io_ref,
                                      ctypes.byref(reset_draws.c) if reset_draws is not None else None,
@@ -240,6 +278,27 @@ class BatchedSwarmEnv(object):
         if rc:
             nat.check(rc, "swarm_step")
         return (self.x, self.xa), self.reward, self._done_view, {}
+
+    def _final_obs_bufs(self, rasterize, grid_out, positions_out):
+        """The terminal observation's targets of one step: the overrides, else the env's own buffers (None, None when the
+        step does not rasterise)."""
+        if not rasterize:
+            return None, None
+        E, A, G = self.E, self.A, self.G
+        if self.final_grid is None and (grid_out is None or positions_out is None):      # built with rasterize=False
+            self.final_grid = torch.zeros(E, G, G, 2, dtype=torch.float32, device=self.device)
+            self.final_positions = torch.zeros(E, A, 2, dtype=torch.uint8, device=self.device)
+        fg = grid_out if grid_out is not None else self.final_grid
+        fp = positions_out if positions_out is not None else self.final_positions
+        for t, shape, dt, name in ((fg, (E, G, G, 2), torch.float32, "final_grid_out"),
+                                   (fp, (E, A, 2), torch.uint8, "final_positions_out")):
+            if t.device != self.device or t.dtype != dt or not t.is_contiguous() or tuple(t.shape) != shape:
+                raise ValueError("%s must be a contiguous %s tensor of shape %s on %s" % (name, dt, shape, self.device))
+        return fg, fp
+
+    def _info(self, fg, fp):
+        return {"terminated": self.terminated.view(torch.bool), "truncated": self.truncated.view(torch.bool),
+                "final_x": self.final_x, "final_xa": self.final_xa, "final_grid": fg, "final_positions": fp}
 
     def stagger_episodes(self, total_envs=None):
         """Opt-in de-synchronisation of the episode boundaries (NOT the reference's behaviour: there every emulator starts

@@ -132,6 +132,19 @@ typedef struct SwarmStepIO {
     uint32_t reserved;
 } SwarmStepIO;
 
+/* What an auto-resetting step overwrites, kept for the caller (swarm_step_final).  Every pointer is nullable.
+ * terminated / truncated are written for every env on every step (done == terminated | truncated; both may be 1);
+ * x / xa / grid / positions only for envs with done[e] -- the rows of the other envs keep their bytes.  The
+ * terminal state is the post-step state BEFORE the auto-reset (without SWARM_STEP_AUTO_RESET: the returned state). */
+typedef struct SwarmStepFinal {
+    double* x;                  /* (E,N,2) nullable: terminal locust positions of envs with done[e]               */
+    double* xa;                 /* (E,A,2) nullable                                                                */
+    uint8_t* terminated;        /* (E) nullable: reward >= 0                                                       */
+    uint8_t* truncated;         /* (E) nullable: max_episode_steps > 0 && elapsed >= max_episode_steps              */
+    float* grid;                /* (E,G,G,2) nullable: process_state of the terminal state (done envs); needs x, xa */
+    uint8_t* positions;         /* (E,A,2) required iff grid                                                       */
+} SwarmStepFinal;
+
 int swarm_abi_version(void);
 const char* swarm_strerror(int status);
 const char* swarm_last_cuda_error(void);
@@ -163,6 +176,17 @@ int swarm_reset(const SwarmParams* p, const SwarmState* st, const uint8_t* mask,
  * reset_draws: nullable; injected draws used by auto-reset instead of Philox. */
 int swarm_step(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io,
                const SwarmInjectedDraws* reset_draws, swarm_stream_t stream);
+
+/* swarm_step that also keeps the terminal step of every env whose episode ends (gymnasium's terminated / truncated
+ * and final observation): the step kernel splits done into fin->terminated / fin->truncated and copies a done env's
+ * post-step state to fin->x / fin->xa before the auto-reset overwrites it.  With fin->grid the standalone rasteriser
+ * then runs once more, after the step, over the done envs only (fin->x / fin->xa as its source, io->done as its mask;
+ * the other envs' CTAs read one byte and leave): bit for bit swarm_rasterize of the terminal state.  One or two
+ * more launches than swarm_step, on `stream`; capturable like it.  fin == NULL is exactly swarm_step.
+ * SWARM_ERR_FLAGS, before any launch: fin->grid without fin->positions, fin->x or fin->xa; fin->positions without
+ * fin->grid; fin->grid not 8-byte aligned. */
+int swarm_step_final(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io, const SwarmStepFinal* fin,
+                     const SwarmInjectedDraws* reset_draws, swarm_stream_t stream);
 
 /* The launch shape swarm_step would use for these arguments (no launch; needs the device for occupancy queries):
  * out = { force mode, filler warp (0/1), rasteriser placement (0 none, 1 follower kernel, 2 raster warps, 3 the step's

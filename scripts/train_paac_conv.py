@@ -5,7 +5,8 @@
     torchrun --nproc-per-node 8 scripts/train_paac_conv.py -ec 8192 --clip_norm=1    # config 5: env batch sharded
 
 Flag names and defaults are the reference's; additions: --n_locusts, --max_updates, --no_cuda_graph,
---reward_indexing, --mask_terminals, --fresh_noise.  '-d/--device' accepts the reference's '/gpu:0' spelling.
+--reward_indexing, --mask_terminals, --bootstrap_truncated, --fresh_noise.
+'-d/--device' accepts the reference's '/gpu:0' spelling.
 """
 import argparse
 import copy
@@ -95,6 +96,8 @@ def get_arg_parser():
     parser.add_argument('--no_cuda_graph', action='store_true')
     parser.add_argument('--reward_indexing', default='reference', choices=['reference', 'per_agent'])
     parser.add_argument('--mask_terminals', action='store_true')
+    parser.add_argument('--bootstrap_truncated', action='store_true',
+                        help="with --mask_terminals: bootstrap a TimeLimit truncation from V of the terminal observation")
     parser.add_argument('--fresh_noise', action='store_true',
                         help="advance the env noise row every step (SURVEY Q1 fixed); default: the reference's frozen row")
     parser.add_argument('--eval_every', default=30.0, type=float,
@@ -122,7 +125,7 @@ def main(args):
     learner = paac.GridPAACLearner(network_creator, env_creator, args, reward_indexing=args.reward_indexing,
                                    mask_terminals=args.mask_terminals, use_cuda_graph=not args.no_cuda_graph,
                                    compact_obs={"auto": "auto", "compact": True, "expanded": False}[args.obs],
-                                   net_precision=args.net_precision)
+                                   net_precision=args.net_precision, bootstrap_truncated=args.bootstrap_truncated)
 
     def on_signal(signum, frame):            # train_paac_conv.py:47-58
         learner.cleanup()
