@@ -33,6 +33,9 @@ SWARM_STEP_ACTIONS_F64 = 4
 SWARM_STEP_NO_ACTION_WIND = 8
 SWARM_STEP_INKERNEL_RASTER = 16
 SWARM_STEP_FRESH_NOISE = 32
+SWARM_PHYSICS_RESAMPLE = 1
+# the columns of a SwarmPhysics table row (SwarmParams' order)
+PHYSICS_COLUMNS = ("noise", "gravity", "wind", "F", "L", "dt")
 # SwarmParams.tuning: bits 4-5 = rasteriser placement (0 automatic); bits 8-12 = the cluster layout (0 one CTA per env,
 # 1..16 a thread-block cluster of K CTAs per env, 31 the library picks K; 512 < N <= 8192); every other bit must be 0
 TUNE_RASTER_FOLLOW, TUNE_RASTER_WARPS, TUNE_RASTER_SELF = 1 << 4, 2 << 4, 3 << 4
@@ -79,6 +82,11 @@ class SwarmStepFinal(ctypes.Structure):
                 ("grid", c_void_p), ("positions", c_void_p)]
 
 
+class SwarmPhysics(ctypes.Structure):
+    _fields_ = [("table", c_void_p), ("flags", c_uint32), ("reserved", c_uint32), ("lo", c_double * 6),
+                ("hi", c_double * 6)]
+
+
 # name -> (restype, argtypes); every symbol include/swarm_b200.h declares
 _P = ctypes.POINTER
 SYMBOLS = {
@@ -91,6 +99,13 @@ SYMBOLS = {
     "swarm_step_final": (c_int, [_P(SwarmParams), _P(SwarmState), _P(SwarmStepIO), _P(SwarmStepFinal),
                                  _P(SwarmInjectedDraws), c_void_p]),
     "swarm_step_plan": (c_int, [_P(SwarmParams), _P(SwarmState), _P(SwarmStepIO), c_void_p]),
+    "swarm_reset_physics": (c_int, [_P(SwarmParams), _P(SwarmState), _P(SwarmPhysics), c_void_p, _P(SwarmInjectedDraws),
+                                    c_void_p]),
+    "swarm_step_physics": (c_int, [_P(SwarmParams), _P(SwarmState), _P(SwarmStepIO), _P(SwarmStepFinal),
+                                   _P(SwarmPhysics), _P(SwarmInjectedDraws), c_void_p]),
+    "swarm_forces_physics": (c_int, [_P(SwarmParams), _P(SwarmPhysics), c_void_p, c_void_p, c_void_p, c_void_p,
+                                     c_void_p]),
+    "swarm_step_plan_physics": (c_int, [_P(SwarmParams), _P(SwarmState), _P(SwarmStepIO), _P(SwarmPhysics), c_void_p]),
     "swarm_step_host": (c_int, [_P(SwarmParams), _P(SwarmState), _P(SwarmStepIO), c_void_p, c_void_p, c_void_p,
                                 c_void_p, c_void_p, c_void_p]),
     "swarm_step_host_clear": (None, []),

@@ -7,6 +7,7 @@
 #include <stdlib.h>
 #include <stdlib.h>
 
+#include <cmath>
 #include <map>
 #include <mutex>
 #include <tuple>
@@ -21,9 +22,11 @@ namespace {
 
 // ------------------------------------------------------------------------------------------ kernels
 
-// Issue the cp.async copies of everything env e's step reads from HBM into stage buffer sg.
+// Issue the cp.async copies of everything env e's step reads from HBM into stage buffer sg (PHYS: and its physics row
+// into sg.ph).
+template <bool PHYS>
 __device__ __forceinline__ void prefetch_env(const Stage& sg, const KP& kp, const SwarmState& st, const SwarmStepIO& io,
-                                             const int e, const Grp& g) {
+                                             const int e, const Grp& g, const SwarmPhysics& phys) {
     const int N = kp.N, A = kp.A;
     const double2* gx = reinterpret_cast<const double2*>(st.x) + (size_t)e * N;
     for (int i = g.tid; i < N; i += g.n) cp_async<16>(sg.xs + i, gx + i);
@@ -42,6 +45,14 @@ __device__ __forceinline__ void prefetch_env(const Stage& sg, const KP& kp, cons
         cp_async<4>(sg.misc, st.elapsed + e);
         if (kp.fresh) cp_async<4>(sg.misc + 1, st.episode + e);
     }
+    if constexpr (PHYS) {
+        if (g.tid < 3) cp_async<16>(sg.ph + 2 * g.tid, phys.table + (size_t)e * kPhysCols + 2 * g.tid);
+    }
+}
+
+// PHYS kernels: the physics rows of the n_stage stage buffers, behind the smem_bytes(...) of the kernel's carve
+__device__ __forceinline__ double* phys_rows(unsigned char* smem_raw, size_t smem) {
+    return reinterpret_cast<double*>(smem_raw + smem);
 }
 
 // SwarmEnv._step + TimeLimit + SwarmRunner auto-reset + process_state for the whole batch.
@@ -61,10 +72,13 @@ __device__ __forceinline__ void prefetch_env(const Stage& sg, const KP& kp, cons
 // copied out of the stage buffer in the (rare) done branch before the auto-reset overwrites it.  Compile time, so that
 // swarm_step's kernels (FIN = false) stay exactly what they were: the same code behind a runtime branch re-schedules
 // the whole kernel and was measured to cost 2.8 % of the C4 step with the feature off (0.1703 -> 0.1751 ms).
-template <int MODE, bool PRECISE, int PLACE, bool FIN>
+// PHYS (swarm_step_physics): per-env physics.  Env e's row is prefetched with the env into its stage buffer's row, and
+// an auto-reset with SWARM_PHYSICS_RESAMPLE draws the new episode's row into it (and the table) before the burn-in.
+// Compile time for the same reason as FIN.
+template <int MODE, bool PRECISE, int PLACE, bool FIN, bool PHYS>
 __global__ void __maxnreg__(64) k_step(const KP kp, const SwarmState st, const SwarmStepIO io,
                                        const SwarmInjectedDraws dr, const int has_draws, const int n_force,
-                                       const SwarmStepFinal fin) {
+                                       const SwarmStepFinal fin, const SwarmPhysics phys) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int N = kp.N, A = kp.A;
     const int n_all = blockDim.x, n_raster = n_all - n_force;
@@ -72,6 +86,15 @@ __global__ void __maxnreg__(64) k_step(const KP kp, const SwarmState st, const S
     constexpr bool self_raster = PLACE == 3;       // the force group rasterises its own env after the step
     const bool filler = self_raster && kp.filler;  // ... while one extra warp issues / awaits the TMA zero fill
     Smem sm = carve(smem_raw, N, A, kp.G, kp.n_stage, true, ModeT<MODE>::SYM, raster ? 1 : (self_raster ? 2 : 0));
+    double* prow = nullptr;
+    if constexpr (PHYS)
+        prow = phys_rows(smem_raw, smem_bytes(N, A, kp.G, kp.n_stage, true, raster ? 1 : (self_raster ? 2 : 0), ModeT<MODE>::SYM));
+    // stage buffer b with its physics row
+    auto stage = [&](const int b) {
+        Stage s = stage_at(smem_raw, N, A, b);
+        if constexpr (PHYS) s.ph = prow + kPhysCols * b;
+        return s;
+    };
 
     // Env assignment: the first two envs of a CTA are static (blockIdx.x, + gridDim.x); with a work queue the
     // later ones are drawn from an atomic counter (index 2 * gridDim.x + ticket), which evens out the CTAs'
@@ -90,14 +113,14 @@ __global__ void __maxnreg__(64) k_step(const KP kp, const SwarmState st, const S
             if (filler) bar_arrive<BAR_FULL>(n_all);       // the table is clean: the filler warp may read its zeros
         }
         pdl_wait();                        // from here on the previous kernels' writes (state, actions, grid) are visible
-        if (e < kp.E) prefetch_env(stage_at(smem_raw, N, A, 0), kp, st, io, e, g);
+        if (e < kp.E) prefetch_env<PHYS>(stage(0), kp, st, io, e, g, phys);
         cp_async_commit();
         int it = 0;
         if (g.tid == 0) trace_mark(kp, blockIdx.x, TR_ENTRY);
         for (; e < kp.E; ++it) {
             int grabbed = 0;                       // the env after next: asked for now, needed an iteration later
             if (dyn && g.tid == 0) grabbed = 2 * (int)gridDim.x + (int)atomicAdd(work, 1u);
-            sm.st = stage_at(smem_raw, N, A, it & 1);
+            sm.st = stage(it & 1);
             cp_async_wait_all();
             g.sync();      // this env's stage buffer has landed; the other one and sm.nx are free again
             if (it == 0 && g.tid == 0) trace_mark(kp, blockIdx.x, TR_LOADED);
@@ -135,7 +158,7 @@ __global__ void __maxnreg__(64) k_step(const KP kp, const SwarmState st, const S
                 }
                 cp_async_commit();      // (an empty group with fresh noise: env_step's wait counts groups)
             }
-            if (e1 < kp.E) prefetch_env(stage_at(smem_raw, N, A, (it + 1) & 1), kp, st, io, e1, g);
+            if (e1 < kp.E) prefetch_env<PHYS>(stage((it + 1) & 1), kp, st, io, e1, g, phys);
             cp_async_commit();     // (possibly empty) group of the next env: env_step waits for all but this one
 
             // actions: HBM dtype -> FP64, optional clip (the owner thread of agent k also moves it)
@@ -181,8 +204,9 @@ __global__ void __maxnreg__(64) k_step(const KP kp, const SwarmState st, const S
             for (;;) {
                 // multiagent.py:30,35-36: _step(add_wind=False) leaves the action alone; the burn-in steps of a reset
                 // always go through step() with the default add_wind=True (multiagent.py:59-61)
-                const double reward = env_step<MODE, PRECISE, self_raster>(sm, kp, g, v_out, (r < 0 && !kp.wind_step) ? 0.0 : kp.wind,
-                                                              (r < 0 && it == 0) ? (long long)blockIdx.x : -1);
+                const double reward = env_step<MODE, PRECISE, self_raster, PHYS>(sm, kp, g, v_out,
+                                                                                  (r < 0 && !kp.wind_step) ? 0.0 : (PHYS ? sm.st.ph[2] : kp.wind),
+                                                                                  (r < 0 && it == 0) ? (long long)blockIdx.x : -1);
                 if (r < 0) {
                     // multiagent.py:44 done = reward >= 0; gym TimeLimit: done |= ++elapsed >= max_episode_steps
                     elapsed = sm.st.misc[0] + 1;
@@ -209,6 +233,11 @@ __global__ void __maxnreg__(64) k_step(const KP kp, const SwarmState st, const S
                     }
                     if (!(done && (io.flags & SWARM_STEP_AUTO_RESET))) break;      // group-uniform
                     ep = st.episode[e];
+                    // the new episode's physics: written after env_step's closing barrier (nobody reads the row any more),
+                    // visible after reset_begin's leading one -- before the first burn-in step moves anything
+                    if constexpr (PHYS) {
+                        if (phys.flags & SWARM_PHYSICS_RESAMPLE) phys_reset_row(sm.st.ph, phys, kp, e, ep, g.tid, true);
+                    }
                     rc = reset_begin(sm, kp, g, e, ep, has_draws != 0, dr);
                     v_out = nullptr;
                     elapsed = 0;
@@ -336,18 +365,24 @@ __global__ void __maxnreg__(64) k_step(const KP kp, const SwarmState st, const S
     }
 }
 
-// SwarmEnv._reset for the masked envs (one CTA per env).
-template <int MODE, bool PRECISE>
+// SwarmEnv._reset for the masked envs (one CTA per env).  PHYS: the env's row (drawn, with SWARM_PHYSICS_RESAMPLE)
+// governs the burn-in.
+template <int MODE, bool PRECISE, bool PHYS>
 __global__ void __maxnreg__(64) k_reset(const KP kp, const SwarmState st, const uint8_t* __restrict__ mask,
-                                        const SwarmInjectedDraws dr, const int has_draws) {
+                                        const SwarmInjectedDraws dr, const int has_draws, const SwarmPhysics phys) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int e = blockIdx.x;
     if (mask && !mask[e]) return;
-    const Smem sm = carve(smem_raw, kp.N, kp.A, kp.G, 1, true, ModeT<MODE>::SYM, 0);
+    Smem sm = carve(smem_raw, kp.N, kp.A, kp.G, 1, true, ModeT<MODE>::SYM, 0);
     const Grp g = {(int)threadIdx.x, (int)blockDim.x};
     const uint32_t ep = st.episode[e];
+    if constexpr (PHYS) {     // visible after reset_begin's leading barrier
+        sm.st.ph = phys_rows(smem_raw, smem_bytes(kp.N, kp.A, kp.G, 1, true, 0, ModeT<MODE>::SYM));
+        phys_reset_row(sm.st.ph, phys, kp, e, ep, g.tid, true);
+    }
     const ResetCtx rc = reset_begin(sm, kp, g, e, ep, has_draws != 0, dr);
-    for (int r = 0; !reset_row(sm, kp, g, rc, r, dr, st); ++r) env_step<MODE, PRECISE>(sm, kp, g, nullptr, kp.wind);
+    for (int r = 0; !reset_row(sm, kp, g, rc, r, dr, st); ++r)
+        env_step<MODE, PRECISE, false, PHYS>(sm, kp, g, nullptr, PHYS ? sm.st.ph[2] : kp.wind);
     double2* ox = reinterpret_cast<double2*>(st.x) + (size_t)e * kp.N;
     double2* oa = reinterpret_cast<double2*>(st.xa) + (size_t)e * kp.A;
     for (int i = g.tid; i < kp.N; i += g.n) ox[i] = sm.st.xs[i];
@@ -449,11 +484,11 @@ __global__ void __launch_bounds__(256) k_rasterize(const KP kp, const double* __
     }
 }
 
-// SwarmEnv.v_calculate for the batch (no integration; one CTA per env).
-template <int MODE, bool PRECISE>
+// SwarmEnv.v_calculate for the batch (no integration; one CTA per env).  PHYS: F, L, wind and gravity of the env's row.
+template <int MODE, bool PRECISE, bool PHYS>
 __global__ void __maxnreg__(64) k_forces(const KP kp, const double* __restrict__ x,
                                          const double* __restrict__ xa, float* __restrict__ v,
-                                         float* __restrict__ reward) {
+                                         float* __restrict__ reward, const SwarmPhysics phys) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int e = blockIdx.x;
     constexpr int T = ModeT<MODE>::T;
@@ -467,7 +502,8 @@ __global__ void __maxnreg__(64) k_forces(const KP kp, const double* __restrict__
     stage_locusts<MODE>(sm, kp, g);
     g.sync();
     float vx[T], vy[T];
-    pair_forces<MODE, PRECISE>(sm, kp, g, vx, vy);
+    if constexpr (PHYS) pair_forces<MODE, PRECISE>(sm, phys_kp(kp, phys.table + (size_t)e * kPhysCols), g, vx, vy);
+    else pair_forces<MODE, PRECISE>(sm, kp, g, vx, vy);
     energy_put<MODE>(sm, kp, g, vx, vy);
     if (v) {
 #pragma unroll
@@ -668,10 +704,11 @@ __device__ __forceinline__ void cl_store(const KP& kp, const CMap& m, double2* x
 
 // SwarmEnv._step + TimeLimit + auto-reset + process_state (k_step's contract) for the cluster layout.
 // FIN: k_step's; each CTA copies its own targets' terminal positions from pn[], rank 0 the agents' from sm.as.
-template <int MODE, bool PRECISE, bool FIN>
+// PHYS: k_step's; every CTA reads (or draws) the env's row into its own shared memory, rank 0 writes a drawn row back.
+template <int MODE, bool PRECISE, bool FIN, bool PHYS>
 __global__ void __maxnreg__(64) k_step_cluster(const KP kp, const SwarmState st, const SwarmStepIO io,
                                                const SwarmInjectedDraws dr, const int has_draws, const int nf,
-                                               const SwarmStepFinal fin) {
+                                               const SwarmStepFinal fin, const SwarmPhysics phys) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     constexpr int T = ModeT<MODE>::T;
     const int N = kp.N, A = kp.A, tid = (int)threadIdx.x;
@@ -683,6 +720,11 @@ __global__ void __maxnreg__(64) k_step_cluster(const KP kp, const SwarmState st,
     double2* xae = reinterpret_cast<double2*>(st.xa) + (size_t)e * A;
     const int elapsed0 = st.elapsed[e];
     const uint32_t episode0 = st.episode[e];
+    double* ph = nullptr;
+    if constexpr (PHYS) {       // the row, visible after the barrier in front of the first agent move
+        ph = phys_rows(smem_raw, cl_smem_bytes(N, A, kp.G, m.K, true));
+        if (tid < kPhysCols) ph[tid] = phys.table[(size_t)e * kPhysCols + tid];
+    }
     ClNoise nz{kp, st, &io, dr, {}, {}, 0u, e, has_draws != 0};
     nz.fresh_d.key = kp.key;
     nz.fresh_d.env = kp.env_off + (uint32_t)e;
@@ -725,11 +767,15 @@ __global__ void __maxnreg__(64) k_step_cluster(const KP kp, const SwarmState st,
         sm.act[k] = a;
         aclip = a;
     }
+    if constexpr (PHYS) __syncthreads();
     float* v_out = io.v_out ? io.v_out + (size_t)e * N * 2 : nullptr;
     int elapsed = 0;
     for (int r = -1;;) {
         double2 pn[T];
-        cl_step_forces<MODE, PRECISE>(sm, kp, m, xe, xae, (r < 0 && !kp.wind_step) ? 0.0 : kp.wind, r, nz, v_out, pn);
+        if constexpr (PHYS)
+            cl_step_forces<MODE, PRECISE>(sm, phys_kp(kp, ph), m, xe, xae, (r < 0 && !kp.wind_step) ? 0.0 : ph[2], r, nz, v_out, pn);
+        else
+            cl_step_forces<MODE, PRECISE>(sm, kp, m, xe, xae, (r < 0 && !kp.wind_step) ? 0.0 : kp.wind, r, nz, v_out, pn);
         cluster_sync();     // every CTA has read the old state (and its actions): the new one may be written
         cl_store(kp, m, xe, pn);
         const double reward = cl_reward(sm, kp, m);
@@ -749,6 +795,11 @@ __global__ void __maxnreg__(64) k_step_cluster(const KP kp, const SwarmState st,
                 if (done && fin.xa && lead && tid < A) reinterpret_cast<double2*>(fin.xa)[(size_t)e * A + tid] = sm.as[tid];
             }
             if (!(done && (io.flags & SWARM_STEP_AUTO_RESET))) break;      // cluster-uniform
+            // the new episode's row: nobody reads the old one since the cluster barrier above; published by the one
+            // that closes this iteration
+            if constexpr (PHYS) {
+                if (phys.flags & SWARM_PHYSICS_RESAMPLE) phys_reset_row(ph, phys, kp, e, episode0, tid, lead);
+            }
             cl_reset_begin(sm, kp, m, e, xe, nz);
             v_out = nullptr;
             elapsed = 0;
@@ -775,10 +826,11 @@ __global__ void __maxnreg__(64) k_step_cluster(const KP kp, const SwarmState st,
     cluster_sync();         // no CTA leaves while a peer may still read its shared memory
 }
 
-// SwarmEnv._reset for the masked envs, cluster layout.
-template <int MODE, bool PRECISE>
+// SwarmEnv._reset for the masked envs, cluster layout.  PHYS: k_reset's (rank 0 writes a drawn row back).
+template <int MODE, bool PRECISE, bool PHYS>
 __global__ void __maxnreg__(64) k_reset_cluster(const KP kp, const SwarmState st, const uint8_t* __restrict__ mask,
-                                                const SwarmInjectedDraws dr, const int has_draws, const int nf) {
+                                                const SwarmInjectedDraws dr, const int has_draws, const int nf,
+                                                const SwarmPhysics phys) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     constexpr int T = ModeT<MODE>::T;
     const int N = kp.N, A = kp.A, tid = (int)threadIdx.x;
@@ -789,6 +841,11 @@ __global__ void __maxnreg__(64) k_reset_cluster(const KP kp, const SwarmState st
     double2* xe = reinterpret_cast<double2*>(st.x) + (size_t)e * N;
     double2* xae = reinterpret_cast<double2*>(st.xa) + (size_t)e * A;
     const uint32_t ep = st.episode[e];
+    double* ph = nullptr;
+    if constexpr (PHYS) {       // visible after the cluster barrier in front of the first burn-in step
+        ph = phys_rows(smem_raw, cl_smem_bytes(N, A, kp.G, m.K, true));
+        phys_reset_row(ph, phys, kp, e, ep, tid, m.rank == 0);
+    }
     ClNoise nz{kp, st, nullptr, dr, {}, {}, 0u, e, has_draws != 0};
     nz.reset_d.key = kp.key;
     nz.reset_d.env = kp.env_off + (uint32_t)e;
@@ -797,7 +854,8 @@ __global__ void __maxnreg__(64) k_reset_cluster(const KP kp, const SwarmState st
     for (int r = 0; !cl_reset_row(sm, kp, m, e, r, st, nz); ++r) {
         cluster_sync();     // the state is in memory before any CTA reads it
         double2 pn[T];
-        cl_step_forces<MODE, PRECISE>(sm, kp, m, xe, xae, kp.wind, r, nz, nullptr, pn);
+        if constexpr (PHYS) cl_step_forces<MODE, PRECISE>(sm, phys_kp(kp, ph), m, xe, xae, ph[2], r, nz, nullptr, pn);
+        else cl_step_forces<MODE, PRECISE>(sm, kp, m, xe, xae, kp.wind, r, nz, nullptr, pn);
         cluster_sync();     // every CTA has read the old state
         cl_store(kp, m, xe, pn);
     }
@@ -811,10 +869,11 @@ __global__ void __maxnreg__(64) k_reset_cluster(const KP kp, const SwarmState st
     }
 }
 
-// SwarmEnv.v_calculate for the batch, cluster layout.
-template <int MODE, bool PRECISE>
+// SwarmEnv.v_calculate for the batch, cluster layout.  PHYS: k_forces'.
+template <int MODE, bool PRECISE, bool PHYS>
 __global__ void __maxnreg__(64) k_forces_cluster(const KP kp, const double* __restrict__ x, const double* __restrict__ xa,
-                                                 float* __restrict__ v, float* __restrict__ reward, const int nf) {
+                                                 float* __restrict__ v, float* __restrict__ reward, const int nf,
+                                                 const SwarmPhysics phys) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     constexpr int T = ModeT<MODE>::T;
     const CMap m = cl_map(nf);
@@ -825,7 +884,8 @@ __global__ void __maxnreg__(64) k_forces_cluster(const KP kp, const double* __re
     cl_stage<false>(sm, kp, xe, xae, 0.0);
     if (m.active) {
         float vx[T], vy[T];
-        cl_forces<MODE, PRECISE>(sm, kp, m, vx, vy);
+        if constexpr (PHYS) cl_forces<MODE, PRECISE>(sm, phys_kp(kp, phys.table + (size_t)e * kPhysCols), m, vx, vy);
+        else cl_forces<MODE, PRECISE>(sm, kp, m, vx, vy);
         if (v) {
 #pragma unroll
             for (int t = 0; t < T; ++t) {
@@ -1140,8 +1200,9 @@ int cluster_occupancy(Kern kernel, int K, int nt, size_t smem, int* out) {
 // the device can hold for the whole batch at once (cudaOccupancyMaxActiveClusters >= E: one wave), else the smallest K.
 // Measured (profiles/r04_cluster.md): K beyond one wave costs a second wave (8192 x 16: K = 6 2.18 ms, K = 7 4.32 ms),
 // and in multi-wave batches more CTAs per env only add the per-CTA work (N = 2048, E = 148: K = 1 0.67 ms, K = 4 0.95).
+// phys_bytes: the PHYS kernels' physics row behind the carve
 template <typename Kern>
-int cluster_shape(const SwarmParams* p, Kern kernel, bool force, ClusterShape* out) {
+int cluster_shape(const SwarmParams* p, Kern kernel, bool force, ClusterShape* out, size_t phys_bytes = 0) {
     const int N = p->n_locusts, cl = tuning_cluster(p);
     const int nf = block_threads(N, force_mode(N)), nw = nf >> 5;
     const bool pick = cl == kClusterAuto;
@@ -1150,7 +1211,8 @@ int cluster_shape(const SwarmParams* p, Kern kernel, bool force, ClusterShape* o
     for (int K = k_hi; K >= k_lo; --K) {
         if (!cl_fits(p, K, force)) continue;
         const int nt = cl_threads(nw, K);
-        const size_t smem = cl_smem_bytes(N, p->n_agents, p->grid_size, K, force);
+        const size_t smem = cl_smem_bytes(N, p->n_agents, p->grid_size, K, force) + phys_bytes;
+        if (smem > kMaxSmem) continue;
         int rc = prep(kernel, smem);
         if (rc) return rc;
         if (K > 8) {
@@ -1246,37 +1308,57 @@ T* mapped_host(T* host) {
 }
 
 typedef void (*StepKernel)(const KP, const SwarmState, const SwarmStepIO, const SwarmInjectedDraws, const int, const int,
-                           const SwarmStepFinal);
+                           const SwarmStepFinal, const SwarmPhysics);
 
-template <int PLACE, bool FIN>
+template <int PLACE, bool FIN, bool PHYS>
 StepKernel step_kernel_p(int mode, bool precise) {
     switch (mode) {
-        case 1: return precise ? k_step<1, true, PLACE, FIN> : k_step<1, false, PLACE, FIN>;
-        case 2: return precise ? k_step<2, true, PLACE, FIN> : k_step<2, false, PLACE, FIN>;
-        case 3: return precise ? k_step<3, true, PLACE, FIN> : k_step<3, false, PLACE, FIN>;
-        default: return precise ? k_step<4, true, PLACE, FIN> : k_step<4, false, PLACE, FIN>;
+        case 1: return precise ? k_step<1, true, PLACE, FIN, PHYS> : k_step<1, false, PLACE, FIN, PHYS>;
+        case 2: return precise ? k_step<2, true, PLACE, FIN, PHYS> : k_step<2, false, PLACE, FIN, PHYS>;
+        case 3: return precise ? k_step<3, true, PLACE, FIN, PHYS> : k_step<3, false, PLACE, FIN, PHYS>;
+        default: return precise ? k_step<4, true, PLACE, FIN, PHYS> : k_step<4, false, PLACE, FIN, PHYS>;
     }
 }
-template <bool FIN>
+template <bool FIN, bool PHYS>
 StepKernel step_kernel_f(int mode, bool precise, int place) {
-    return place == 2 ? step_kernel_p<2, FIN>(mode, precise)
-                      : (place == 3 ? step_kernel_p<3, FIN>(mode, precise) : step_kernel_p<0, FIN>(mode, precise));
+    return place == 2 ? step_kernel_p<2, FIN, PHYS>(mode, precise)
+                      : (place == 3 ? step_kernel_p<3, FIN, PHYS>(mode, precise) : step_kernel_p<0, FIN, PHYS>(mode, precise));
 }
-// place: RasterPlace (NONE / FOLLOW share the rasteriser-less kernel); fin: the swarm_step_final variant
-StepKernel step_kernel(int mode, bool precise, int place, bool fin) {
-    return fin ? step_kernel_f<true>(mode, precise, place) : step_kernel_f<false>(mode, precise, place);
+// place: RasterPlace (NONE / FOLLOW share the rasteriser-less kernel); fin: the swarm_step_final variant; phys: the
+// swarm_step_physics one
+StepKernel step_kernel(int mode, bool precise, int place, bool fin, bool phys) {
+    if (phys) return fin ? step_kernel_f<true, true>(mode, precise, place) : step_kernel_f<false, true>(mode, precise, place);
+    return fin ? step_kernel_f<true, false>(mode, precise, place) : step_kernel_f<false, false>(mode, precise, place);
 }
 
-StepKernel step_kernel_cluster(int mode, bool precise, bool fin) {
-    if (fin)
-        return mode == 2 ? (precise ? k_step_cluster<2, true, true> : k_step_cluster<2, false, true>)
-                         : (precise ? k_step_cluster<4, true, true> : k_step_cluster<4, false, true>);
-    return mode == 2 ? (precise ? k_step_cluster<2, true, false> : k_step_cluster<2, false, false>)
-                     : (precise ? k_step_cluster<4, true, false> : k_step_cluster<4, false, false>);
+template <bool FIN, bool PHYS>
+StepKernel step_kernel_cluster_f(int mode, bool precise) {
+    return mode == 2 ? (precise ? k_step_cluster<2, true, FIN, PHYS> : k_step_cluster<2, false, FIN, PHYS>)
+                     : (precise ? k_step_cluster<4, true, FIN, PHYS> : k_step_cluster<4, false, FIN, PHYS>);
+}
+StepKernel step_kernel_cluster(int mode, bool precise, bool fin, bool phys) {
+    if (phys) return fin ? step_kernel_cluster_f<true, true>(mode, precise) : step_kernel_cluster_f<false, true>(mode, precise);
+    return fin ? step_kernel_cluster_f<true, false>(mode, precise) : step_kernel_cluster_f<false, false>(mode, precise);
 }
 
 const SwarmInjectedDraws kNoDraws = {nullptr, nullptr, nullptr, nullptr, nullptr};
 const SwarmStepFinal kNoFinal = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
+const SwarmPhysics kNoPhysics = {nullptr, 0u, 0u, {0, 0, 0, 0, 0, 0}, {0, 0, 0, 0, 0, 0}};
+
+// SwarmPhysics' host checks (before any CUDA call)
+int check_physics(const SwarmPhysics* ph) {
+    if (!ph || !ph->table) return SWARM_ERR_NULL;
+    if ((reinterpret_cast<uintptr_t>(ph->table) & 15) || (ph->flags & ~SWARM_PHYSICS_RESAMPLE) || ph->reserved)
+        return SWARM_ERR_FLAGS;
+    if (ph->flags & SWARM_PHYSICS_RESAMPLE) {
+        for (int c = 0; c < kPhysCols; ++c) {
+            const double lo = ph->lo[c], hi = ph->hi[c];
+            if (!std::isfinite(lo) || !std::isfinite(hi) || !(lo <= hi) || !std::isfinite(hi - lo)) return SWARM_ERR_SIZE;
+        }
+        if (!(ph->lo[4] > 0.0)) return SWARM_ERR_SIZE;       // L: the pair force divides by it
+    }
+    return SWARM_OK;
+}
 
 bool draws_complete(const SwarmInjectedDraws* d) {
     return d->x0 && d->xa0 && d->burn_actions && d->agent_noise && d->particle_noise;
@@ -1329,38 +1411,62 @@ const char* swarm_last_cuda_error(void) { return g_cuda_err; }
 
 int swarm_validate(const SwarmParams* p) { return validate(p); }
 
-int swarm_reset(const SwarmParams* p, const SwarmState* st, const uint8_t* mask, const SwarmInjectedDraws* draws,
-                swarm_stream_t stream) {
-    int rc = validate(p);
-    if (rc) return rc;
+}  // extern "C"
+
+namespace {
+
+// swarm_reset's launches (PHYS: the k_reset* variants with per-env physics)
+template <bool PHYS>
+int reset_launch(const SwarmParams* p, const SwarmState* st, const SwarmPhysics& phys, const uint8_t* mask,
+                 const SwarmInjectedDraws* draws, swarm_stream_t stream) {
+    int rc = 0;
     if (!st || !st->x || !st->xa || !st->noise_x || !st->noise_a || !st->elapsed || !st->episode) return SWARM_ERR_NULL;
     if (draws && !draws_complete(draws)) return SWARM_ERR_NULL;
     const int mode = force_mode(p->n_locusts);
     const KP kp = make_kp(p, mode);
     cudaStream_t s = (cudaStream_t)stream;
+    const size_t phys_bytes = PHYS ? kPhysRowBytes : 0;
     if (tuning_cluster(p)) {
         const SwarmInjectedDraws dr = draws ? *draws : kNoDraws;
         const int has = draws ? 1 : 0;
         ClusterShape sh;
         auto go = [&](auto kernel) {
-            int r = cluster_shape(p, kernel, true, &sh);
-            return r ? r : launch_cluster(kernel, sh, kp.E, s, "swarm_reset", kp, *st, mask, dr, has, sh.nf);
+            int r = cluster_shape(p, kernel, true, &sh, phys_bytes);
+            return r ? r : launch_cluster(kernel, sh, kp.E, s, "swarm_reset", kp, *st, mask, dr, has, sh.nf, phys);
         };
-        if (mode == 2) return p->math_mode ? go(k_reset_cluster<2, true>) : go(k_reset_cluster<2, false>);
-        return p->math_mode ? go(k_reset_cluster<4, true>) : go(k_reset_cluster<4, false>);
+        if (mode == 2) return p->math_mode ? go(k_reset_cluster<2, true, PHYS>) : go(k_reset_cluster<2, false, PHYS>);
+        return p->math_mode ? go(k_reset_cluster<4, true, PHYS>) : go(k_reset_cluster<4, false, PHYS>);
     }
-    const size_t smem = step_smem(p, 0, 1, mode);
+    const size_t smem = step_smem(p, 0, 1, mode) + phys_bytes;
+    if (smem > kMaxSmem) return SWARM_ERR_SIZE;
     const int nt = block_threads(kp.N, mode);
     if (nt > kMaxThreads) return SWARM_ERR_SIZE;
     DISPATCH_T(mode,
         if (p->math_mode) {
-            if ((rc = prep(k_reset<TT, true>, smem))) return rc;
-            k_reset<TT, true><<<kp.E, nt, smem, s>>>(kp, *st, mask, draws ? *draws : kNoDraws, draws ? 1 : 0);
+            if ((rc = prep(k_reset<TT, true, PHYS>, smem))) return rc;
+            k_reset<TT, true, PHYS><<<kp.E, nt, smem, s>>>(kp, *st, mask, draws ? *draws : kNoDraws, draws ? 1 : 0, phys);
         } else {
-            if ((rc = prep(k_reset<TT, false>, smem))) return rc;
-            k_reset<TT, false><<<kp.E, nt, smem, s>>>(kp, *st, mask, draws ? *draws : kNoDraws, draws ? 1 : 0);
+            if ((rc = prep(k_reset<TT, false, PHYS>, smem))) return rc;
+            k_reset<TT, false, PHYS><<<kp.E, nt, smem, s>>>(kp, *st, mask, draws ? *draws : kNoDraws, draws ? 1 : 0, phys);
         })
     return check_launch("swarm_reset");
+}
+
+}  // namespace
+
+extern "C" {
+
+int swarm_reset(const SwarmParams* p, const SwarmState* st, const uint8_t* mask, const SwarmInjectedDraws* draws,
+                swarm_stream_t stream) {
+    const int rc = validate(p);
+    return rc ? rc : reset_launch<false>(p, st, kNoPhysics, mask, draws, stream);
+}
+
+int swarm_reset_physics(const SwarmParams* p, const SwarmState* st, const SwarmPhysics* phys, const uint8_t* mask,
+                        const SwarmInjectedDraws* draws, swarm_stream_t stream) {
+    int rc = validate(p);
+    if (!rc) rc = check_physics(phys);
+    return rc ? rc : reset_launch<true>(p, st, *phys, mask, draws, stream);
 }
 
 }  // extern "C"
@@ -1379,8 +1485,9 @@ struct StepPlan {
 
 // Validates the arguments of swarm_step and decides its launch shape (automatic, or forced through
 // SwarmParams::tuning).  Touches the GPU only for attribute / occupancy queries (cached per device).
+// phys: the PHYS kernels, with the physics rows of their stage buffers behind their shared memory.
 int plan_step(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io, const SwarmInjectedDraws* reset_draws,
-              StepPlan* out, const bool fin = false) {
+              StepPlan* out, const bool fin = false, const bool phys = false) {
     int rc = validate(p);
     if (rc) return rc;
     if (!st || !io) return SWARM_ERR_NULL;
@@ -1420,8 +1527,8 @@ int plan_step(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io,
     if (tuning_cluster(p)) {
         // one env per thread-block cluster; the observation (if any) comes from the cluster itself, st->work is not used
         ClusterShape sh;
-        out->kernel = step_kernel_cluster(mode, p->math_mode != 0, fin);
-        if ((rc = cluster_shape(p, out->kernel, true, &sh))) return rc;
+        out->kernel = step_kernel_cluster(mode, p->math_mode != 0, fin, phys);
+        if ((rc = cluster_shape(p, out->kernel, true, &sh, phys ? kPhysRowBytes : 0))) return rc;
         out->mode = mode; out->place = RASTER_CLUSTER;
         out->raster = 0; out->n_stage = 0; out->filler = 0; out->dynamic = 0;
         out->nf = sh.nf; out->nt = sh.nt; out->smem = sh.smem; out->cluster = sh.K;
@@ -1438,14 +1545,15 @@ int plan_step(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io,
     // raster CTAs per SM that keep pace with the step (measured at 4096 envs: N = 160: 4 -> 0.110 ms, 2 -> 0.118; N = 192 and up: 2)
     int follow_per_sm = (N + A) <= 128 ? 6 : (N < 192 ? 4 : 2);
     while (follow_per_sm > 0 &&
-           follow_per_sm * (follow_smem + 1024) + step_smem(p, 0, 1, mode) + 1024 > kMaxSmem) --follow_per_sm;
+           follow_per_sm * (follow_smem + 1024) + step_smem(p, 0, 1, mode) + (phys ? kPhysRowBytes : 0) + 1024 > kMaxSmem)
+        --follow_per_sm;
     const bool no_follower = (io->flags & SWARM_STEP_INKERNEL_RASTER) || env_flag("SWARM_B200_NO_FOLLOWER");
-    const StepKernel kernel = step_kernel(mode, p->math_mode != 0, RASTER_FOLLOW, fin);     // the rasteriser-less kernel
+    const StepKernel kernel = step_kernel(mode, p->math_mode != 0, RASTER_FOLLOW, fin, phys);     // the rasteriser-less kernel
     bool follow_fits = have_flags && !no_follower && follow_per_sm > 0 && follow_per_sm * follow_threads + nf <= 2048;
     int rgrid = 0;
     if (want_grid && follow_fits) {
         // registers: follow_per_sm follower CTAs must leave room for at least one step CTA on every SM
-        const size_t smem0 = step_smem(p, 0, 1, mode);
+        const size_t smem0 = step_smem(p, 0, 1, mode) + (phys ? kPhysRowBytes : 0);
         int o = 0;
         if ((rc = prep(kernel, smem0)) || (rc = occupancy(kernel, nf, smem0, &o))) return rc;
         if ((rc = prep(k_raster_follow, follow_smem))) return rc;
@@ -1455,7 +1563,8 @@ int plan_step(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io,
         if (follow_per_sm * follow_threads * rf + nf * rs > 65536) follow_fits = false;
         if (rgrid > sms * follow_per_sm) rgrid = sms * follow_per_sm;
     }
-    const bool warps_fit = nf + raster_threads(N, A, nf, E, sms) <= kMaxThreads && step_smem(p, 1, 2, mode) <= kMaxSmem;
+    const bool warps_fit = nf + raster_threads(N, A, nf, E, sms) <= kMaxThreads &&
+                           step_smem(p, 1, 2, mode) + (phys ? 2 * kPhysRowBytes : 0) <= kMaxSmem;
     int place = RASTER_NONE;
     if (want_grid) {
         const int forced = (p->tuning >> 4) & 3;
@@ -1480,7 +1589,7 @@ int plan_step(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io,
     out->mode = mode; out->place = place;
     out->raster = warps ? 1 : (self ? 2 : 0);
     out->n_stage = warps ? 2 : 1;         // one env per CTA (no raster warps): nothing to prefetch into a second buffer
-    out->smem = step_smem(p, out->raster, out->n_stage, mode);
+    out->smem = step_smem(p, out->raster, out->n_stage, mode) + (phys ? out->n_stage * kPhysRowBytes : 0);
     if (out->smem > kMaxSmem) return SWARM_ERR_SIZE;
     out->nf = nf;
     // SELF: one extra warp issues / awaits the TMA zero fill (possible when the grid is a whole number of 16-byte words
@@ -1489,7 +1598,7 @@ int plan_step(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io,
     out->filler = (self && ((p->grid_size * p->grid_size) & 7) == 0 && (reinterpret_cast<uintptr_t>(io->grid) & 15) == 0 &&
                    nf + 32 <= kMaxThreads && E <= (long long)sms * (65536 / (64 * (nf + 32)))) ? 1 : 0;
     out->nt = nf + (warps ? raster_threads(N, A, nf, E, sms) : 0) + (out->filler ? 32 : 0);
-    out->kernel = step_kernel(mode, p->math_mode != 0, place, fin);
+    out->kernel = step_kernel(mode, p->math_mode != 0, place, fin, phys);
     if ((rc = prep(out->kernel, out->smem))) return rc;
     int grid = 0;
     if ((rc = persistent_grid(out->kernel, out->nt, out->smem, E, &grid))) return rc;
@@ -1509,15 +1618,26 @@ int plan_step(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io,
 
 extern "C" {
 
-int swarm_step_plan(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io, int32_t out[8]) {
+static int step_plan_out(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io, const bool phys, int32_t out[8]) {
     if (!out) return SWARM_ERR_NULL;
     StepPlan pl;
-    const int rc = plan_step(p, st, io, nullptr, &pl);
+    const int rc = plan_step(p, st, io, nullptr, &pl, false, phys);
     if (rc) return rc;
     out[0] = pl.mode; out[1] = pl.filler; out[2] = pl.place; out[3] = pl.nt; out[4] = pl.grid;
     out[5] = (int32_t)pl.smem; out[6] = pl.place == RASTER_FOLLOW ? pl.rgrid : (pl.place == RASTER_CLUSTER ? pl.cluster : 0);
     out[7] = pl.place == RASTER_FOLLOW ? 2 : 1;
     return SWARM_OK;
+}
+
+int swarm_step_plan(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io, int32_t out[8]) {
+    return step_plan_out(p, st, io, false, out);
+}
+
+int swarm_step_plan_physics(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io, const SwarmPhysics* phys,
+                            int32_t out[8]) {
+    int rc = validate(p);
+    if (!rc) rc = check_physics(phys);
+    return rc ? rc : step_plan_out(p, st, io, true, out);
 }
 
 // SwarmStateProcessor.process_state of the batch (or of the envs with mask[e] != 0): swarm_rasterize's launches.
@@ -1547,12 +1667,14 @@ static int rasterize_launch(const SwarmParams* p, const double* x, const double*
     return check_launch("swarm_rasterize");
 }
 
-// swarm_step's launches; with terminal outputs (fin_out != NULL) the FIN variants of the step kernels
+// swarm_step's launches; with terminal outputs (fin_out != NULL) the FIN variants of the step kernels, with per-env
+// physics (phys_in != NULL, checked) the PHYS ones
 static int step_launch(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io, const SwarmStepFinal* fin_out,
-                       const SwarmInjectedDraws* reset_draws, swarm_stream_t stream) {
+                       const SwarmInjectedDraws* reset_draws, swarm_stream_t stream, const SwarmPhysics* phys_in = nullptr) {
     StepPlan pl;
-    int rc = plan_step(p, st, io, reset_draws, &pl, fin_out != nullptr);
+    int rc = plan_step(p, st, io, reset_draws, &pl, fin_out != nullptr, phys_in != nullptr);
     const SwarmStepFinal fin = fin_out ? *fin_out : kNoFinal;
+    const SwarmPhysics phys = phys_in ? *phys_in : kNoPhysics;
     if (rc) return rc;
     KP kp = make_kp(p, pl.mode);
     kp.raster = pl.raster;
@@ -1569,7 +1691,7 @@ static int step_launch(const SwarmParams* p, const SwarmState* st, const SwarmSt
     const size_t smem = pl.smem, follow_smem = pl.follow_smem;
     if (pl.place == RASTER_CLUSTER) {      // no PDL: a cluster launch is an ordinary dependent of its predecessor
         const ClusterShape sh = {pl.cluster, nf, nt, smem};
-        return launch_cluster(kernel, sh, p->n_envs, s, "swarm_step", kp, *st, *io, dr, has, nf, fin);
+        return launch_cluster(kernel, sh, p->n_envs, s, "swarm_step", kp, *st, *io, dr, has, nf, fin, phys);
     }
     if (pl.place != RASTER_FOLLOW) {
         // Single-kernel shapes are launched as programmatic dependents of whatever precedes them in the stream: when that is
@@ -1590,7 +1712,7 @@ static int step_launch(const SwarmParams* p, const SwarmState* st, const SwarmSt
         const bool pdl = !no_pdl && (pl.place == RASTER_WARPS ? p->n_envs <= sms
                                                                : (p->n_locusts < 160 || p->n_envs <= 2 * sms));
         if (!pdl) {
-            kernel<<<grid, nt, smem, s>>>(kp, *st, *io, dr, has, nf, fin);
+            kernel<<<grid, nt, smem, s>>>(kp, *st, *io, dr, has, nf, fin, phys);
             return check_launch("swarm_step");
         }
         cudaLaunchConfig_t cfg;
@@ -1604,7 +1726,7 @@ static int step_launch(const SwarmParams* p, const SwarmState* st, const SwarmSt
         attr[0].val.programmaticStreamSerializationAllowed = 1;
         cfg.attrs = attr;
         cfg.numAttrs = 1;
-        const cudaError_t le = cudaLaunchKernelEx(&cfg, kernel, kp, *st, *io, dr, has, nf, fin);
+        const cudaError_t le = cudaLaunchKernelEx(&cfg, kernel, kp, *st, *io, dr, has, nf, fin, phys);
         if (le != cudaSuccess) return cuda_fail(le, "swarm_step (cudaLaunchKernelEx)");
         return check_launch("swarm_step");
     }
@@ -1638,7 +1760,7 @@ static int step_launch(const SwarmParams* p, const SwarmState* st, const SwarmSt
     err = cudaEventRecord(ss.fork, s);
     if (err == cudaSuccess) err = cudaStreamWaitEvent(ss.stream, ss.fork, 0);
     if (err != cudaSuccess) return cuda_fail(err, "fork");
-    kernel<<<grid, nt, smem, s>>>(kp, *st, *io, dr, has, nf, fin);
+    kernel<<<grid, nt, smem, s>>>(kp, *st, *io, dr, has, nf, fin, phys);
     if ((rc = check_launch("swarm_step"))) return rc;
     k_raster_follow<<<rgrid, follow_threads, follow_smem, ss.stream>>>(kp, st->x, st->xa, io->grid, io->positions,
                                                                         st->work + 2);
@@ -1654,18 +1776,31 @@ int swarm_step(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io
     return step_launch(p, st, io, nullptr, reset_draws, stream);
 }
 
-int swarm_step_final(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io, const SwarmStepFinal* fin,
-                     const SwarmInjectedDraws* reset_draws, swarm_stream_t stream) {
-    if (!fin) return step_launch(p, st, io, nullptr, reset_draws, stream);
+// swarm_step_final with optional per-env physics (phys checked by the caller)
+static int step_final_launch(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io, const SwarmStepFinal* fin,
+                             const SwarmInjectedDraws* reset_draws, swarm_stream_t stream, const SwarmPhysics* phys) {
+    if (!fin) return step_launch(p, st, io, nullptr, reset_draws, stream, phys);
     if ((fin->grid != nullptr) != (fin->positions != nullptr)) return SWARM_ERR_FLAGS;
     if (fin->grid && (!fin->x || !fin->xa || !grid_aligned(fin->grid))) return SWARM_ERR_FLAGS;
-    int rc = step_launch(p, st, io, fin, reset_draws, stream);
+    int rc = step_launch(p, st, io, fin, reset_draws, stream, phys);
     if (rc || !fin->grid) return rc;
     // The terminal observations: the standalone rasteriser over the done envs, as an ORDINARY launch behind the step (and
     // the follower's join), so it reads fin->x / io->done only once the step grid has completed -- k_step triggers its
     // programmatic dependents early, this kernel is not one.  The next step's PDL launch then depends on this kernel
     // and waits (griddepcontrol.wait) for its completion before touching the state, done or grid.
     return rasterize_launch(p, fin->x, fin->xa, fin->grid, fin->positions, nullptr, io->done, stream);
+}
+
+int swarm_step_final(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io, const SwarmStepFinal* fin,
+                     const SwarmInjectedDraws* reset_draws, swarm_stream_t stream) {
+    return step_final_launch(p, st, io, fin, reset_draws, stream, nullptr);
+}
+
+int swarm_step_physics(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io, const SwarmStepFinal* fin,
+                       const SwarmPhysics* phys, const SwarmInjectedDraws* reset_draws, swarm_stream_t stream) {
+    int rc = validate(p);
+    if (!rc) rc = check_physics(phys);
+    return rc ? rc : step_final_launch(p, st, io, fin, reset_draws, stream, phys);
 }
 
 void swarm_step_host_clear(void) { host_cache().clear(); }
@@ -1822,10 +1957,13 @@ int swarm_expand_obs(const SwarmParams* p, const float* grid, const uint8_t* pos
     return check_launch("swarm_expand_obs");
 }
 
-int swarm_forces(const SwarmParams* p, const double* x, const double* xa, float* v, float* reward,
-                 swarm_stream_t stream) {
-    int rc = validate(p);
-    if (rc) return rc;
+}  // extern "C"
+
+// swarm_forces' launches (PHYS: the k_forces* variants with per-env physics)
+template <bool PHYS>
+static int forces_launch(const SwarmParams* p, const SwarmPhysics& phys, const double* x, const double* xa, float* v,
+                         float* reward, swarm_stream_t stream) {
+    int rc = 0;
     if (!x || !xa || (!v && !reward)) return SWARM_ERR_NULL;
     const int mode = force_mode(p->n_locusts);
     const KP kp = make_kp(p, mode);
@@ -1834,23 +1972,38 @@ int swarm_forces(const SwarmParams* p, const double* x, const double* xa, float*
         ClusterShape sh;
         auto go = [&](auto kernel) {
             int r = cluster_shape(p, kernel, true, &sh);
-            return r ? r : launch_cluster(kernel, sh, kp.E, s, "swarm_forces", kp, x, xa, v, reward, sh.nf);
+            return r ? r : launch_cluster(kernel, sh, kp.E, s, "swarm_forces", kp, x, xa, v, reward, sh.nf, phys);
         };
-        if (mode == 2) return p->math_mode ? go(k_forces_cluster<2, true>) : go(k_forces_cluster<2, false>);
-        return p->math_mode ? go(k_forces_cluster<4, true>) : go(k_forces_cluster<4, false>);
+        if (mode == 2) return p->math_mode ? go(k_forces_cluster<2, true, PHYS>) : go(k_forces_cluster<2, false, PHYS>);
+        return p->math_mode ? go(k_forces_cluster<4, true, PHYS>) : go(k_forces_cluster<4, false, PHYS>);
     }
     const size_t smem = step_smem(p, 0, 1, mode);
     const int nt = block_threads(kp.N, mode);
     if (nt > kMaxThreads) return SWARM_ERR_SIZE;
     DISPATCH_T(mode,
         if (p->math_mode) {
-            if ((rc = prep(k_forces<TT, true>, smem))) return rc;
-            k_forces<TT, true><<<kp.E, nt, smem, s>>>(kp, x, xa, v, reward);
+            if ((rc = prep(k_forces<TT, true, PHYS>, smem))) return rc;
+            k_forces<TT, true, PHYS><<<kp.E, nt, smem, s>>>(kp, x, xa, v, reward, phys);
         } else {
-            if ((rc = prep(k_forces<TT, false>, smem))) return rc;
-            k_forces<TT, false><<<kp.E, nt, smem, s>>>(kp, x, xa, v, reward);
+            if ((rc = prep(k_forces<TT, false, PHYS>, smem))) return rc;
+            k_forces<TT, false, PHYS><<<kp.E, nt, smem, s>>>(kp, x, xa, v, reward, phys);
         })
     return check_launch("swarm_forces");
+}
+
+extern "C" {
+
+int swarm_forces(const SwarmParams* p, const double* x, const double* xa, float* v, float* reward,
+                 swarm_stream_t stream) {
+    const int rc = validate(p);
+    return rc ? rc : forces_launch<false>(p, kNoPhysics, x, xa, v, reward, stream);
+}
+
+int swarm_forces_physics(const SwarmParams* p, const SwarmPhysics* phys, const double* x, const double* xa, float* v,
+                         float* reward, swarm_stream_t stream) {
+    int rc = validate(p);
+    if (!rc) rc = check_physics(phys);
+    return rc ? rc : forces_launch<true>(p, *phys, x, xa, v, reward, stream);
 }
 
 int swarm_x_update(double* x, double* v, const double* noise, int64_t n, double dt, swarm_stream_t stream) {

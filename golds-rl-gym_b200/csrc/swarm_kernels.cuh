@@ -73,6 +73,7 @@ struct Stage {
     double2* an;            // A   agent noise row
     unsigned char* araw;    // A x 16 B: the env's actions as they sit in HBM (f32 pair or f64 pair)
     int* misc;              // [0] = TimeLimit elapsed steps, [1] = resets so far (fresh noise only)
+    double* ph;             // PHYS kernels: the env's physics row (6 doubles, behind the kernel's shared memory, see phys_rows)
 };
 
 struct Smem {
@@ -234,6 +235,62 @@ __device__ __forceinline__ void move_particle(double2& p, double2 v, double2 n, 
     p.x = __dadd_rn(p.x, __dadd_rn(__dmul_rn(dt, v.x), __dmul_rn(sigma, n.x)));
     p.y = __dadd_rn(p.y, __dadd_rn(__dmul_rn(dt, v.y), __dmul_rn(sigma, n.y)));
     if (p.y <= 0.0) p.y = 0.0;
+}
+
+// ------------------------------------------------------------------------------------------
+// Per-env physics (SwarmPhysics; the PHYS kernel instantiations).  A row is {noise, gravity, wind, F, L, dt} in
+// SwarmParams' order.  The PHYS kernels keep the row of each stage buffer in kPhysRowBytes behind the kernel's own shared
+// memory (so every other offset stays put) and take the env's constants from it with make_kp's roundings: a row equal to
+// SwarmParams gives the bits of the launch constants.
+constexpr int kPhysCols = 6;
+constexpr size_t kPhysRowBytes = sizeof(double) * kPhysCols;     // 48: three 16-byte cp.async pieces
+
+// kp with the constants of row ph (F and -1/L: make_kp's roundings; -1.0 / L == -RN(1 / L) exactly)
+__device__ __forceinline__ KP phys_kp(const KP& kp, const double* ph) {
+    KP k = kp;
+    k.sigma = ph[0];
+    k.wind = ph[2];
+    k.dt = ph[5];
+    k.Gv = (float)ph[1];
+    k.U = (float)ph[2];
+    k.F = (float)ph[3];
+    k.nInvL = (float)(-__drcp_rn(ph[4]));
+    return k;
+}
+
+// Column c of a SWARM_PHYSICS_RESAMPLE row: lo + (hi - lo) u, u from Philox stream 5 of the reset's DrawCtx.  The bounds
+// are picked with constant indices: a thread-dependent index into the kernel parameter would copy lo / hi to local memory.
+__device__ __forceinline__ double phys_draw(const DrawCtx& d, const SwarmPhysics& P, const int c) {
+    const double2 u = draw_uniform2(d, STREAM_PHYSICS, (uint32_t)(c >> 1));
+    double lo = P.lo[0], hi = P.hi[0];
+#pragma unroll
+    for (int i = 1; i < kPhysCols; ++i) {
+        if (c == i) {
+            lo = P.lo[i];
+            hi = P.hi[i];
+        }
+    }
+    return __dadd_rn(lo, __dmul_rn(__dadd_rn(hi, -lo), (c & 1) ? u.y : u.x));
+}
+
+// The row of env e's new episode into row (shared memory), by threads tid < 6: with SWARM_PHYSICS_RESAMPLE drawn (and
+// written back to the table when `store`), else the table's.  Visible to the other threads after their next barrier.
+__device__ __forceinline__ void phys_reset_row(double* row, const SwarmPhysics& P, const KP& kp, const int e,
+                                               const uint32_t episode, const int tid, const bool store) {
+    if (tid < kPhysCols) {
+        double v;
+        if (P.flags & SWARM_PHYSICS_RESAMPLE) {
+            DrawCtx d;
+            d.key = kp.key;
+            d.env = kp.env_off + (uint32_t)e;
+            d.episode = episode;
+            v = phys_draw(d, P, tid);
+            if (store) P.table[(size_t)e * kPhysCols + tid] = v;
+        } else {
+            v = P.table[(size_t)e * kPhysCols + tid];
+        }
+        row[tid] = v;
+    }
 }
 
 // Named barriers (bar.sync id, n) of the warp-specialised step kernel.  0 stays __syncthreads.
@@ -911,7 +968,8 @@ __device__ __forceinline__ double energy_get(const Smem& sm, const KP& kp, const
 // SwarmEnv._step on the stage buffer sm.st.  Preconditions: st.xs/as/an, sm.nx and sm.act filled, each
 // element written by the thread that owns it here (element i <-> thread i mod n) or visible through
 // a barrier.  Postcondition: state updated and visible to the whole group; returns the reward.
-template <int MODE, bool PRECISE, bool AGF = false>
+// PHYS: the physics constants come from the row sm.st.ph (visible to the group), read where they are used.
+template <int MODE, bool PRECISE, bool AGF = false, bool PHYS = false>
 __device__ __forceinline__ double env_step(const Smem& sm, const KP& kp, const Grp& g, float* v_out, const double wind_a,
                                            const long long trace_rec = -1) {
     constexpr int T = ModeT<MODE>::T;
@@ -922,14 +980,16 @@ __device__ __forceinline__ double env_step(const Smem& sm, const KP& kp, const G
         double2 a = sm.st.as[k];
         double2 w = sm.act[k];
         w.x = __dadd_rn(w.x, wind_a);
-        move_particle(a, w, sm.st.an[k], kp.dt, kp.sigma);
+        if constexpr (PHYS) move_particle(a, w, sm.st.an[k], sm.st.ph[5], sm.st.ph[0]);
+        else move_particle(a, w, sm.st.an[k], kp.dt, kp.sigma);
         sm.st.as[k] = a;
         ag[k] = split_hilo(a, kp.cscale);
     }
     stage_locusts<MODE>(sm, kp, g);
     g.sync();
     float vx[T], vy[T];
-    pair_forces<MODE, PRECISE, AGF>(sm, kp, g, vx, vy, trace_rec);
+    if constexpr (PHYS) pair_forces<MODE, PRECISE, AGF>(sm, phys_kp(kp, sm.st.ph), g, vx, vy, trace_rec);
+    else pair_forces<MODE, PRECISE, AGF>(sm, kp, g, vx, vy, trace_rec);
     if (g.tid == 0) trace_mark(kp, trace_rec, TR_FORCES);
     energy_put<MODE>(sm, kp, g, vx, vy);
     cp_async_wait_but_one();   // this thread's own noise rows have landed in sm.nx (no-op outside k_step)
@@ -940,7 +1000,8 @@ __device__ __forceinline__ double env_step(const Smem& sm, const KP& kp, const G
         if (j < kp.N) {
             if (v_out) reinterpret_cast<float2*>(v_out)[j] = make_float2(vx[t], vy[t]);
             double2 p = sm.st.xs[j];
-            move_particle(p, make_double2((double)vx[t], (double)vy[t]), sm.nx[j], kp.dt, kp.sigma);
+            if constexpr (PHYS) move_particle(p, make_double2((double)vx[t], (double)vy[t]), sm.nx[j], sm.st.ph[5], sm.st.ph[0]);
+            else move_particle(p, make_double2((double)vx[t], (double)vy[t]), sm.nx[j], kp.dt, kp.sigma);
             sm.st.xs[j] = p;
         }
     }

@@ -11,12 +11,14 @@
 //          3: agent noise (rows 0..n_burn + elapsed)   4: particle noise (rows 0..n_burn + elapsed)
 //   (rows 0..n_burn-1 feed the burn-in, row n_burn the first step after the reset -- and every later step
 //   in the frozen mode of the reference; with SWARM_STEP_FRESH_NOISE step `elapsed` uses row n_burn + elapsed)
+//   stream 5: the physics row of SWARM_PHYSICS_RESAMPLE (uniform pairs 0..2, row 0: column c is pair c / 2, .x / .y)
 #pragma once
 #include <stdint.h>
 
 namespace swarm {
 
-enum : uint32_t { STREAM_X0 = 0, STREAM_XA0 = 1, STREAM_BURN = 2, STREAM_NOISE_A = 3, STREAM_NOISE_X = 4 };
+enum : uint32_t { STREAM_X0 = 0, STREAM_XA0 = 1, STREAM_BURN = 2, STREAM_NOISE_A = 3, STREAM_NOISE_X = 4,
+                  STREAM_PHYSICS = 5 };
 
 __device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint2 k) {
 #pragma unroll

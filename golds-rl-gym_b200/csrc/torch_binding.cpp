@@ -1,5 +1,6 @@
 // libswarm_b200_torch.so -- the C ABI of include/swarm_b200.h exposed as a PyTorch extension:
-//   torch.ops.swarm_b200.{step, step_final, step_host, reset, rasterize, expand_obs, clip_actions, forces}
+//   torch.ops.swarm_b200.{step, step_final, step_host, reset, rasterize, expand_obs, clip_actions, forces,
+//                         reset_physics, step_physics, forces_physics}
 // Each op checks device / dtype / contiguity / shape of its tensors, takes the CURRENT CUDA stream of
 // the tensors' device and forwards plain pointers to the extern "C" entry point of libswarm_b200.so.
 // No arithmetic happens here.  `params` is a CPU uint8 tensor holding the SwarmParams POD
@@ -162,6 +163,23 @@ void op_step_final(const at::Tensor& params, at::Tensor x, at::Tensor xa, at::Te
     check(swarm_step_final(&p, &st, &io, &fin, reset_draws.size() ? &dr : nullptr, stream_of(x)), "swarm_step_final");
 }
 
+// SwarmPhysics of the *_physics ops: the (E,6) f64 table on x's device, the flags and the per-column ranges
+SwarmPhysics make_physics(const SwarmParams& p, const at::Tensor& table, int64_t flags, at::ArrayRef<double> lo,
+                          at::ArrayRef<double> hi, const at::Tensor& x) {
+    need(table, at::kDouble, {p.n_envs, 6}, "physics");
+    TORCH_CHECK(table.get_device() == x.get_device(), "physics is on another device than x");
+    TORCH_CHECK(lo.size() == 6 && hi.size() == 6, "physics_lo and physics_hi must have 6 entries");
+    SwarmPhysics ph;
+    std::memset(&ph, 0, sizeof(ph));
+    ph.table = table.data_ptr<double>();
+    ph.flags = (uint32_t)flags;
+    for (int c = 0; c < 6; ++c) {
+        ph.lo[c] = lo[c];
+        ph.hi[c] = hi[c];
+    }
+    return ph;
+}
+
 void op_reset(const at::Tensor& params, at::Tensor x, at::Tensor xa, at::Tensor noise_x, at::Tensor noise_a, at::Tensor elapsed,
               at::Tensor episode, c10::optional<at::Tensor> mask, at::TensorList draws) {
     const SwarmParams p = unpack(params);
@@ -224,6 +242,75 @@ void op_forces(const at::Tensor& params, const at::Tensor& x, const at::Tensor& 
           "swarm_forces");
 }
 
+void op_reset_physics(const at::Tensor& params, at::Tensor x, at::Tensor xa, at::Tensor noise_x, at::Tensor noise_a,
+                      at::Tensor elapsed, at::Tensor episode, c10::optional<at::Tensor> mask, at::TensorList draws,
+                      at::Tensor physics, int64_t physics_flags, at::ArrayRef<double> physics_lo,
+                      at::ArrayRef<double> physics_hi) {
+    const SwarmParams p = unpack(params);
+    c10::cuda::CUDAGuard guard(x.device());
+    const SwarmState st = make_state(p, x, xa, noise_x, noise_a, elapsed, episode);
+    if (mask.has_value()) need(*mask, at::kByte, {p.n_envs}, "mask");
+    SwarmInjectedDraws dr;
+    if (draws.size()) dr = make_draws(p, draws);
+    const SwarmPhysics ph = make_physics(p, physics, physics_flags, physics_lo, physics_hi, x);
+    check(swarm_reset_physics(&p, &st, &ph, ptr<uint8_t>(mask), draws.size() ? &dr : nullptr, stream_of(x)),
+          "swarm_reset_physics");
+}
+
+// op_step_final with per-env physics; without any of the final_* / terminated / truncated tensors it is op_step's call
+void op_step_physics(const at::Tensor& params, at::Tensor x, at::Tensor xa, at::Tensor noise_x, at::Tensor noise_a,
+                     at::Tensor elapsed, at::Tensor episode, c10::optional<at::Tensor> work, at::Tensor actions,
+                     c10::optional<at::Tensor> noise_a_step, c10::optional<at::Tensor> noise_x_step, at::Tensor reward,
+                     at::Tensor done, c10::optional<at::Tensor> grid, c10::optional<at::Tensor> positions,
+                     c10::optional<at::Tensor> v_out, int64_t flags, at::TensorList reset_draws, at::Tensor physics,
+                     int64_t physics_flags, at::ArrayRef<double> physics_lo, at::ArrayRef<double> physics_hi,
+                     c10::optional<at::Tensor> final_x, c10::optional<at::Tensor> final_xa,
+                     c10::optional<at::Tensor> terminated, c10::optional<at::Tensor> truncated,
+                     c10::optional<at::Tensor> final_grid, c10::optional<at::Tensor> final_positions) {
+    const SwarmParams p = unpack(params);
+    c10::cuda::CUDAGuard guard(x.device());
+    const SwarmState st = make_state(p, x, xa, noise_x, noise_a, elapsed, episode, work);
+    const SwarmStepIO io = make_io(p, actions, noise_a_step, noise_x_step, reward, done, grid, positions, v_out, flags);
+    const int64_t E = p.n_envs, N = p.n_locusts, A = p.n_agents, G = p.grid_size;
+    if (final_x.has_value()) need(*final_x, at::kDouble, {E, N, 2}, "final_x");
+    if (final_xa.has_value()) need(*final_xa, at::kDouble, {E, A, 2}, "final_xa");
+    if (terminated.has_value()) need(*terminated, at::kByte, {E}, "terminated");
+    if (truncated.has_value()) need(*truncated, at::kByte, {E}, "truncated");
+    if (final_grid.has_value()) need(*final_grid, at::kFloat, {E, G, G, 2}, "final_grid");
+    if (final_positions.has_value()) need(*final_positions, at::kByte, {E, A, 2}, "final_positions");
+    bool same = actions.get_device() == x.get_device() && reward.get_device() == x.get_device() &&
+                done.get_device() == x.get_device();
+    for (const c10::optional<at::Tensor>* t : {&grid, &positions, &final_x, &final_xa, &terminated, &truncated, &final_grid,
+                                               &final_positions})
+        same = same && (!t->has_value() || (*t)->get_device() == x.get_device());
+    TORCH_CHECK(same, "step_physics: all tensors must be on x's device");
+    const SwarmPhysics ph = make_physics(p, physics, physics_flags, physics_lo, physics_hi, x);
+    SwarmInjectedDraws dr;
+    if (reset_draws.size()) dr = make_draws(p, reset_draws);
+    const bool any_fin = final_x.has_value() || final_xa.has_value() || terminated.has_value() || truncated.has_value() ||
+                         final_grid.has_value() || final_positions.has_value();
+    const SwarmStepFinal fin{ptr<double>(final_x), ptr<double>(final_xa), ptr<uint8_t>(terminated), ptr<uint8_t>(truncated),
+                             ptr<float>(final_grid), ptr<uint8_t>(final_positions)};
+    check(swarm_step_physics(&p, &st, &io, any_fin ? &fin : nullptr, &ph, reset_draws.size() ? &dr : nullptr, stream_of(x)),
+          "swarm_step_physics");
+}
+
+void op_forces_physics(const at::Tensor& params, const at::Tensor& x, const at::Tensor& xa, c10::optional<at::Tensor> v,
+                       c10::optional<at::Tensor> reward, at::Tensor physics, int64_t physics_flags,
+                       at::ArrayRef<double> physics_lo, at::ArrayRef<double> physics_hi) {
+    const SwarmParams p = unpack(params);
+    c10::cuda::CUDAGuard guard(x.device());
+    const int64_t E = p.n_envs, N = p.n_locusts, A = p.n_agents;
+    need(x, at::kDouble, {E, N, 2}, "x");
+    need(xa, at::kDouble, {E, A, 2}, "xa");
+    if (v.has_value()) need(*v, at::kFloat, {E, N, 2}, "v");
+    if (reward.has_value()) need(*reward, at::kFloat, {E}, "reward");
+    const SwarmPhysics ph = make_physics(p, physics, physics_flags, physics_lo, physics_hi, x);
+    check(swarm_forces_physics(&p, &ph, x.data_ptr<double>(), xa.data_ptr<double>(), ptr<float>(v), ptr<float>(reward),
+                               stream_of(x)),
+          "swarm_forces_physics");
+}
+
 int64_t op_abi_version() { return swarm_abi_version(); }
 
 }  // namespace
@@ -246,5 +333,17 @@ TORCH_LIBRARY(swarm_b200, m) {
     m.def("expand_obs(Tensor params, Tensor grid, Tensor positions, Tensor(a!) expanded) -> ()", &op_expand_obs);
     m.def("clip_actions(Tensor(a!) actions, float max_norm) -> ()", &op_clip_actions);
     m.def("forces(Tensor params, Tensor x, Tensor xa, Tensor(a!)? v, Tensor(b!)? reward) -> ()", &op_forces);
+    m.def("reset_physics(Tensor params, Tensor(a!) x, Tensor(b!) xa, Tensor(c!) noise_x, Tensor(d!) noise_a, "
+          "Tensor(e!) elapsed, Tensor(f!) episode, Tensor? mask, Tensor[] draws, Tensor(g!) physics, int physics_flags, "
+          "float[] physics_lo, float[] physics_hi) -> ()", &op_reset_physics);
+    m.def("step_physics(Tensor params, Tensor(a!) x, Tensor(b!) xa, Tensor(c!) noise_x, Tensor(d!) noise_a, "
+          "Tensor(e!) elapsed, Tensor(f!) episode, Tensor(m!)? work, Tensor(g!) actions, Tensor? noise_a_step, "
+          "Tensor? noise_x_step, Tensor(h!) reward, Tensor(i!) done, Tensor(j!)? grid, Tensor(k!)? positions, "
+          "Tensor(l!)? v_out, int flags, Tensor[] reset_draws, Tensor(t!) physics, int physics_flags, float[] physics_lo, "
+          "float[] physics_hi, Tensor(n!)? final_x, Tensor(o!)? final_xa, Tensor(p!)? terminated, Tensor(q!)? truncated, "
+          "Tensor(r!)? final_grid, Tensor(s!)? final_positions) -> ()",
+          &op_step_physics);
+    m.def("forces_physics(Tensor params, Tensor x, Tensor xa, Tensor(a!)? v, Tensor(b!)? reward, Tensor physics, "
+          "int physics_flags, float[] physics_lo, float[] physics_hi) -> ()", &op_forces_physics);
     m.def("abi_version() -> int", &op_abi_version);
 }

@@ -81,6 +81,10 @@ class BatchedSwarmEnv(object):
     dict: ``terminated`` (reward >= 0) and ``truncated`` (TimeLimit) as (E,) bool, and for the envs that are done the
     terminal state ``final_x`` / ``final_xa`` and, when rasterising, its observation ``final_grid`` / ``final_positions``
     (the rows of the other envs keep their old bytes).  They alias buffers of the env, like reward and done.
+    With ``physics`` every env has its own noise, gravity, wind, F, L and dt: row e of ``self.physics`` (E,6) f64, columns
+    ``_native.PHYSICS_COLUMNS`` (SwarmPhysics).  ``"table"`` fills it from the class constants and leaves it to the
+    caller, who may write rows between calls; a dict of per-column ranges such as ``{"F": (0.3, 0.7), "L": (5, 15)}``
+    draws each env's row anew, uniformly, at every reset of that env (explicit or auto-reset), inside the kernels.
     """
 
     # fed_gym/envs/multiagent.py:8-21
@@ -96,14 +100,16 @@ class BatchedSwarmEnv(object):
 
     def __init__(self, num_envs, n_locusts=None, n_agents=None, grid_size=84, max_episode_steps=128,
                  seed=0, env_id_offset=0, device=None, math_mode="fast", auto_reset=True, rasterize=True,
-                 binding="torch", tuning=0, noise="frozen", cluster=None, final_obs=False):
+                 binding="torch", tuning=0, noise="frozen", cluster=None, final_obs=False, physics=None):
         """binding: "torch" = the hot calls go through torch.ops.swarm_b200.* (the C ABI as a PyTorch
         extension, csrc/torch_binding.cpp), "ctypes" = straight into the C ABI.  Same kernels either way.
         tuning: SwarmParams.tuning (0 = automatic launch shape; anything else only changes speed, never bits).
         noise: "frozen" (the reference: every step after a reset re-uses noise row N_BURN_IN) or "fresh" (step k of
         an episode uses row N_BURN_IN + k, drawn by Philox inside the step kernel; SWARM_STEP_FRESH_NOISE).
         cluster: None = one CTA per env up to 2048 locusts and a thread-block cluster of the library's size above; an
-        integer K = a cluster of K CTAs per env (1..16, for 512 < n_locusts <= 8192; bitwise the same results)."""
+        integer K = a cluster of K CTAs per env (1..16, for 512 < n_locusts <= 8192; bitwise the same results).
+        physics: None (every env uses the class constants), "table" (per-env rows in self.physics, written by the caller)
+        or a dict {column: (lo, hi)} (per-env rows redrawn at every reset; unnamed columns stay at the class constant)."""
         self.lib = nat.load()
         if binding not in ("torch", "ctypes"):
             raise ValueError("binding must be 'torch' or 'ctypes'")
@@ -172,7 +178,32 @@ class BatchedSwarmEnv(object):
             self._fin = nat.SwarmStepFinal(_ptr(self.final_x), _ptr(self.final_xa), _ptr(self.terminated),
                                            _ptr(self.truncated), None, None)
             self._fin_ref = ctypes.byref(self._fin)
+        self._init_physics(physics)
         self.refresh_params()
+
+    def _init_physics(self, physics):
+        self.physics = None
+        if physics is None:
+            return
+        fixed = [float(getattr(self.params, c)) for c in nat.PHYSICS_COLUMNS]
+        lo, hi, flags = list(fixed), list(fixed), 0
+        if isinstance(physics, dict):
+            for name, rng in physics.items():
+                if name not in nat.PHYSICS_COLUMNS:
+                    raise ValueError("unknown physics column %r (columns: %s)" % (name, ", ".join(nat.PHYSICS_COLUMNS)))
+                c = nat.PHYSICS_COLUMNS.index(name)
+                lo[c], hi[c] = float(rng[0]), float(rng[1])
+            flags = nat.SWARM_PHYSICS_RESAMPLE
+        elif physics != "table":
+            raise ValueError("physics must be None, 'table' or a dict {column: (lo, hi)}")
+        self.physics = torch.tensor([fixed] * self.E, dtype=torch.float64, device=self.device)
+        self._phys_flags, self._phys_lo, self._phys_hi = flags, lo, hi
+        self._phys_c = nat.SwarmPhysics(self.physics.data_ptr(), flags, 0, (ctypes.c_double * 6)(*lo),
+                                        (ctypes.c_double * 6)(*hi))
+        self._phys_ref = ctypes.byref(self._phys_c)
+
+    def _phys_args(self):
+        return self.physics, self._phys_flags, self._phys_lo, self._phys_hi
 
     def refresh_params(self):
         self._state_t = (self.x, self.xa, self.noise_x, self.noise_a, self.elapsed, self.episode, self.work)
@@ -196,14 +227,23 @@ class BatchedSwarmEnv(object):
         if draws is not None:
             draws.check(self.E, self.N, self.A, self.N_BURN_IN)
         if self.ops is not None:
+            dts = draws.tensors() if draws is not None else []
             with torch.cuda.device(self.device):
-                self.ops.reset(self._blob, *self._state_t[:6], m, draws.tensors() if draws is not None else [])
+                if self.physics is not None:
+                    self.ops.reset_physics(self._blob, *self._state_t[:6], m, dts, *self._phys_args())
+                else:
+                    self.ops.reset(self._blob, *self._state_t[:6], m, dts)
             self._was_reset = True
             return self.x, self.xa
         with self._ctx:
-            nat.check(self.lib.swarm_reset(ctypes.byref(self.params), ctypes.byref(self.state_c), _ptr(m),
-                                           ctypes.byref(draws.c) if draws is not None else None,
-                                           _stream(self.device)), "swarm_reset")
+            dr = ctypes.byref(draws.c) if draws is not None else None
+            if self.physics is not None:
+                nat.check(self.lib.swarm_reset_physics(ctypes.byref(self.params), ctypes.byref(self.state_c),
+                                                       self._phys_ref, _ptr(m), dr, _stream(self.device)),
+                          "swarm_reset_physics")
+            else:
+                nat.check(self.lib.swarm_reset(ctypes.byref(self.params), ctypes.byref(self.state_c), _ptr(m), dr,
+                                               _stream(self.device)), "swarm_reset")
         self._was_reset = True
         return self.x, self.xa
 
@@ -233,6 +273,16 @@ class BatchedSwarmEnv(object):
                 raise ValueError("actions must be float32 or float64")
             g_t = (grid_out if grid_out is not None else self.grid) if rasterize else None
             p_t = (positions_out if positions_out is not None else self.positions) if rasterize else None
+            if self.physics is not None:
+                dts = reset_draws.tensors() if reset_draws is not None else []
+                fin = [None] * 6
+                if self.final_obs:
+                    fg, fp = self._final_obs_bufs(rasterize, final_grid_out, final_positions_out)
+                    fin = [self.final_x, self.final_xa, self.terminated, self.truncated, fg, fp]
+                self.ops.step_physics(self._blob, *self._state_t, actions, noise_a, noise_x, self.reward, self.done_u8,
+                                      g_t, p_t, v_out, flags, dts, *self._phys_args(), *fin)
+                info = self._info(fin[4], fin[5]) if self.final_obs else {}
+                return (self.x, self.xa), self.reward, self._done_view, info
             if self.final_obs:
                 fg, fp = self._final_obs_bufs(rasterize, final_grid_out, final_positions_out)
                 self.ops.step_final(self._blob, *self._state_t, actions, noise_a, noise_x, self.reward, self.done_u8,
@@ -261,6 +311,19 @@ class BatchedSwarmEnv(object):
             io.grid, io.positions = None, None
         io.v_out = v_out.data_ptr() if v_out is not None else None
         io.flags = flags
+        if self.physics is not None:
+            fin_ref, info = None, {}
+            if self.final_obs:
+                fg, fp = self._final_obs_bufs(rasterize, final_grid_out, final_positions_out)
+                self._fin.grid, self._fin.positions = _ptr(fg), _ptr(fp)
+                fin_ref, info = self._fin_ref, self._info(fg, fp)
+            with self._ctx:
+                rc = self.lib.swarm_step_physics(self._params_ref, self._state_ref, self._io_ref, fin_ref, self._phys_ref,
+                                                 ctypes.byref(reset_draws.c) if reset_draws is not None else None,
+                                                 torch.cuda.current_stream(self.device).cuda_stream)
+            if rc:
+                nat.check(rc, "swarm_step_physics")
+            return (self.x, self.xa), self.reward, self._done_view, info
         if self.final_obs:
             fg, fp = self._final_obs_bufs(rasterize, final_grid_out, final_positions_out)
             self._fin.grid, self._fin.positions = _ptr(fg), _ptr(fp)
@@ -324,7 +387,12 @@ class BatchedSwarmEnv(object):
         io.flags = nat.SWARM_STEP_AUTO_RESET if self.auto_reset else 0
         out = (ctypes.c_int32 * 8)()
         with self._ctx:
-            nat.check(self.lib.swarm_step_plan(self._params_ref, self._state_ref, ctypes.byref(io), out), "swarm_step_plan")
+            if self.physics is not None:
+                nat.check(self.lib.swarm_step_plan_physics(self._params_ref, self._state_ref, ctypes.byref(io),
+                                                           self._phys_ref, out), "swarm_step_plan_physics")
+            else:
+                nat.check(self.lib.swarm_step_plan(self._params_ref, self._state_ref, ctypes.byref(io), out),
+                          "swarm_step_plan")
         keys = ("force_mode", "filler_warp", "raster_place", "threads", "ctas", "smem_bytes", "follower_ctas", "launches")
         d = dict(zip(keys, list(out)))
         cluster = d["raster_place"] == 4
@@ -341,7 +409,10 @@ class BatchedSwarmEnv(object):
         """swarm_step_host: actions come from / reward+done go to HOST tensors; the observation stays in HBM
         for the device-resident policy unless host_grid / host_positions are given (then it is also copied back:
         the numpy-out case of the reference's process_state).  Synchronises the stream.  Pinned tensors are read /
-        written by the kernel itself over PCIe (zero-copy); self.reward / self.done_u8 are then NOT updated."""
+        written by the kernel itself over PCIe (zero-copy); self.reward / self.done_u8 are then NOT updated.
+        Not available with per-env physics (swarm_step_host takes no SwarmPhysics)."""
+        if self.physics is not None:
+            raise ValueError("step_host has no per-env physics (swarm_step_host takes no SwarmPhysics); use step()")
         io = self._io_host
         if io is None:
             io = self._io_host = nat.SwarmStepIO()
@@ -392,7 +463,16 @@ class BatchedSwarmEnv(object):
         if reward is None:
             reward = torch.empty(self.E, dtype=torch.float32, device=self.device)
         if self.ops is not None:
-            self.ops.forces(self._blob, x, xa, v, reward)
+            if self.physics is not None:
+                self.ops.forces_physics(self._blob, x, xa, v, reward, *self._phys_args())
+            else:
+                self.ops.forces(self._blob, x, xa, v, reward)
+            return v, reward
+        if self.physics is not None:
+            with self._ctx:
+                nat.check(self.lib.swarm_forces_physics(ctypes.byref(self.params), self._phys_ref, _ptr(x), _ptr(xa),
+                                                        _ptr(v), _ptr(reward), _stream(self.device)),
+                          "swarm_forces_physics")
             return v, reward
         with self._ctx:
             nat.check(self.lib.swarm_forces(ctypes.byref(self.params), _ptr(x), _ptr(xa), _ptr(v), _ptr(reward),
@@ -426,7 +506,7 @@ class BatchedSwarmEnv(object):
 
     # ------------------------------------------------------------------ checkpointing
     def state_dict(self):
-        keys = ("x", "xa", "noise_x", "noise_a", "elapsed", "episode")
+        keys = ("x", "xa", "noise_x", "noise_a", "elapsed", "episode") + (("physics",) if self.physics is not None else ())
         return {k: getattr(self, k).clone() for k in keys}
 
     def load_state_dict(self, sd):

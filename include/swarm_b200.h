@@ -145,6 +145,26 @@ typedef struct SwarmStepFinal {
     uint8_t* positions;         /* (E,A,2) required iff grid                                                       */
 } SwarmStepFinal;
 
+/* Per-env physics (swarm_reset_physics / swarm_step_physics / swarm_forces_physics): env e takes noise, gravity, wind, F,
+ * L and dt from row e of a device table instead of SwarmParams, with the same roundings (F, 1/L, wind and gravity to
+ * FP32 for the pair forces; noise, wind and dt FP64), so a row equal to SwarmParams gives their bits exactly.
+ * With SWARM_PHYSICS_RESAMPLE every reset of env e (explicit or auto-reset) first draws a new row:
+ *   column c = lo[c] + (hi[c] - lo[c]) u   (each operation rounded once; lo == hi gives lo exactly)
+ * u = the .x (even c) or .y (odd c) of the uniform pair c / 2 of Philox stream 5 of the reset (seed, global env id,
+ * episode counter before the reset's increment) -- always Philox, also with injected draws.  The row is written to
+ * table[e] and governs the reset's burn-in and every step of the new episode.  Without the flag the table is only read
+ * (once per step / reset / forces call), so the caller may edit rows between calls.
+ * Before any CUDA call: phys or table NULL -> SWARM_ERR_NULL; table not 16-byte aligned, unknown flag bits or
+ * reserved != 0 -> SWARM_ERR_FLAGS; with RESAMPLE a non-finite bound, lo > hi, a non-finite hi - lo or lo[4] (L) <= 0
+ * -> SWARM_ERR_SIZE.  The table's values are device data and are not checked. */
+#define SWARM_PHYSICS_RESAMPLE 1u
+typedef struct SwarmPhysics {
+    double* table;              /* (E,6) f64 device, 16-byte aligned: env e's {noise, gravity, wind, F, L, dt}         */
+    uint32_t flags;             /* SWARM_PHYSICS_RESAMPLE                                                               */
+    uint32_t reserved;          /* must be 0                                                                            */
+    double lo[6], hi[6];        /* per-column uniform range of SWARM_PHYSICS_RESAMPLE                                   */
+} SwarmPhysics;
+
 int swarm_abi_version(void);
 const char* swarm_strerror(int status);
 const char* swarm_last_cuda_error(void);
@@ -187,6 +207,19 @@ int swarm_step(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io
  * fin->grid; fin->grid not 8-byte aligned. */
 int swarm_step_final(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io, const SwarmStepFinal* fin,
                      const SwarmInjectedDraws* reset_draws, swarm_stream_t stream);
+
+/* swarm_reset / swarm_step_final / swarm_forces with per-env physics (SwarmPhysics above).  fin is nullable like
+ * swarm_step_final's.  Separate kernel instantiations: the kernels of swarm_reset / swarm_step / swarm_step_final /
+ * swarm_forces are unchanged. */
+int swarm_reset_physics(const SwarmParams* p, const SwarmState* st, const SwarmPhysics* phys, const uint8_t* mask,
+                        const SwarmInjectedDraws* draws, swarm_stream_t stream);
+int swarm_step_physics(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io, const SwarmStepFinal* fin,
+                       const SwarmPhysics* phys, const SwarmInjectedDraws* reset_draws, swarm_stream_t stream);
+int swarm_forces_physics(const SwarmParams* p, const SwarmPhysics* phys, const double* x, const double* xa, float* v,
+                         float* reward, swarm_stream_t stream);
+/* swarm_step_plan for swarm_step_physics (its kernels hold the physics rows in shared memory). */
+int swarm_step_plan_physics(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io, const SwarmPhysics* phys,
+                            int32_t out[8]);
 
 /* The launch shape swarm_step would use for these arguments (no launch; needs the device for occupancy queries):
  * out = { force mode, filler warp (0/1), rasteriser placement (0 none, 1 follower kernel, 2 raster warps, 3 the step's

@@ -5,7 +5,7 @@
     torchrun --nproc-per-node 8 scripts/train_paac_conv.py -ec 8192 --clip_norm=1    # config 5: env batch sharded
 
 Flag names and defaults are the reference's; additions: --n_locusts, --max_updates, --no_cuda_graph,
---reward_indexing, --mask_terminals, --bootstrap_truncated, --fresh_noise.
+--reward_indexing, --mask_terminals, --bootstrap_truncated, --fresh_noise, --physics.
 '-d/--device' accepts the reference's '/gpu:0' spelling.
 """
 import argparse
@@ -31,12 +31,28 @@ def bool_arg(string):
     raise argparse.ArgumentTypeError("Expected True or False, but got {}".format(string))
 
 
+def physics_ranges(spec):
+    """'F=0.3:0.7,L=5:15' -> {'F': (0.3, 0.7), 'L': (5.0, 15.0)} (BatchedSwarmEnv's physics ranges); '' -> None."""
+    if not spec:
+        return None
+    out = {}
+    for item in spec.split(","):
+        try:
+            name, rng = item.split("=")
+            lo, hi = rng.split(":")
+            out[name.strip()] = (float(lo), float(hi))
+        except ValueError:
+            raise argparse.ArgumentTypeError("expected NAME=LO:HI[,NAME=LO:HI...], got %r" % spec)
+    return out
+
+
 def get_network_and_environment_creator(args, random_seed=3):
     import golds_rl_gym_b200 as pkg
     ec = pkg.submodule("agents.paac.environment_creator")
     pv = pkg.submodule("agents.paac.policy_v_network")
     env_creator = ec.SwarmEnvironmentCreator(n_locusts=args.n_locusts, grid_size=args.height,
-                                             noise="fresh" if getattr(args, "fresh_noise", False) else "frozen")
+                                             noise="fresh" if getattr(args, "fresh_noise", False) else "frozen",
+                                             physics=getattr(args, "physics", None))
     args.num_actions = env_creator.num_actions
     args.random_seed = random_seed
     network_conf = {
@@ -100,6 +116,9 @@ def get_arg_parser():
                         help="with --mask_terminals: bootstrap a TimeLimit truncation from V of the terminal observation")
     parser.add_argument('--fresh_noise', action='store_true',
                         help="advance the env noise row every step (SURVEY Q1 fixed); default: the reference's frozen row")
+    parser.add_argument('--physics', default=None, type=physics_ranges,
+                        help="per-env physics redrawn at every reset of each training env, e.g. 'F=0.3:0.7,L=5:15' "
+                             "(columns noise, gravity, wind, F, L, dt; unnamed ones keep the reference's constant)")
     parser.add_argument('--eval_every', default=30.0, type=float,
                         help="seconds between evaluation episodes on Swarm-eval-v0 (policy_monitor.py); 0 = off")
     parser.add_argument('--net_precision', default='fp32', choices=['fp32', 'tf32', 'bf16'],
