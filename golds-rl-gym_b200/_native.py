@@ -106,6 +106,10 @@ SYMBOLS = {
     "swarm_forces_physics": (c_int, [_P(SwarmParams), _P(SwarmPhysics), c_void_p, c_void_p, c_void_p, c_void_p,
                                      c_void_p]),
     "swarm_step_plan_physics": (c_int, [_P(SwarmParams), _P(SwarmState), _P(SwarmStepIO), _P(SwarmPhysics), c_void_p]),
+    "swarm_step_repeat": (c_int, [_P(SwarmParams), _P(SwarmState), _P(SwarmStepIO), _P(SwarmStepFinal), _P(SwarmPhysics),
+                                  c_int32, _P(SwarmInjectedDraws), c_void_p]),
+    "swarm_step_plan_repeat": (c_int, [_P(SwarmParams), _P(SwarmState), _P(SwarmStepIO), _P(SwarmPhysics), c_int32,
+                                       c_void_p]),
     "swarm_step_host": (c_int, [_P(SwarmParams), _P(SwarmState), _P(SwarmStepIO), c_void_p, c_void_p, c_void_p,
                                 c_void_p, c_void_p, c_void_p]),
     "swarm_step_host_clear": (None, []),

@@ -7,7 +7,9 @@ process_state -> get_local_states until done; track the best score and dump its 
 reference replays (make_swarm_gif.py:62-67).  Summaries keep the reference tags eval/total_reward and
 eval/episode_length (returned as a dict; a tensorboard SummaryWriter is used when one is passed in).
 
-The eval env is the E=1 view of the batched CUDA env, the observation the rasteriser kernel's.
+The eval env is the E=1 view of the batched CUDA env, the observation the rasteriser kernel's.  With ``action_repeat``
+K > 1 (the training envs' action repeat) each chosen action is stepped K times, stopping at done, and the rewards are
+summed, so that eval scores are on the scale of the training rewards; the episode length counts decisions.
 """
 import copy
 import json
@@ -24,7 +26,7 @@ from .emulator_runner import SwarmRunner
 
 class SwarmPolicyMonitor(object):
     def __init__(self, env=None, global_policy_net=None, state_processor=None, summary_writer=None, saver=None,
-                 network_conf=None, out_dir=".", fresh_noise=False):
+                 network_conf=None, out_dir=".", fresh_noise=False, action_repeat=1):
         # fresh_noise: the default eval env follows the training envs' noise mode (SURVEY Q1 fixed or not)
         self.env = env if env is not None else ma.make("Swarm-eval-v0", fresh_noise=fresh_noise)
         self.global_policy_net = global_policy_net
@@ -32,6 +34,9 @@ class SwarmPolicyMonitor(object):
         self.summary_writer = summary_writer
         self.best_score = -np.inf
         self.out_dir = out_dir
+        self.action_repeat = int(action_repeat)
+        if self.action_repeat < 1:
+            raise ValueError("action_repeat must be >= 1")
         self.policy_net = self._create_policy_estimator(global_policy_net)
 
     @staticmethod
@@ -73,7 +78,12 @@ class SwarmPolicyMonitor(object):
         while not done:
             action = self.get_action_from_policy(obs) if actions is None else np.asarray(actions.get(), dtype=np.float32)
             taken.append(np.asarray(action).tolist())
-            state, reward, done, _ = self.env.step(action)
+            reward = 0.0
+            for _ in range(self.action_repeat):
+                state, r, done, _ = self.env.step(action)
+                reward += float(r)
+                if done:
+                    break
             obs = self._observe(state)
             total_reward += float(reward)
             episode_length += 1

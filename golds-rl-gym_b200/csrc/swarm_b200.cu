@@ -75,10 +75,14 @@ __device__ __forceinline__ double* phys_rows(unsigned char* smem_raw, size_t sme
 // PHYS (swarm_step_physics): per-env physics.  Env e's row is prefetched with the env into its stage buffer's row, and
 // an auto-reset with SWARM_PHYSICS_RESAMPLE draws the new episode's row into it (and the table) before the burn-in.
 // Compile time for the same reason as FIN.
-template <int MODE, bool PRECISE, int PLACE, bool FIN, bool PHYS>
+// REP (swarm_step_repeat, with either FIN): action repeat.  The step proper runs up to `repeat` substeps with
+// the same actions through the one env_step call site, summing the FP32 rewards in order and stopping at the first done
+// substep; the done / auto-reset / write-back / rasterise tail then runs once.  `repeat` is a kernel parameter rather
+// than a KP field: a longer KP would move every later parameter of every kernel and change the default kernels' code.
+template <int MODE, bool PRECISE, int PLACE, bool FIN, bool PHYS, bool REP>
 __global__ void __maxnreg__(64) k_step(const KP kp, const SwarmState st, const SwarmStepIO io,
                                        const SwarmInjectedDraws dr, const int has_draws, const int n_force,
-                                       const SwarmStepFinal fin, const SwarmPhysics phys) {
+                                       const SwarmStepFinal fin, const SwarmPhysics phys, const int repeat) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int N = kp.N, A = kp.A;
     const int n_all = blockDim.x, n_raster = n_all - n_force;
@@ -201,6 +205,8 @@ __global__ void __maxnreg__(64) k_step(const KP kp, const SwarmState st, const S
             uint32_t ep = 0;
             int r = -1;                              // -1: the step proper; >= 0: burn-in row being stepped
             float* v_out = io.v_out ? io.v_out + (size_t)e * N * 2 : nullptr;
+            int sub = 0;                             // REP: substep of the step proper
+            float rsum = 0.0f;                       // REP: FP32 sum of the substeps' rewards
             for (;;) {
                 // multiagent.py:30,35-36: _step(add_wind=False) leaves the action alone; the burn-in steps of a reset
                 // always go through step() with the default add_wind=True (multiagent.py:59-61)
@@ -210,9 +216,33 @@ __global__ void __maxnreg__(64) k_step(const KP kp, const SwarmState st, const S
                 if (r < 0) {
                     // multiagent.py:44 done = reward >= 0; gym TimeLimit: done |= ++elapsed >= max_episode_steps
                     elapsed = sm.st.misc[0] + 1;
+                    if constexpr (REP) elapsed += sub;
                     const bool done = (reward >= 0.0) || (kp.max_steps > 0 && elapsed >= kp.max_steps);
+                    if constexpr (REP) {
+                        // in substep order from the first substep's reward (not 0.0f): repeat 1 and -0.0 keep their bits
+                        rsum = sub == 0 ? (float)reward : __fadd_rn(rsum, (float)reward);
+                        if (!done && ++sub < repeat) {
+                            // Fresh noise: substep sub uses row nrow + sub, drawn with the prologue's owner mappings (targets
+                            // of this thread into sm.nx, agents k = tid mod n into sm.st.an).  env_step reads each of these
+                            // elements only with the thread that writes it here, and the previous substep's reads of them
+                            // were by this same thread: no barrier.  Frozen rows and overrides stay where they are.
+                            if (kp.fresh) {
+                                const uint32_t row = nrow + (uint32_t)sub;
+                                if (!io.noise_x) {
+#pragma unroll
+                                    for (int t = 0; t < T; ++t) {
+                                        const int j = target_index<MODE>(g, t, kp);
+                                        if (j < N) sm.nx[j] = draw_normal2(nd, STREAM_NOISE_X, row, (uint32_t)j);
+                                    }
+                                }
+                                if (!io.noise_a)
+                                    for (int k = g.tid; k < A; k += g.n) sm.st.an[k] = draw_normal2(nd, STREAM_NOISE_A, row, (uint32_t)k);
+                            }
+                            continue;
+                        }
+                    }
                     if (g.tid == 0) {
-                        io.reward[e] = (float)reward;
+                        io.reward[e] = REP ? rsum : (float)reward;
                         io.done[e] = done ? 1 : 0;
                         if constexpr (FIN) {
                             if (fin.terminated) fin.terminated[e] = reward >= 0.0 ? 1 : 0;
@@ -705,10 +735,11 @@ __device__ __forceinline__ void cl_store(const KP& kp, const CMap& m, double2* x
 // SwarmEnv._step + TimeLimit + auto-reset + process_state (k_step's contract) for the cluster layout.
 // FIN: k_step's; each CTA copies its own targets' terminal positions from pn[], rank 0 the agents' from sm.as.
 // PHYS: k_step's; every CTA reads (or draws) the env's row into its own shared memory, rank 0 writes a drawn row back.
-template <int MODE, bool PRECISE, bool FIN, bool PHYS>
+// REP: k_step's; the reward is cluster-uniform, and so is the early stop.
+template <int MODE, bool PRECISE, bool FIN, bool PHYS, bool REP>
 __global__ void __maxnreg__(64) k_step_cluster(const KP kp, const SwarmState st, const SwarmStepIO io,
                                                const SwarmInjectedDraws dr, const int has_draws, const int nf,
-                                               const SwarmStepFinal fin, const SwarmPhysics phys) {
+                                               const SwarmStepFinal fin, const SwarmPhysics phys, const int repeat) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     constexpr int T = ModeT<MODE>::T;
     const int N = kp.N, A = kp.A, tid = (int)threadIdx.x;
@@ -770,6 +801,8 @@ __global__ void __maxnreg__(64) k_step_cluster(const KP kp, const SwarmState st,
     if constexpr (PHYS) __syncthreads();
     float* v_out = io.v_out ? io.v_out + (size_t)e * N * 2 : nullptr;
     int elapsed = 0;
+    int sub = 0;                // REP: substep of the step proper
+    float rsum = 0.0f;          // REP: FP32 sum of the substeps' rewards
     for (int r = -1;;) {
         double2 pn[T];
         if constexpr (PHYS)
@@ -781,9 +814,22 @@ __global__ void __maxnreg__(64) k_step_cluster(const KP kp, const SwarmState st,
         const double reward = cl_reward(sm, kp, m);
         if (r < 0) {
             elapsed = elapsed0 + 1;
+            if constexpr (REP) elapsed += sub;
             const bool done = (reward >= 0.0) || (kp.max_steps > 0 && elapsed >= kp.max_steps);
+            if constexpr (REP) {
+                rsum = sub == 0 ? (float)reward : __fadd_rn(rsum, (float)reward);
+                if (!done && ++sub < repeat) {
+                    // the next substep's fresh rows: the locusts' are drawn inside cl_step_forces from nz.fresh_row, the
+                    // agents' here, where cl_reset_row writes a burn-in row (read after the barrier below)
+                    ++nz.fresh_row;
+                    if (kp.fresh && !io.noise_a && tid < A)
+                        sm.an[tid] = draw_normal2(nz.fresh_d, STREAM_NOISE_A, nz.fresh_row, (uint32_t)tid);
+                    cluster_sync();     // the new state is in memory before any CTA reads it again
+                    continue;
+                }
+            }
             if (lead && tid == 0) {
-                io.reward[e] = (float)reward;
+                io.reward[e] = REP ? rsum : (float)reward;
                 io.done[e] = done ? 1 : 0;
                 if constexpr (FIN) {
                     if (fin.terminated) fin.terminated[e] = reward >= 0.0 ? 1 : 0;
@@ -1308,35 +1354,41 @@ T* mapped_host(T* host) {
 }
 
 typedef void (*StepKernel)(const KP, const SwarmState, const SwarmStepIO, const SwarmInjectedDraws, const int, const int,
-                           const SwarmStepFinal, const SwarmPhysics);
+                           const SwarmStepFinal, const SwarmPhysics, const int);
 
-template <int PLACE, bool FIN, bool PHYS>
+template <int PLACE, bool FIN, bool PHYS, bool REP>
 StepKernel step_kernel_p(int mode, bool precise) {
     switch (mode) {
-        case 1: return precise ? k_step<1, true, PLACE, FIN, PHYS> : k_step<1, false, PLACE, FIN, PHYS>;
-        case 2: return precise ? k_step<2, true, PLACE, FIN, PHYS> : k_step<2, false, PLACE, FIN, PHYS>;
-        case 3: return precise ? k_step<3, true, PLACE, FIN, PHYS> : k_step<3, false, PLACE, FIN, PHYS>;
-        default: return precise ? k_step<4, true, PLACE, FIN, PHYS> : k_step<4, false, PLACE, FIN, PHYS>;
+        case 1: return precise ? k_step<1, true, PLACE, FIN, PHYS, REP> : k_step<1, false, PLACE, FIN, PHYS, REP>;
+        case 2: return precise ? k_step<2, true, PLACE, FIN, PHYS, REP> : k_step<2, false, PLACE, FIN, PHYS, REP>;
+        case 3: return precise ? k_step<3, true, PLACE, FIN, PHYS, REP> : k_step<3, false, PLACE, FIN, PHYS, REP>;
+        default: return precise ? k_step<4, true, PLACE, FIN, PHYS, REP> : k_step<4, false, PLACE, FIN, PHYS, REP>;
     }
 }
-template <bool FIN, bool PHYS>
+template <bool FIN, bool PHYS, bool REP = false>
 StepKernel step_kernel_f(int mode, bool precise, int place) {
-    return place == 2 ? step_kernel_p<2, FIN, PHYS>(mode, precise)
-                      : (place == 3 ? step_kernel_p<3, FIN, PHYS>(mode, precise) : step_kernel_p<0, FIN, PHYS>(mode, precise));
+    return place == 2 ? step_kernel_p<2, FIN, PHYS, REP>(mode, precise)
+                      : (place == 3 ? step_kernel_p<3, FIN, PHYS, REP>(mode, precise)
+                                    : step_kernel_p<0, FIN, PHYS, REP>(mode, precise));
 }
 // place: RasterPlace (NONE / FOLLOW share the rasteriser-less kernel); fin: the swarm_step_final variant; phys: the
-// swarm_step_physics one
-StepKernel step_kernel(int mode, bool precise, int place, bool fin, bool phys) {
+// swarm_step_physics one; rep: the swarm_step_repeat one (with and without FIN: a FIN kernel whose fin pointers are all
+// null was measured 2.8 % slower than the FIN = false one on the C4 step, profiles/r07_action_repeat.md)
+StepKernel step_kernel(int mode, bool precise, int place, bool fin, bool phys, bool rep) {
+    if (rep && phys) return fin ? step_kernel_f<true, true, true>(mode, precise, place) : step_kernel_f<false, true, true>(mode, precise, place);
+    if (rep) return fin ? step_kernel_f<true, false, true>(mode, precise, place) : step_kernel_f<false, false, true>(mode, precise, place);
     if (phys) return fin ? step_kernel_f<true, true>(mode, precise, place) : step_kernel_f<false, true>(mode, precise, place);
     return fin ? step_kernel_f<true, false>(mode, precise, place) : step_kernel_f<false, false>(mode, precise, place);
 }
 
-template <bool FIN, bool PHYS>
+template <bool FIN, bool PHYS, bool REP = false>
 StepKernel step_kernel_cluster_f(int mode, bool precise) {
-    return mode == 2 ? (precise ? k_step_cluster<2, true, FIN, PHYS> : k_step_cluster<2, false, FIN, PHYS>)
-                     : (precise ? k_step_cluster<4, true, FIN, PHYS> : k_step_cluster<4, false, FIN, PHYS>);
+    return mode == 2 ? (precise ? k_step_cluster<2, true, FIN, PHYS, REP> : k_step_cluster<2, false, FIN, PHYS, REP>)
+                     : (precise ? k_step_cluster<4, true, FIN, PHYS, REP> : k_step_cluster<4, false, FIN, PHYS, REP>);
 }
-StepKernel step_kernel_cluster(int mode, bool precise, bool fin, bool phys) {
+StepKernel step_kernel_cluster(int mode, bool precise, bool fin, bool phys, bool rep) {
+    if (rep && phys) return fin ? step_kernel_cluster_f<true, true, true>(mode, precise) : step_kernel_cluster_f<false, true, true>(mode, precise);
+    if (rep) return fin ? step_kernel_cluster_f<true, false, true>(mode, precise) : step_kernel_cluster_f<false, false, true>(mode, precise);
     if (phys) return fin ? step_kernel_cluster_f<true, true>(mode, precise) : step_kernel_cluster_f<false, true>(mode, precise);
     return fin ? step_kernel_cluster_f<true, false>(mode, precise) : step_kernel_cluster_f<false, false>(mode, precise);
 }
@@ -1485,9 +1537,10 @@ struct StepPlan {
 
 // Validates the arguments of swarm_step and decides its launch shape (automatic, or forced through
 // SwarmParams::tuning).  Touches the GPU only for attribute / occupancy queries (cached per device).
-// phys: the PHYS kernels, with the physics rows of their stage buffers behind their shared memory.
+// phys: the PHYS kernels, with the physics rows of their stage buffers behind their shared memory.  repeat > 1: the REP
+// kernels.
 int plan_step(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io, const SwarmInjectedDraws* reset_draws,
-              StepPlan* out, const bool fin = false, const bool phys = false) {
+              StepPlan* out, const bool fin = false, const bool phys = false, const int repeat = 1) {
     int rc = validate(p);
     if (rc) return rc;
     if (!st || !io) return SWARM_ERR_NULL;
@@ -1523,11 +1576,12 @@ int plan_step(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io,
     const int filler_threads = 32;                           // the SELF shape's TMA zero-fill warp
     const int mode = force_mode(N);
     const int nf = block_threads(N, mode);
+    const bool rep = repeat > 1;
     out->cluster = 0;
     if (tuning_cluster(p)) {
         // one env per thread-block cluster; the observation (if any) comes from the cluster itself, st->work is not used
         ClusterShape sh;
-        out->kernel = step_kernel_cluster(mode, p->math_mode != 0, fin, phys);
+        out->kernel = step_kernel_cluster(mode, p->math_mode != 0, fin, phys, rep);
         if ((rc = cluster_shape(p, out->kernel, true, &sh, phys ? kPhysRowBytes : 0))) return rc;
         out->mode = mode; out->place = RASTER_CLUSTER;
         out->raster = 0; out->n_stage = 0; out->filler = 0; out->dynamic = 0;
@@ -1548,7 +1602,7 @@ int plan_step(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io,
            follow_per_sm * (follow_smem + 1024) + step_smem(p, 0, 1, mode) + (phys ? kPhysRowBytes : 0) + 1024 > kMaxSmem)
         --follow_per_sm;
     const bool no_follower = (io->flags & SWARM_STEP_INKERNEL_RASTER) || env_flag("SWARM_B200_NO_FOLLOWER");
-    const StepKernel kernel = step_kernel(mode, p->math_mode != 0, RASTER_FOLLOW, fin, phys);     // the rasteriser-less kernel
+    const StepKernel kernel = step_kernel(mode, p->math_mode != 0, RASTER_FOLLOW, fin, phys, rep);     // the rasteriser-less kernel
     bool follow_fits = have_flags && !no_follower && follow_per_sm > 0 && follow_per_sm * follow_threads + nf <= 2048;
     int rgrid = 0;
     if (want_grid && follow_fits) {
@@ -1581,6 +1635,11 @@ int plan_step(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io,
         // batch is XU-bound like a multi-wave one and the follower overlaps better (1024 x 192: 43.5 vs 46.0 us).
         else if (E > sms && nf >= 96 && E <= (long long)sms * (N >= 160 && per_sm > 4 ? 4 : per_sm)) place = RASTER_SELF;
         else if (N >= 160) place = RASTER_FOLLOW;
+        // Action repeat keeps each env K times longer in its step CTA.  Measured (profiles/r07_action_repeat.md): in
+        // multi-wave batches with three or more force warps the follower then overtakes the raster warps (4096 x 80:
+        // K = 2 85.3 vs 89.7 us per decision, K = 4 140.7 vs 154.1, K = 8 252.3 vs 284.6); with one force warp it does
+        // not (1024 x 64, K = 4: 40.4 vs 32.4).  K = 1 keeps its choice.
+        else if (rep && E > sms && nf >= 96) place = RASTER_FOLLOW;
         else place = RASTER_WARPS;
         if (place == RASTER_FOLLOW && !follow_fits) place = RASTER_WARPS;
         if (place == RASTER_WARPS && !warps_fit) place = RASTER_SELF;
@@ -1598,7 +1657,7 @@ int plan_step(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io,
     out->filler = (self && ((p->grid_size * p->grid_size) & 7) == 0 && (reinterpret_cast<uintptr_t>(io->grid) & 15) == 0 &&
                    nf + 32 <= kMaxThreads && E <= (long long)sms * (65536 / (64 * (nf + 32)))) ? 1 : 0;
     out->nt = nf + (warps ? raster_threads(N, A, nf, E, sms) : 0) + (out->filler ? 32 : 0);
-    out->kernel = step_kernel(mode, p->math_mode != 0, place, fin, phys);
+    out->kernel = step_kernel(mode, p->math_mode != 0, place, fin, phys, rep);
     if ((rc = prep(out->kernel, out->smem))) return rc;
     int grid = 0;
     if ((rc = persistent_grid(out->kernel, out->nt, out->smem, E, &grid))) return rc;
@@ -1618,10 +1677,11 @@ int plan_step(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io,
 
 extern "C" {
 
-static int step_plan_out(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io, const bool phys, int32_t out[8]) {
+static int step_plan_out(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io, const bool phys, int32_t out[8],
+                         const int repeat = 1) {
     if (!out) return SWARM_ERR_NULL;
     StepPlan pl;
-    const int rc = plan_step(p, st, io, nullptr, &pl, false, phys);
+    const int rc = plan_step(p, st, io, nullptr, &pl, false, phys, repeat);
     if (rc) return rc;
     out[0] = pl.mode; out[1] = pl.filler; out[2] = pl.place; out[3] = pl.nt; out[4] = pl.grid;
     out[5] = (int32_t)pl.smem; out[6] = pl.place == RASTER_FOLLOW ? pl.rgrid : (pl.place == RASTER_CLUSTER ? pl.cluster : 0);
@@ -1638,6 +1698,14 @@ int swarm_step_plan_physics(const SwarmParams* p, const SwarmState* st, const Sw
     int rc = validate(p);
     if (!rc) rc = check_physics(phys);
     return rc ? rc : step_plan_out(p, st, io, true, out);
+}
+
+int swarm_step_plan_repeat(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io, const SwarmPhysics* phys,
+                           int32_t repeat, int32_t out[8]) {
+    int rc = validate(p);
+    if (!rc && repeat < 1) rc = SWARM_ERR_SIZE;
+    if (!rc && phys) rc = check_physics(phys);
+    return rc ? rc : step_plan_out(p, st, io, phys != nullptr, out, repeat);
 }
 
 // SwarmStateProcessor.process_state of the batch (or of the envs with mask[e] != 0): swarm_rasterize's launches.
@@ -1668,11 +1736,12 @@ static int rasterize_launch(const SwarmParams* p, const double* x, const double*
 }
 
 // swarm_step's launches; with terminal outputs (fin_out != NULL) the FIN variants of the step kernels, with per-env
-// physics (phys_in != NULL, checked) the PHYS ones
+// physics (phys_in != NULL, checked) the PHYS ones, with repeat > 1 the REP ones
 static int step_launch(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io, const SwarmStepFinal* fin_out,
-                       const SwarmInjectedDraws* reset_draws, swarm_stream_t stream, const SwarmPhysics* phys_in = nullptr) {
+                       const SwarmInjectedDraws* reset_draws, swarm_stream_t stream, const SwarmPhysics* phys_in = nullptr,
+                       const int repeat = 1) {
     StepPlan pl;
-    int rc = plan_step(p, st, io, reset_draws, &pl, fin_out != nullptr, phys_in != nullptr);
+    int rc = plan_step(p, st, io, reset_draws, &pl, fin_out != nullptr, phys_in != nullptr, repeat);
     const SwarmStepFinal fin = fin_out ? *fin_out : kNoFinal;
     const SwarmPhysics phys = phys_in ? *phys_in : kNoPhysics;
     if (rc) return rc;
@@ -1691,7 +1760,7 @@ static int step_launch(const SwarmParams* p, const SwarmState* st, const SwarmSt
     const size_t smem = pl.smem, follow_smem = pl.follow_smem;
     if (pl.place == RASTER_CLUSTER) {      // no PDL: a cluster launch is an ordinary dependent of its predecessor
         const ClusterShape sh = {pl.cluster, nf, nt, smem};
-        return launch_cluster(kernel, sh, p->n_envs, s, "swarm_step", kp, *st, *io, dr, has, nf, fin, phys);
+        return launch_cluster(kernel, sh, p->n_envs, s, "swarm_step", kp, *st, *io, dr, has, nf, fin, phys, repeat);
     }
     if (pl.place != RASTER_FOLLOW) {
         // Single-kernel shapes are launched as programmatic dependents of whatever precedes them in the stream: when that is
@@ -1712,7 +1781,7 @@ static int step_launch(const SwarmParams* p, const SwarmState* st, const SwarmSt
         const bool pdl = !no_pdl && (pl.place == RASTER_WARPS ? p->n_envs <= sms
                                                                : (p->n_locusts < 160 || p->n_envs <= 2 * sms));
         if (!pdl) {
-            kernel<<<grid, nt, smem, s>>>(kp, *st, *io, dr, has, nf, fin, phys);
+            kernel<<<grid, nt, smem, s>>>(kp, *st, *io, dr, has, nf, fin, phys, repeat);
             return check_launch("swarm_step");
         }
         cudaLaunchConfig_t cfg;
@@ -1726,7 +1795,7 @@ static int step_launch(const SwarmParams* p, const SwarmState* st, const SwarmSt
         attr[0].val.programmaticStreamSerializationAllowed = 1;
         cfg.attrs = attr;
         cfg.numAttrs = 1;
-        const cudaError_t le = cudaLaunchKernelEx(&cfg, kernel, kp, *st, *io, dr, has, nf, fin, phys);
+        const cudaError_t le = cudaLaunchKernelEx(&cfg, kernel, kp, *st, *io, dr, has, nf, fin, phys, repeat);
         if (le != cudaSuccess) return cuda_fail(le, "swarm_step (cudaLaunchKernelEx)");
         return check_launch("swarm_step");
     }
@@ -1760,7 +1829,7 @@ static int step_launch(const SwarmParams* p, const SwarmState* st, const SwarmSt
     err = cudaEventRecord(ss.fork, s);
     if (err == cudaSuccess) err = cudaStreamWaitEvent(ss.stream, ss.fork, 0);
     if (err != cudaSuccess) return cuda_fail(err, "fork");
-    kernel<<<grid, nt, smem, s>>>(kp, *st, *io, dr, has, nf, fin, phys);
+    kernel<<<grid, nt, smem, s>>>(kp, *st, *io, dr, has, nf, fin, phys, repeat);
     if ((rc = check_launch("swarm_step"))) return rc;
     k_raster_follow<<<rgrid, follow_threads, follow_smem, ss.stream>>>(kp, st->x, st->xa, io->grid, io->positions,
                                                                         st->work + 2);
@@ -1776,13 +1845,14 @@ int swarm_step(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io
     return step_launch(p, st, io, nullptr, reset_draws, stream);
 }
 
-// swarm_step_final with optional per-env physics (phys checked by the caller)
+// swarm_step_final with optional per-env physics (phys checked by the caller) and action repeat
 static int step_final_launch(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io, const SwarmStepFinal* fin,
-                             const SwarmInjectedDraws* reset_draws, swarm_stream_t stream, const SwarmPhysics* phys) {
-    if (!fin) return step_launch(p, st, io, nullptr, reset_draws, stream, phys);
+                             const SwarmInjectedDraws* reset_draws, swarm_stream_t stream, const SwarmPhysics* phys,
+                             const int repeat = 1) {
+    if (!fin) return step_launch(p, st, io, nullptr, reset_draws, stream, phys, repeat);
     if ((fin->grid != nullptr) != (fin->positions != nullptr)) return SWARM_ERR_FLAGS;
     if (fin->grid && (!fin->x || !fin->xa || !grid_aligned(fin->grid))) return SWARM_ERR_FLAGS;
-    int rc = step_launch(p, st, io, fin, reset_draws, stream, phys);
+    int rc = step_launch(p, st, io, fin, reset_draws, stream, phys, repeat);
     if (rc || !fin->grid) return rc;
     // The terminal observations: the standalone rasteriser over the done envs, as an ORDINARY launch behind the step (and
     // the follower's join), so it reads fin->x / io->done only once the step grid has completed -- k_step triggers its
@@ -1801,6 +1871,15 @@ int swarm_step_physics(const SwarmParams* p, const SwarmState* st, const SwarmSt
     int rc = validate(p);
     if (!rc) rc = check_physics(phys);
     return rc ? rc : step_final_launch(p, st, io, fin, reset_draws, stream, phys);
+}
+
+int swarm_step_repeat(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io, const SwarmStepFinal* fin,
+                      const SwarmPhysics* phys, int32_t repeat, const SwarmInjectedDraws* reset_draws, swarm_stream_t stream) {
+    int rc = validate(p);
+    if (!rc && repeat < 1) rc = SWARM_ERR_SIZE;
+    if (!rc && phys) rc = check_physics(phys);
+    // repeat 1: the kernels and launches of swarm_step / swarm_step_final / swarm_step_physics
+    return rc ? rc : step_final_launch(p, st, io, fin, reset_draws, stream, phys, repeat);
 }
 
 void swarm_step_host_clear(void) { host_cache().clear(); }

@@ -1,6 +1,6 @@
 // libswarm_b200_torch.so -- the C ABI of include/swarm_b200.h exposed as a PyTorch extension:
 //   torch.ops.swarm_b200.{step, step_final, step_host, reset, rasterize, expand_obs, clip_actions, forces,
-//                         reset_physics, step_physics, forces_physics}
+//                         reset_physics, step_physics, forces_physics, step_repeat}
 // Each op checks device / dtype / contiguity / shape of its tensors, takes the CURRENT CUDA stream of
 // the tensors' device and forwards plain pointers to the extern "C" entry point of libswarm_b200.so.
 // No arithmetic happens here.  `params` is a CPU uint8 tensor holding the SwarmParams POD
@@ -295,6 +295,47 @@ void op_step_physics(const at::Tensor& params, at::Tensor x, at::Tensor xa, at::
           "swarm_step_physics");
 }
 
+// action repeat (swarm_step_repeat): op_step_physics with the physics table optional and the repeat count
+void op_step_repeat(const at::Tensor& params, at::Tensor x, at::Tensor xa, at::Tensor noise_x, at::Tensor noise_a,
+                    at::Tensor elapsed, at::Tensor episode, c10::optional<at::Tensor> work, at::Tensor actions,
+                    c10::optional<at::Tensor> noise_a_step, c10::optional<at::Tensor> noise_x_step, at::Tensor reward,
+                    at::Tensor done, c10::optional<at::Tensor> grid, c10::optional<at::Tensor> positions,
+                    c10::optional<at::Tensor> v_out, int64_t flags, at::TensorList reset_draws, int64_t repeat,
+                    c10::optional<at::Tensor> physics, int64_t physics_flags, at::ArrayRef<double> physics_lo,
+                    at::ArrayRef<double> physics_hi, c10::optional<at::Tensor> final_x, c10::optional<at::Tensor> final_xa,
+                    c10::optional<at::Tensor> terminated, c10::optional<at::Tensor> truncated,
+                    c10::optional<at::Tensor> final_grid, c10::optional<at::Tensor> final_positions) {
+    const SwarmParams p = unpack(params);
+    c10::cuda::CUDAGuard guard(x.device());
+    TORCH_CHECK(repeat >= 1 && repeat <= INT32_MAX, "repeat must be a positive int32, got ", repeat);
+    const SwarmState st = make_state(p, x, xa, noise_x, noise_a, elapsed, episode, work);
+    const SwarmStepIO io = make_io(p, actions, noise_a_step, noise_x_step, reward, done, grid, positions, v_out, flags);
+    const int64_t E = p.n_envs, N = p.n_locusts, A = p.n_agents, G = p.grid_size;
+    if (final_x.has_value()) need(*final_x, at::kDouble, {E, N, 2}, "final_x");
+    if (final_xa.has_value()) need(*final_xa, at::kDouble, {E, A, 2}, "final_xa");
+    if (terminated.has_value()) need(*terminated, at::kByte, {E}, "terminated");
+    if (truncated.has_value()) need(*truncated, at::kByte, {E}, "truncated");
+    if (final_grid.has_value()) need(*final_grid, at::kFloat, {E, G, G, 2}, "final_grid");
+    if (final_positions.has_value()) need(*final_positions, at::kByte, {E, A, 2}, "final_positions");
+    bool same = actions.get_device() == x.get_device() && reward.get_device() == x.get_device() &&
+                done.get_device() == x.get_device();
+    for (const c10::optional<at::Tensor>* t : {&grid, &positions, &final_x, &final_xa, &terminated, &truncated, &final_grid,
+                                               &final_positions})
+        same = same && (!t->has_value() || (*t)->get_device() == x.get_device());
+    TORCH_CHECK(same, "step_repeat: all tensors must be on x's device");
+    SwarmPhysics ph;
+    if (physics.has_value()) ph = make_physics(p, *physics, physics_flags, physics_lo, physics_hi, x);
+    SwarmInjectedDraws dr;
+    if (reset_draws.size()) dr = make_draws(p, reset_draws);
+    const bool any_fin = final_x.has_value() || final_xa.has_value() || terminated.has_value() || truncated.has_value() ||
+                         final_grid.has_value() || final_positions.has_value();
+    const SwarmStepFinal fin{ptr<double>(final_x), ptr<double>(final_xa), ptr<uint8_t>(terminated), ptr<uint8_t>(truncated),
+                             ptr<float>(final_grid), ptr<uint8_t>(final_positions)};
+    check(swarm_step_repeat(&p, &st, &io, any_fin ? &fin : nullptr, physics.has_value() ? &ph : nullptr, (int32_t)repeat,
+                            reset_draws.size() ? &dr : nullptr, stream_of(x)),
+          "swarm_step_repeat");
+}
+
 void op_forces_physics(const at::Tensor& params, const at::Tensor& x, const at::Tensor& xa, c10::optional<at::Tensor> v,
                        c10::optional<at::Tensor> reward, at::Tensor physics, int64_t physics_flags,
                        at::ArrayRef<double> physics_lo, at::ArrayRef<double> physics_hi) {
@@ -345,5 +386,12 @@ TORCH_LIBRARY(swarm_b200, m) {
           &op_step_physics);
     m.def("forces_physics(Tensor params, Tensor x, Tensor xa, Tensor(a!)? v, Tensor(b!)? reward, Tensor physics, "
           "int physics_flags, float[] physics_lo, float[] physics_hi) -> ()", &op_forces_physics);
+    m.def("step_repeat(Tensor params, Tensor(a!) x, Tensor(b!) xa, Tensor(c!) noise_x, Tensor(d!) noise_a, "
+          "Tensor(e!) elapsed, Tensor(f!) episode, Tensor(m!)? work, Tensor(g!) actions, Tensor? noise_a_step, "
+          "Tensor? noise_x_step, Tensor(h!) reward, Tensor(i!) done, Tensor(j!)? grid, Tensor(k!)? positions, "
+          "Tensor(l!)? v_out, int flags, Tensor[] reset_draws, int repeat, Tensor(t!)? physics, int physics_flags, "
+          "float[] physics_lo, float[] physics_hi, Tensor(n!)? final_x, Tensor(o!)? final_xa, Tensor(p!)? terminated, "
+          "Tensor(q!)? truncated, Tensor(r!)? final_grid, Tensor(s!)? final_positions) -> ()",
+          &op_step_repeat);
     m.def("abi_version() -> int", &op_abi_version);
 }

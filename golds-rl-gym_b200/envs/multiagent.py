@@ -85,6 +85,10 @@ class BatchedSwarmEnv(object):
     ``_native.PHYSICS_COLUMNS`` (SwarmPhysics).  ``"table"`` fills it from the class constants and leaves it to the
     caller, who may write rows between calls; a dict of per-column ranges such as ``{"F": (0.3, 0.7), "L": (5, 15)}``
     draws each env's row anew, uniformly, at every reset of that env (explicit or auto-reset), inside the kernels.
+    With ``action_repeat`` K > 1 every step() makes up to K env steps with the same actions inside one kernel
+    (swarm_step_repeat): reward is the FP32 sum of the substeps' rewards, an env stops at its first done substep (and
+    then auto-resets once), elapsed and the TimeLimit count env steps, and the observation is that of the returned state.
+    The attribute may be changed between calls.
     """
 
     # fed_gym/envs/multiagent.py:8-21
@@ -100,7 +104,8 @@ class BatchedSwarmEnv(object):
 
     def __init__(self, num_envs, n_locusts=None, n_agents=None, grid_size=84, max_episode_steps=128,
                  seed=0, env_id_offset=0, device=None, math_mode="fast", auto_reset=True, rasterize=True,
-                 binding="torch", tuning=0, noise="frozen", cluster=None, final_obs=False, physics=None):
+                 binding="torch", tuning=0, noise="frozen", cluster=None, final_obs=False, physics=None,
+                 action_repeat=1):
         """binding: "torch" = the hot calls go through torch.ops.swarm_b200.* (the C ABI as a PyTorch
         extension, csrc/torch_binding.cpp), "ctypes" = straight into the C ABI.  Same kernels either way.
         tuning: SwarmParams.tuning (0 = automatic launch shape; anything else only changes speed, never bits).
@@ -109,7 +114,8 @@ class BatchedSwarmEnv(object):
         cluster: None = one CTA per env up to 2048 locusts and a thread-block cluster of the library's size above; an
         integer K = a cluster of K CTAs per env (1..16, for 512 < n_locusts <= 8192; bitwise the same results).
         physics: None (every env uses the class constants), "table" (per-env rows in self.physics, written by the caller)
-        or a dict {column: (lo, hi)} (per-env rows redrawn at every reset; unnamed columns stay at the class constant)."""
+        or a dict {column: (lo, hi)} (per-env rows redrawn at every reset; unnamed columns stay at the class constant).
+        action_repeat: env steps per step() call with the same actions (1 = one step, the default)."""
         self.lib = nat.load()
         if binding not in ("torch", "ctypes"):
             raise ValueError("binding must be 'torch' or 'ctypes'")
@@ -179,7 +185,16 @@ class BatchedSwarmEnv(object):
                                            _ptr(self.truncated), None, None)
             self._fin_ref = ctypes.byref(self._fin)
         self._init_physics(physics)
+        self.action_repeat = action_repeat
+        self._repeat()
         self.refresh_params()
+
+    def _repeat(self):
+        """self.action_repeat, checked (the caller may change it between calls)."""
+        k = self.action_repeat
+        if isinstance(k, bool) or int(k) != k or not 1 <= int(k) < 2 ** 31:
+            raise ValueError("action_repeat must be a positive integer, got %r" % (k,))
+        return int(k)
 
     def _init_physics(self, physics):
         self.physics = None
@@ -268,11 +283,23 @@ class BatchedSwarmEnv(object):
         auto_reset = self.auto_reset if auto_reset is None else auto_reset
         flags = (nat.SWARM_STEP_AUTO_RESET if auto_reset else 0) | (nat.SWARM_STEP_CLIP_ACTIONS if clip else 0) | \
                 (0 if add_wind else nat.SWARM_STEP_NO_ACTION_WIND) | self._noise_flag
+        repeat = self._repeat()
         if self.ops is not None:
             if actions.dtype not in (torch.float32, torch.float64):
                 raise ValueError("actions must be float32 or float64")
             g_t = (grid_out if grid_out is not None else self.grid) if rasterize else None
             p_t = (positions_out if positions_out is not None else self.positions) if rasterize else None
+            if repeat > 1:
+                fin = [None] * 6
+                if self.final_obs:
+                    fg, fp = self._final_obs_bufs(rasterize, final_grid_out, final_positions_out)
+                    fin = [self.final_x, self.final_xa, self.terminated, self.truncated, fg, fp]
+                phys = self._phys_args() if self.physics is not None else (None, 0, [0.0] * 6, [0.0] * 6)
+                self.ops.step_repeat(self._blob, *self._state_t, actions, noise_a, noise_x, self.reward, self.done_u8,
+                                     g_t, p_t, v_out, flags, reset_draws.tensors() if reset_draws is not None else [],
+                                     repeat, *phys, *fin)
+                info = self._info(fin[4], fin[5]) if self.final_obs else {}
+                return (self.x, self.xa), self.reward, self._done_view, info
             if self.physics is not None:
                 dts = reset_draws.tensors() if reset_draws is not None else []
                 fin = [None] * 6
@@ -311,6 +338,20 @@ class BatchedSwarmEnv(object):
             io.grid, io.positions = None, None
         io.v_out = v_out.data_ptr() if v_out is not None else None
         io.flags = flags
+        if repeat > 1:
+            fin_ref, info = None, {}
+            if self.final_obs:
+                fg, fp = self._final_obs_bufs(rasterize, final_grid_out, final_positions_out)
+                self._fin.grid, self._fin.positions = _ptr(fg), _ptr(fp)
+                fin_ref, info = self._fin_ref, self._info(fg, fp)
+            with self._ctx:
+                rc = self.lib.swarm_step_repeat(self._params_ref, self._state_ref, self._io_ref, fin_ref,
+                                                self._phys_ref if self.physics is not None else None, repeat,
+                                                ctypes.byref(reset_draws.c) if reset_draws is not None else None,
+                                                torch.cuda.current_stream(self.device).cuda_stream)
+            if rc:
+                nat.check(rc, "swarm_step_repeat")
+            return (self.x, self.xa), self.reward, self._done_view, info
         if self.physics is not None:
             fin_ref, info = None, {}
             if self.final_obs:
@@ -386,8 +427,13 @@ class BatchedSwarmEnv(object):
             io.grid, io.positions = self._grid_ptr, self._pos_ptr
         io.flags = nat.SWARM_STEP_AUTO_RESET if self.auto_reset else 0
         out = (ctypes.c_int32 * 8)()
+        repeat = self._repeat()
         with self._ctx:
-            if self.physics is not None:
+            if repeat > 1:
+                nat.check(self.lib.swarm_step_plan_repeat(self._params_ref, self._state_ref, ctypes.byref(io),
+                                                          self._phys_ref if self.physics is not None else None, repeat,
+                                                          out), "swarm_step_plan_repeat")
+            elif self.physics is not None:
                 nat.check(self.lib.swarm_step_plan_physics(self._params_ref, self._state_ref, ctypes.byref(io),
                                                            self._phys_ref, out), "swarm_step_plan_physics")
             else:
@@ -410,9 +456,11 @@ class BatchedSwarmEnv(object):
         for the device-resident policy unless host_grid / host_positions are given (then it is also copied back:
         the numpy-out case of the reference's process_state).  Synchronises the stream.  Pinned tensors are read /
         written by the kernel itself over PCIe (zero-copy); self.reward / self.done_u8 are then NOT updated.
-        Not available with per-env physics (swarm_step_host takes no SwarmPhysics)."""
+        Not available with per-env physics or action repeat (swarm_step_host takes neither)."""
         if self.physics is not None:
             raise ValueError("step_host has no per-env physics (swarm_step_host takes no SwarmPhysics); use step()")
+        if self._repeat() > 1:
+            raise ValueError("step_host has no action repeat (swarm_step_host makes one env step); use step()")
         io = self._io_host
         if io is None:
             io = self._io_host = nat.SwarmStepIO()

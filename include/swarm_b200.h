@@ -221,6 +221,24 @@ int swarm_forces_physics(const SwarmParams* p, const SwarmPhysics* phys, const d
 int swarm_step_plan_physics(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io, const SwarmPhysics* phys,
                             int32_t out[8]);
 
+/* Action repeat (frame skip): one call makes up to `repeat` env steps per env with the call's actions, each exactly the
+ * step swarm_step makes (actions converted and, with SWARM_STEP_CLIP_ACTIONS, clipped and written back once; elapsed
+ * advances per substep; fresh noise draws row n_burn_in + elapsed for each substep; io->noise_a / io->noise_x overrides
+ * serve every substep).  An env stops at its first done substep; then the auto-reset (if requested) runs once.
+ * reward[e] is the FP32 sum, in substep order, of the stepped substeps' rewards; done, fin->terminated / truncated /
+ * x / xa and v_out are the last stepped substep's; grid / positions are the observation of the state the call returns.
+ * Bit for bit: one swarm_step* call with the call's flags, then up to repeat - 1 calls without SWARM_STEP_CLIP_ACTIONS
+ * and SWARM_STEP_AUTO_RESET, each env stopping at its first done, a masked swarm_reset* of the done envs (with
+ * auto-reset), and the observation of the final state.
+ * fin and phys are nullable: with both NULL this is swarm_step, with one of them swarm_step_final / swarm_step_physics.
+ * repeat == 1 launches exactly the kernels of those calls.  The argument checks are theirs; repeat < 1 is
+ * SWARM_ERR_SIZE, before any CUDA call.  swarm_step_host has no repeat. */
+int swarm_step_repeat(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io, const SwarmStepFinal* fin,
+                      const SwarmPhysics* phys, int32_t repeat, const SwarmInjectedDraws* reset_draws, swarm_stream_t stream);
+/* swarm_step_plan for swarm_step_repeat (phys nullable). */
+int swarm_step_plan_repeat(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io, const SwarmPhysics* phys,
+                           int32_t repeat, int32_t out[8]);
+
 /* The launch shape swarm_step would use for these arguments (no launch; needs the device for occupancy queries):
  * out = { force mode, filler warp (0/1), rasteriser placement (0 none, 1 follower kernel, 2 raster warps, 3 the step's
  * own threads, 4 the env's thread-block cluster), threads per CTA, CTAs (E K in the cluster layout), dynamic shared
@@ -235,7 +253,9 @@ int swarm_step_plan(const SwarmParams* p, const SwarmState* st, const SwarmStepI
  * io->reward / io->done back.
  * host_grid / host_positions: nullable (both or neither; need io->grid): the compact observation
  * (E,G,G,2) f32 + (E,A,2) u8 is also copied back to the host (copy engine, after the step) -- the
- * numpy-out case of the reference's process_state. */
+ * numpy-out case of the reference's process_state.
+ * One env step per call, with the class-wide physics: no per-env physics and no action repeat (swarm_step_physics,
+ * swarm_step_repeat). */
 int swarm_step_host(const SwarmParams* p, const SwarmState* st, const SwarmStepIO* io,
                     const float* host_actions, float* host_reward, uint8_t* host_done,
                     float* host_grid, uint8_t* host_positions, swarm_stream_t stream);

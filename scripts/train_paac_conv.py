@@ -5,7 +5,7 @@
     torchrun --nproc-per-node 8 scripts/train_paac_conv.py -ec 8192 --clip_norm=1    # config 5: env batch sharded
 
 Flag names and defaults are the reference's; additions: --n_locusts, --max_updates, --no_cuda_graph,
---reward_indexing, --mask_terminals, --bootstrap_truncated, --fresh_noise, --physics.
+--reward_indexing, --mask_terminals, --bootstrap_truncated, --fresh_noise, --physics, --action_repeat.
 '-d/--device' accepts the reference's '/gpu:0' spelling.
 """
 import argparse
@@ -52,7 +52,8 @@ def get_network_and_environment_creator(args, random_seed=3):
     pv = pkg.submodule("agents.paac.policy_v_network")
     env_creator = ec.SwarmEnvironmentCreator(n_locusts=args.n_locusts, grid_size=args.height,
                                              noise="fresh" if getattr(args, "fresh_noise", False) else "frozen",
-                                             physics=getattr(args, "physics", None))
+                                             physics=getattr(args, "physics", None),
+                                             action_repeat=getattr(args, "action_repeat", 1))
     args.num_actions = env_creator.num_actions
     args.random_seed = random_seed
     network_conf = {
@@ -119,6 +120,8 @@ def get_arg_parser():
     parser.add_argument('--physics', default=None, type=physics_ranges,
                         help="per-env physics redrawn at every reset of each training env, e.g. 'F=0.3:0.7,L=5:15' "
                              "(columns noise, gravity, wind, F, L, dt; unnamed ones keep the reference's constant)")
+    parser.add_argument('--action_repeat', default=1, type=int,
+                        help="env steps per decision, rewards summed (frame skip); gamma stays per decision")
     parser.add_argument('--eval_every', default=30.0, type=float,
                         help="seconds between evaluation episodes on Swarm-eval-v0 (policy_monitor.py); 0 = off")
     parser.add_argument('--net_precision', default='fp32', choices=['fp32', 'tf32', 'bf16'],
@@ -158,7 +161,8 @@ def main(args):
         sp = pkg.submodule("agents.state_processors")
         monitor = pm.SwarmPolicyMonitor(global_policy_net=learner.network,
                                         state_processor=sp.SwarmStateProcessor(grid_size=args.height),
-                                        out_dir=args.debugging_folder, fresh_noise=args.fresh_noise)
+                                        out_dir=args.debugging_folder, fresh_noise=args.fresh_noise,
+                                        action_repeat=args.action_repeat)
     fps = learner.train(max_updates=args.max_updates, monitor=monitor, eval_every=args.eval_every,
                         summary_dir=args.debugging_folder)     # scalars: global_norm, rl/reward (summaries.jsonl)
     if int(os.environ.get("RANK", "0")) == 0:
